@@ -7,7 +7,7 @@ full-row search range (x' in [0, x]), SAD cost, first-minimum selection, then th
 reference's ResolveMatchList over the winners on the device (resolved disparity map).
 290 625 windows and 90 965 625 candidate evaluations per pair.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...     (one rank per GPU; no data-path collective)
 
 `value`  : pairs/s of the whole step (matching kernel + resolve kernel) with the frames already
@@ -22,6 +22,10 @@ reference's ResolveMatchList over the winners on the device (resolved disparity 
 `configs`: the other BASELINE configurations on the same line (C3 device-resident, C4 this rank's
            shard of the 4096-pair 1080p batch device-resident and end to end, C5 paired
            unsynchronised streams end to end), each with its own parity flag.
+`--dump-outputs DIR`: after the timed steps, what the last step computed for rank 0 — resolved_disparity_u16,
+           disparity_u16 and raw_cost_u16 of DUMP_PAIRS pairs drawn with a fixed seed, [pairs, rows, cols] —
+           as DIR/<name>.npy in float32 (NO_DISPARITY stays 65535). The inputs are seeded, so two builds run
+           with the same arguments can be compared output for output.
 `cpu_baseline` / `--impl reference`: the CPU arms, timed on the box's host cores on a bounded
            sample of the same workload: `sliding` (oracle/sliding_sad_cpu.c — the GPU kernel's own
            formulation, OpenMP, all cores; this is the arm `--impl reference` reports, so that the
@@ -49,6 +53,7 @@ PAIRS_PER_GPU = 256
 # leaving it, and one VIMNMX at twice the VABSDIFF4 issue rate (counted 0.5).
 ALU_OPS_PER_EVAL = 2.5
 HOST_BIN = os.path.join(ROOT, "unsynchronized_stereo_vision_proj325_b200", "usv_host_test")
+DUMP_PAIRS = 16  # 3 arrays x 16 pairs x 290 625 windows x 4 B = 56 MB
 
 
 class ClockSampler(threading.Thread):
@@ -237,7 +242,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3 / C4 / C5 block (dev only)")
     ap.add_argument("--c4-pairs", type=int, default=4096, help="global C4 batch (dev only; BASELINE says 4096)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -320,6 +328,12 @@ def main():
     t_clk0 = time.time()
     ms_total = timed_loop(step_device, args.steps)
     launches = ctx.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        pairs = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_PAIRS), replace=False))
+        for name, o in (("resolved_disparity_u16", o_res), ("disparity_u16", o_disp), ("raw_cost_u16", o_cost)):
+            a = np.stack([o[int(i) * n_win:(int(i) + 1) * n_win].cpu().numpy().view(np.uint16) for i in pairs])
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a.astype(np.float32).reshape(len(pairs), ny, nx))
     ms_step = ms_total / args.steps
     value = world * n * args.steps / (ms_total * 1e-3)
     # the matching kernel alone, same inputs: the roofline's launch

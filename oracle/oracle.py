@@ -4,6 +4,7 @@ TEST INFRASTRUCTURE ONLY — imported by tests/, __graft_entry__.smoke() and
 bench.py's cpu_baseline / --impl reference legs, never by the product package.
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -14,6 +15,9 @@ from unsynchronized_stereo_vision_proj325_b200 import _abi
 HERE = os.path.dirname(os.path.abspath(__file__))
 ORACLE_SO = os.path.join(HERE, "_build", "libusv_oracle.so")
 REF_SO = os.path.join(HERE, "_ref", "libusv_ref.so")
+# the reference's answers on the inputs the tests give it (tests/golden/make_ref_answers.py): the ref_* functions
+# below answer from this file when the reference's own code is not built, which is the case in any plain checkout
+REF_ANSWERS = os.path.join(HERE, "..", "tests", "golden", "ref_answers.npz")
 
 
 def build(quiet=True):
@@ -92,6 +96,39 @@ def ref():
         R.ref_rad2deg.argtypes = [C.c_double]
         _ref = R
     return _ref
+
+
+_answers = None
+
+
+def answer_key(name, *inputs):
+    """Key of one call of the reference in REF_ANSWERS: a 64-bit digest of the function's name and its inputs."""
+    h = hashlib.sha256(name.encode())
+    for a in inputs:
+        a = np.ascontiguousarray(a)
+        h.update(repr((a.shape, a.dtype.descr)).encode())
+        h.update(a.tobytes())
+    return int.from_bytes(h.digest()[:8], "little")
+
+
+def recorded_answer(name, *inputs):
+    """The reference's recorded answer to `name` on these inputs. REF_ANSWERS holds, per function, the keys of its
+    calls, their answers concatenated along the first axis, and where each answer starts."""
+    global _answers
+    if _answers is None:
+        _answers = {}
+        with np.load(REF_ANSWERS) as z:
+            for f in z.files:
+                if f.endswith(".keys"):
+                    fn = f[:-len(".keys")]
+                    offsets, data = z[fn + ".offsets"], z[fn + ".data"]
+                    for i, k in enumerate(z[f]):
+                        _answers[fn, int(k)] = data[offsets[i]:offsets[i + 1]]
+    key = answer_key(name, *inputs)
+    if (name, key) not in _answers:
+        raise LookupError("no recorded reference answer for this %s input (key %016x): build oracle/_ref from the reference "
+                          "source, or record it with tests/golden/make_ref_answers.py" % (name, key))
+    return _answers[name, key]
 
 
 def _ptr(a):
@@ -212,6 +249,9 @@ def resolve_match_list(matches):
 
 
 def ref_resolve_match_list(matches):
+    if ref() is None:  # recorded as the input positions of the output records: every output record is an input record
+        m = np.ascontiguousarray(matches, dtype=_abi.MATCH_DTYPE)
+        return m[recorded_answer("resolve_match_list", m)]
     return _resolve(ref().ref_resolve_match_list, matches)
 
 
@@ -231,6 +271,8 @@ def id_matcher(cur, old):
 
 
 def ref_id_matcher(cur, old):
+    if ref() is None:
+        return recorded_answer("id_matcher", np.asarray(cur, _abi.MATCH_DTYPE), np.asarray(old, _abi.MATCH_DTYPE))
     return _id_matcher(ref().ref_id_matcher, cur, old)
 
 
@@ -255,8 +297,12 @@ def moving_object_distance(*a):
     return _moving(lib().usv_oracle_moving_object_distance, False, *a)
 
 
-def ref_moving_object_distance(*a):
-    return _moving(ref().ref_moving_object_distance, True, *a)
+def ref_moving_object_distance(camera_side, t_this, this_xy, other_xy, old_xy, older_xy, idx3, t_other, t_old, t_older):
+    if ref() is None:
+        return recorded_answer("moving_object_distance", np.array([camera_side, t_this, t_other, t_old, t_older], np.int64),
+                               *map(_f32, (this_xy, other_xy, old_xy, older_xy)), np.asarray(idx3, np.int32).reshape(-1, 3))
+    return _moving(ref().ref_moving_object_distance, True, camera_side, t_this, this_xy, other_xy, old_xy, older_xy, idx3,
+                   t_other, t_old, t_older)
 
 
 def coordinate_position(camera_side, dist, xy):
@@ -270,9 +316,23 @@ def coordinate_position(camera_side, dist, xy):
 def ref_coordinate_position(camera_side, dist, xy):
     dist = np.ascontiguousarray(dist, np.float64)
     xy = _f32(xy)
+    if ref() is None:
+        return recorded_answer("coordinate_position", np.int32(camera_side), dist, xy)
     out = np.zeros((len(dist), 3), np.float64)
     n = ref().ref_coordinate_position(C.c_int(int(camera_side)), _ptr(dist), _ptr(xy), C.c_int(len(dist)), _ptr(out))
     return out[:n]
+
+
+def ref_sizeof_match():
+    return int(recorded_answer("sizeof_match")[0]) if ref() is None else ref().ref_sizeof_match()
+
+
+def ref_deg2rad(v):
+    return float(recorded_answer("deg2rad", np.float64(v))[0]) if ref() is None else ref().ref_deg2rad(v)
+
+
+def ref_rad2deg(v):
+    return float(recorded_answer("rad2deg", np.float64(v))[0]) if ref() is None else ref().ref_rad2deg(v)
 
 
 def pair_nearest(t_left, t_right, max_dt):
