@@ -86,7 +86,7 @@ int BlockSearch(bool CameraSide, const usv::ImageView* ImportGrayThisCamera, con
 // thread per device, each with its own context, pinned ring and CUDA streams; pair p goes to device floor(p * G / N)
 // (contiguous blocks, no inter-GPU exchange); every worker lands its results in its own disjoint slice of the caller's
 // arrays. Per window: ResolvedDisparity = d of the window's winner if its record survives ResolveMatchList
-// (generate -> accept -> resolve all on the device), else 0xFFFF; RawCost (optional, SAD with 255 * n < 65536) = the
+// (generate -> accept -> resolve all on the device), else 0xFFFF; RawCost (optional, SAD with 255 * n < 65535) = the
 // winner's integer cost. Distance = DistanceTable(...)[d]. Page-lock the frame and result arrays once with
 // BlockSearchPinHostBuffer for asynchronous copies (pageable memory works, slower).
 struct BlockSearchBatchStats {

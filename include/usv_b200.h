@@ -118,8 +118,9 @@ typedef struct usv_outputs {
                             * (candidate on the other side of the window) is stored modulo 2^16, and -1 then
                             * reads as USV_NO_DISPARITY — take right_index or matches for such ranges */
   uint16_t *raw_cost_u16;  /* raw_cost as u16 (0xFFFF = no candidate): SAD only,
-                              and only when 255*tmpl_w*tmpl_h*channels fits 16
-                              bits (else USV_ERR_UNSUPPORTED); lossless        */
+                              and only when 255*tmpl_w*tmpl_h*channels < 0xFFFF,
+                              so that no real cost reads as "no candidate"
+                              (else USV_ERR_UNSUPPORTED); lossless             */
   uint16_t *resolved_disparity_u16;
   /* Dense sweep only. The disparity map after ResolveMatchList (P/Main.cpp:432-477)
    * has run over the pair's accepted winners ON THE DEVICE: entry = d of the window's

@@ -152,7 +152,7 @@ def _with_cost_u16(arrs, mask, had_raw):
     """raw_cost_u16 (include/usv_b200.h): the u32 cost narrowed to 16 bits; ~0 (no candidate) becomes 0xFFFF."""
     if mask & _abi.OUT_RAW_COST_U16:
         rc = arrs["raw_cost"]
-        assert (rc[rc != 0xFFFFFFFF] <= 0xFFFF).all(), "raw_cost_u16 requested for costs that do not fit"
+        assert (rc[rc != 0xFFFFFFFF] < 0xFFFF).all(), "raw_cost_u16 requested for costs that do not fit below 0xFFFF"
         arrs["raw_cost_u16"] = rc.astype(np.uint16)
         if not had_raw:
             del arrs["raw_cost"]

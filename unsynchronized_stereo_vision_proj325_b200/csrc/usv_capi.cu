@@ -16,6 +16,7 @@
 
 namespace usv {
 cudaError_t launch_direct(const DevJob& J, int n_pairs, cudaStream_t st);
+bool direct_supported(const DevJob& J);
 // returns cudaErrorNotSupported when the dense kernels do not cover the job
 size_t dense_scratch_bytes_per_pair(const DevJob& J);
 cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
@@ -159,10 +160,19 @@ static int check_common(usv_ctx* ctx, const usv_frame_desc* f, const usv_search_
   return USV_OK;
 }
 
-// raw_cost_u16 is lossless or refused: every SAD of the template must fit 16 bits
+// raw_cost_u16 is lossless or refused: every SAD of the template must fit 16 bits below 0xFFFF, the "no candidate" value
 static int check_cost_u16(usv_ctx* ctx, const usv_frame_desc* f, const usv_search_params* p) {
-  if (p->cost_kind != USV_COST_SAD || 255ll * p->tmpl_w * p->tmpl_h * f->channels > 0xFFFFll)
-    return fail(ctx, USV_ERR_UNSUPPORTED, "raw_cost_u16 needs SAD with 255*tmpl_w*tmpl_h*channels <= 65535");
+  if (p->cost_kind != USV_COST_SAD || 255ll * p->tmpl_w * p->tmpl_h * f->channels >= 0xFFFFll)
+    return fail(ctx, USV_ERR_UNSUPPORTED, "raw_cost_u16 needs SAD with 255*tmpl_w*tmpl_h*channels < 65535");
+  return USV_OK;
+}
+
+// only the direct form serves sparse lists and whatever the dense sweeps do not cover; some narrow, tall templates do not
+// fit its shared memory
+static int check_direct(usv_ctx* ctx, const DevJob& J) {
+  if (!usv::direct_supported(J))
+    return fail(ctx, USV_ERR_UNSUPPORTED, "template %dx%dx%d: no kernel serves this shape (direct form: shared memory)", J.tw, J.th,
+                J.channels);
   return USV_OK;
 }
 
@@ -351,6 +361,7 @@ static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, bool s
       (void)cudaGetLastError();
     }
   }
+  if ((rc = check_direct(ctx, J))) return rc;
   cudaError_t e = usv::launch_direct(J, n_pairs, st);
   if (e != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "direct launch: %s", cudaGetErrorString(e));
   ctx->launches++;
@@ -489,6 +500,9 @@ static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_righ
         return fail(ctx, USV_ERR_INVALID_ARG, "template %d at (%d,%d) outside the frame", i, h_tx[i], h_ty[i]);
     n_win = n_templates;
     if (n_templates == 0) return USV_OK;
+    DevJob J;
+    fill_job(ctx, J, nullptr, nullptr, f, p, nullptr);
+    if ((rc = check_direct(ctx, J))) return rc;
   } else {
     int32_t nx, ny;
     if (usv_grid_dims(f, p, &nx, &ny, nullptr)) return fail(ctx, USV_ERR_INVALID_ARG, "bad geometry");

@@ -256,26 +256,44 @@ block_cost_argmin_direct(const DevJob J, int tmpl_pitch_words, int strip_pitch_w
 }
 
 // ---- host-side launcher ----------------------------------------------------
-template <int KIND>
-static cudaError_t launch_direct_c(const DevJob& J, int n_pairs, cudaStream_t st) {
+struct DirectLayout {
+  int tmpl_pitch_words, strip_pitch_words, rows;
+  size_t smem;  // 0: the job does not fit the shared memory of one CTA
+};
+
+static DirectLayout direct_layout(const DevJob& J) {
+  DirectLayout d;
   const int nw = (J.row_bytes + 3) / 4;
   // odd pitch in words avoids bank conflicts; the whole template area is padded to 16 B so the
   // strip area that follows it stays cp.async (16-byte) aligned
-  const int tmpl_pitch_words = nw + 1;
+  d.tmpl_pitch_words = nw + 1;
   // widest strip a pass can need: (chunk candidates + template) bytes + alignment slack
   int max_c = J.nxc < kChunkCands ? J.nxc : kChunkCands;
   int strip_bytes = ((max_c + J.tw) * J.channels + 47) & ~15;
-  int strip_pitch_words = strip_bytes / 4 + 4;  // +16 B slack: the funnel shift reads one word ahead
+  d.strip_pitch_words = strip_bytes / 4 + 4;  // +16 B slack: the funnel shift reads one word ahead
   // the template's aligned staging copy temporarily lives in the strip area
-  int tmpl_stage_bytes = J.th * (((J.row_bytes + 15 + 16) & ~15) + 16);
-  int rows = kStripBudget / (strip_pitch_words * 4);
-  if (rows < 1) return cudaErrorInvalidValue;
-  if (rows > J.th) rows = J.th;
-  size_t strip_area = (size_t)rows * strip_pitch_words * 4;
-  if (strip_area < (size_t)tmpl_stage_bytes) strip_area = tmpl_stage_bytes;
-  size_t smem = ((((size_t)J.th * tmpl_pitch_words + 3) & ~(size_t)3) * 4) + strip_area;
+  size_t tmpl_stage_bytes = (size_t)J.th * (((J.row_bytes + 15 + 16) & ~15) + 16);
+  d.rows = kStripBudget / (d.strip_pitch_words * 4);
+  d.smem = 0;
+  if (d.rows < 1) return d;
+  if (d.rows > J.th) d.rows = J.th;
+  size_t strip_area = (size_t)d.rows * d.strip_pitch_words * 4;
+  if (strip_area < tmpl_stage_bytes) strip_area = tmpl_stage_bytes;
+  size_t smem = ((((size_t)J.th * d.tmpl_pitch_words + 3) & ~(size_t)3) * 4) + strip_area;
   smem = (smem + 15) & ~(size_t)15;
-  if (smem > 200 * 1024) return cudaErrorInvalidValue;
+  if (smem <= 200 * 1024) d.smem = smem;
+  return d;
+}
+
+// the whole template and one strip chunk must fit one CTA's shared memory (narrow, tall templates may not)
+bool direct_supported(const DevJob& J) { return direct_layout(J).smem != 0; }
+
+template <int KIND>
+static cudaError_t launch_direct_c(const DevJob& J, int n_pairs, cudaStream_t st) {
+  const DirectLayout d = direct_layout(J);
+  if (d.smem == 0) return cudaErrorInvalidValue;
+  const size_t smem = d.smem;
+  const int tmpl_pitch_words = d.tmpl_pitch_words, strip_pitch_words = d.strip_pitch_words, rows = d.rows;
   dim3 grid(J.n_templates, n_pairs), block(kDirectThreads);
 #define USV_LAUNCH_C(CC)                                                                              \
   {                                                                                                   \
