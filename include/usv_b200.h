@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define USV_ABI_VERSION 3
+#define USV_ABI_VERSION 4
 
 /* ---- status codes ------------------------------------------------------ */
 #define USV_OK 0
@@ -64,6 +64,7 @@ extern "C" {
 
 #define USV_NO_MATCH 0xFFFFFFFFu /* RightIndex of a window with no accepted candidate */
 #define USV_NO_DISPARITY 0xFFFFu
+#define USV_NO_SUBPIXEL (-2147483647 - 1) /* INT32_MIN: window without a refined disparity */
 
 /* ---- records ----------------------------------------------------------- */
 
@@ -182,6 +183,38 @@ int usv_match_dense_host(usv_ctx *ctx, const uint8_t *h_left,
                          const uint8_t *h_right, const usv_frame_desc *frame,
                          int32_t n_pairs, const usv_search_params *params,
                          const usv_outputs *h_out);
+
+/* ---- sub-pixel disparity of the dense sweep's winners, 1/16 px ---------------
+ * Input per window of the dense grid (layout [pair][iy*nx + ix], as usv_outputs): the RightIndex r the sweep wrote.
+ * Output per window: disparity_x16 (int32, 1/16 px) and distance (f64, cm, from the refined disparity).
+ *   - r == USV_NO_MATCH, or r not a candidate of its window (r / nxc != y, or x* = r % nxc outside the window's clipped
+ *     candidate range): disparity_x16 = USV_NO_SUBPIXEL, distance = 0.0; no frame byte is read for it.
+ *   - c(x') = the candidate's cost in the sweep's terms: SAD / SSD the exact integer cost, NCC / ZNCC MatchValue =
+ *     1 - score. Refined only when x*-1 and x*+1 are both candidates of the window (in the frame and in
+ *     [search_min, search_max]); otherwise q = 0.
+ *   - SAD / SSD, int64: num = c(x*-1) - c(x*+1), den = c(x*-1) + c(x*+1) - 2 c(x*);
+ *     den > 0: q = sgn(num) * floor((16 |num| + den) / (2 den)), clamped to [-8, 8]; else q = 0.
+ *   - NCC / ZNCC, f64, every operation correctly rounded: num = v- - v+, den = (v- - v0) + (v+ - v0);
+ *     den > 0: q = round(8 num / den) (half away from zero), clamped to [-8, 8]; else q = 0.
+ *   - disparity_x16 = 16 d - q (USV_LEFT_CAM, d = x - x*) or 16 d + q (USV_RIGHT_CAM, d = x* - x): the parabola's
+ *     vertex in 1/16 px, rounded half away from zero. distance = distance_kind's formula at disparity_x16 / 16.0.
+ * For the sweep's own winners den > 0 always (the first minimum in ascending x' has c(x*-1) > c(x*) <= c(x*+1)); a tie
+ * c(x*+1) == c(x*) gives q = +8, the midpoint of the tied pair. The other outputs (distance, disparity_u16, matches,
+ * resolved_disparity_u16) keep the integer disparity. To combine with the resolved map, take disparity_x16 where
+ * resolved_disparity_u16 != USV_NO_DISPARITY. Frames wider than 2^26 pixels are refused (USV_ERR_UNSUPPORTED).
+ * At least one of the two output pointers must be non-NULL. */
+/* Device pointers (frames as usv_match_dense_device), enqueued on cuda_stream. */
+int usv_refine_subpixel_device(usv_ctx *ctx, const uint8_t *d_left, const uint8_t *d_right,
+                               const usv_frame_desc *frame, int32_t n_pairs,
+                               const usv_search_params *params, const uint32_t *d_right_index,
+                               int32_t *d_disparity_x16, double *d_distance, void *cuda_stream);
+/* Host buffers: the dense sweep into h_out (byte for byte what usv_match_dense_host returns; h_out may be NULL or all
+ * NULL, RightIndex then stays on the device), the refinement of its winners, D2H and a final synchronise.
+ * usv_last_kernel names the sweep's kernel. */
+int usv_match_dense_subpixel_host(usv_ctx *ctx, const uint8_t *h_left, const uint8_t *h_right,
+                                  const usv_frame_desc *frame, int32_t n_pairs,
+                                  const usv_search_params *params, const usv_outputs *h_out,
+                                  int32_t *h_disparity_x16, double *h_distance);
 
 /* ---- sparse templates: explicit (x, y) list, shared by all pairs -------- */
 /* cost_rows (optional): [n_pairs][n_templates][row_cap] u32 costs of every

@@ -3,7 +3,7 @@ import ctypes as C
 
 import numpy as np
 
-USV_ABI_VERSION = 3
+USV_ABI_VERSION = 4
 USV_OK, USV_ERR_INVALID_ARG, USV_ERR_CUDA, USV_ERR_NO_DEVICE, USV_ERR_UNSUPPORTED, USV_ERR_NOMEM = 0, -1, -2, -3, -4, -5
 COST_SAD, COST_SSD, COST_NCC, COST_ZNCC = 0, 1, 2, 3
 COST_NAMES = {"sad": COST_SAD, "ssd": COST_SSD, "ncc": COST_NCC, "zncc": COST_ZNCC}
@@ -11,6 +11,7 @@ DIST_NONE, DIST_PINHOLE, DIST_POWERLAW = 0, 1, 2
 LEFT_CAM, RIGHT_CAM = 1, 0
 NO_MATCH = 0xFFFFFFFF
 NO_DISPARITY = 0xFFFF
+NO_SUBPIXEL = -2**31  # disparity_x16 of a window without a refined disparity (INT32_MIN)
 
 OUT_MATCHES, OUT_RIGHT_INDEX, OUT_RAW_COST, OUT_SCORE = 0x01, 0x02, 0x04, 0x08
 OUT_DISTANCE, OUT_DISTANCE_F32, OUT_DISPARITY_U16, OUT_RAW_COST_U16 = 0x10, 0x20, 0x40, 0x80

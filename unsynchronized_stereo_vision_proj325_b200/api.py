@@ -26,6 +26,7 @@ EXPORTS = (
     "usv_stream_wait", "usv_host_register", "usv_host_unregister",
     "usv_stream_bytes_per_pair", "usv_probe_issue_rate", "usv_match_contours",
     "usv_resolve_match_list", "usv_resolve_match_list_device", "usv_id_matcher", "usv_preprocess_device", "usv_preprocess_host",
+    "usv_refine_subpixel_device", "usv_match_dense_subpixel_host",
 )
 
 
@@ -164,6 +165,23 @@ class Context:
         self._check(rc, "usv_match_dense_host")
         return {k: v.reshape(n, ny * nx) for k, v in arrs.items()}
 
+    def match_dense_subpixel(self, left, right, params, mask=ALL_OUTPUTS):
+        """match_dense plus the sub-pixel refinement of its winners (usv_match_dense_subpixel_host): the same dict, plus
+        "disparity_x16" (int32, 1/16 px, NO_SUBPIXEL where there is none) and "subpixel_distance" (f64, cm, from the
+        refined disparity), each [n, ny*nx]."""
+        assert left.shape == right.shape and left.strides == right.strides
+        f = _abi.frame_desc_for(left)
+        nx, ny, _ = grid_dims(f, params)
+        n = left.shape[0]
+        arrs, st = _alloc_host_outputs(n * nx * ny, mask)
+        x16 = np.zeros(n * nx * ny, np.int32)
+        dist = np.zeros(n * nx * ny, np.float64)
+        rc = lib().usv_match_dense_subpixel_host(self._h, _ptr(left), _ptr(right), C.byref(f), C.c_int32(n), C.byref(params),
+                                                 C.byref(st), _ptr(x16), _ptr(dist))
+        self._check(rc, "usv_match_dense_subpixel_host")
+        arrs["disparity_x16"], arrs["subpixel_distance"] = x16, dist
+        return {k: v.reshape(n, ny * nx) for k, v in arrs.items()}
+
     def match_templates(self, left, right, tx, ty, params, mask=ALL_OUTPUTS, rows=False):
         assert left.shape == right.shape and left.strides == right.strides
         f = _abi.frame_desc_for(left)
@@ -213,6 +231,14 @@ class Context:
                                               _ptr(d_ty), C.c_int32(n_templates), C.byref(params), C.byref(d_out), _ptr(d_cost_rows),
                                               _ptr(d_score_rows), C.c_int32(row_cap), C.c_void_p(int(stream)))
         self._check(rc, "usv_match_templates_device")
+
+    def refine_subpixel_device(self, d_left, d_right, frame, n_pairs, params, d_right_index, d_disparity_x16, d_distance=None,
+                               stream=0):
+        """Sub-pixel refinement of dense winners, raw device pointers (ints); asynchronous on `stream`."""
+        rc = lib().usv_refine_subpixel_device(self._h, _ptr(d_left), _ptr(d_right), C.byref(frame), C.c_int32(n_pairs),
+                                              C.byref(params), _ptr(d_right_index), _ptr(d_disparity_x16), _ptr(d_distance),
+                                              C.c_void_p(int(stream)))
+        self._check(rc, "usv_refine_subpixel_device")
 
     # ---- distance family --------------------------------------------------------
     def disparity_to_distance(self, disp, kind):

@@ -14,7 +14,7 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["--threads", "0", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-ccbin", "/usr/bin/g++"]
 
-LIB_SOURCES = ["usv_capi.cu", "usv_direct.cu", "usv_dense.cu", "usv_dense_g8.cu", "usv_dense_colour.cu", "usv_distance.cu", "usv_probe.cu", "usv_contours.cu", "usv_resolve.cu", "usv_resolve_rows.cu", "usv_preprocess.cu", "usv_dense_corr.cu", "usv_dense_mma.cu", "usv_dense_umma.cu"]
+LIB_SOURCES = ["usv_capi.cu", "usv_direct.cu", "usv_dense.cu", "usv_dense_g8.cu", "usv_dense_colour.cu", "usv_distance.cu", "usv_probe.cu", "usv_contours.cu", "usv_resolve.cu", "usv_resolve_rows.cu", "usv_preprocess.cu", "usv_dense_corr.cu", "usv_dense_mma.cu", "usv_dense_umma.cu", "usv_subpixel.cu"]
 HOST_SOURCES = ["host/Match.cpp", "host/SearchAlgorithms.cpp", "host/DistanceCalculator.cpp"]
 
 

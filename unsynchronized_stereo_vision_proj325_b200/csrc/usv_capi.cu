@@ -56,6 +56,8 @@ cudaError_t launch_moving_object_distance(int camera_side, long long t_this, con
                                           const int* idx3, int n_idx, long long t_other, long long t_old, long long t_older,
                                           double* out, cudaStream_t st);
 cudaError_t launch_coordinate_position(int camera_side, const double* dist, const float* xy, long long n, double* xyz, cudaStream_t st);
+cudaError_t launch_subpixel_refine(const DevJob& J, int n_pairs, const uint32_t* d_right_index, int* d_x16, double* d_dist,
+                                   cudaStream_t st);
 }  // namespace usv
 
 namespace usv { int g_sm_count = 148; }
@@ -89,6 +91,7 @@ struct usv_ctx {
   size_t pin_cap[3] = {0, 0, 0};  // usv_destroy refuses while a usv_stream of this context is alive
   // grow-only scratch for the host paths
   DevBuf in_l, in_r, tx, ty, rows_u32, rows_f64, out[9], misc[8], resolve_ws, pre_ws, corr_ws, win_ws;
+  DevBuf sub_ri, sub_x16, sub_dist;  // usv_match_dense_subpixel_host: winners' RightIndex, refined disparity, distance
 };
 
 static const int kNumOut = 9;
@@ -273,6 +276,7 @@ extern "C" int usv_destroy(usv_ctx* ctx) {
   if (ctx->pre_ws.p) cudaFree(ctx->pre_ws.p);
   if (ctx->corr_ws.p) cudaFree(ctx->corr_ws.p);
   if (ctx->win_ws.p) cudaFree(ctx->win_ws.p);
+  for (DevBuf* b : {&ctx->sub_ri, &ctx->sub_x16, &ctx->sub_dist}) if (b->p) cudaFree(b->p);
   for (double* l : ctx->lut) if (l) cudaFree(l);
   for (void* l : ctx->retired) cudaFree(l);
   if (ctx->h_status) cudaFreeHost(ctx->h_status);
@@ -462,7 +466,46 @@ extern "C" int usv_match_templates_device(usv_ctx* ctx, const uint8_t* d_left, c
                       row_cap, (cudaStream_t)cuda_stream);
 }
 
+// ---- sub-pixel refinement of dense winners (usv_subpixel.cu) --------------------------
+static int check_subpixel(usv_ctx* ctx, const usv_frame_desc* f, const void* x16, const void* dist) {
+  if (!x16 && !dist) return fail(ctx, USV_ERR_INVALID_ARG, "sub-pixel refinement: both output pointers are NULL");
+  // 16 * d must fit int32
+  if (f->width > (1 << 26)) return fail(ctx, USV_ERR_UNSUPPORTED, "sub-pixel refinement: frame wider than 2^26 pixels");
+  return USV_OK;
+}
+
+static int refine_device(usv_ctx* ctx, const uint8_t* d_left, const uint8_t* d_right, const usv_frame_desc* f, int32_t n_pairs,
+                         const usv_search_params* p, const uint32_t* d_ri, int32_t* d_x16, double* d_dist, cudaStream_t st) {
+  int rc = check_common(ctx, f, p, n_pairs);
+  if (rc || (rc = check_subpixel(ctx, f, d_x16, d_dist))) return rc;
+  if (!d_left || !d_right || !d_ri) return fail(ctx, USV_ERR_INVALID_ARG, "null device pointer");
+  if (!aligned16(d_left) || !aligned16(d_right) || (f->row_stride & 15) || (f->frame_stride & 15))
+    return fail(ctx, USV_ERR_INVALID_ARG, "device frames need 16-byte aligned base, row_stride and frame_stride");
+  if (n_pairs == 0) return USV_OK;
+  CU(cudaSetDevice(ctx->device));
+  DevJob J;
+  fill_job(ctx, J, d_left, d_right, f, p, nullptr);
+  cudaError_t e = usv::launch_subpixel_refine(J, n_pairs, d_ri, d_x16, d_dist, st);
+  if (e != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "sub-pixel launch: %s", cudaGetErrorString(e));
+  ctx->launches++;
+  return USV_OK;
+}
+
+extern "C" int usv_refine_subpixel_device(usv_ctx* ctx, const uint8_t* d_left, const uint8_t* d_right, const usv_frame_desc* frame,
+                                          int32_t n_pairs, const usv_search_params* params, const uint32_t* d_right_index,
+                                          int32_t* d_disparity_x16, double* d_distance, void* cuda_stream) {
+  if (!ctx) return USV_ERR_INVALID_ARG;
+  return refine_device(ctx, d_left, d_right, frame, n_pairs, params, d_right_index, d_disparity_x16, d_distance,
+                       (cudaStream_t)cuda_stream);
+}
+
 // ---- matching: host pointers (H2D + kernels + D2H + sync inside) --------------------
+// optional step after the dense sweep of match_host: refine its winners into these host arrays (either may be NULL)
+struct SubpixelOut {
+  int32_t* disparity_x16;
+  double* distance;
+};
+
 static int upload_frames(usv_ctx* ctx, DevBuf& dst, const uint8_t* h, const usv_frame_desc* f, int n_pairs, usv_frame_desc* df,
                          cudaStream_t st) {
   const int row_bytes = f->width * f->channels;
@@ -483,10 +526,12 @@ static int upload_frames(usv_ctx* ctx, DevBuf& dst, const uint8_t* h, const usv_
 
 static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_right, const usv_frame_desc* f, int32_t n_pairs,
                       const usv_search_params* p, const usv_outputs* h_out, const int32_t* h_tx, const int32_t* h_ty,
-                      int32_t n_templates, uint32_t* h_cost_rows, double* h_score_rows, int32_t row_cap) {
+                      int32_t n_templates, uint32_t* h_cost_rows, double* h_score_rows, int32_t row_cap,
+                      const SubpixelOut* sub = nullptr) {
   int rc = check_common(ctx, f, p, n_pairs);
   if (rc) return rc;
   if (!h_left || !h_right || !h_out) return fail(ctx, USV_ERR_INVALID_ARG, "null host pointer");
+  if (sub && (rc = check_subpixel(ctx, f, sub->disparity_x16, sub->distance))) return rc;
   if (n_pairs == 0) return USV_OK;
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
@@ -541,9 +586,31 @@ static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_righ
       CU(cudaMemcpyAsync(d_srows, h_score_rows, sizeof(double) * n_res * row_cap, cudaMemcpyHostToDevice, st));
     }
   }
+  // the refinement reads the winners' RightIndex: the caller's array when it was asked for, scratch otherwise
+  if (sub && !d_out.right_index) {
+    if ((rc = grow(ctx, ctx->sub_ri, 4 * n_res))) return rc;
+    d_out.right_index = (uint32_t*)ctx->sub_ri.p;
+  }
   rc = match_device(ctx, (const uint8_t*)ctx->in_l.p, (const uint8_t*)ctx->in_r.p, &df, n_pairs, p, &d_out, d_tx, d_ty, n_templates,
                     d_rows, d_srows, row_cap, st);
   if (rc) return rc;
+  if (sub) {
+    int32_t* d_x16 = nullptr;
+    double* d_dist = nullptr;
+    if (sub->disparity_x16) {
+      if ((rc = grow(ctx, ctx->sub_x16, 4 * n_res))) return rc;
+      d_x16 = (int32_t*)ctx->sub_x16.p;
+    }
+    if (sub->distance) {
+      if ((rc = grow(ctx, ctx->sub_dist, 8 * n_res))) return rc;
+      d_dist = (double*)ctx->sub_dist.p;
+    }
+    if ((rc = refine_device(ctx, (const uint8_t*)ctx->in_l.p, (const uint8_t*)ctx->in_r.p, &df, n_pairs, p, d_out.right_index, d_x16,
+                            d_dist, st)))
+      return rc;
+    if (d_x16) CU(cudaMemcpyAsync(sub->disparity_x16, d_x16, 4 * n_res, cudaMemcpyDeviceToHost, st));
+    if (d_dist) CU(cudaMemcpyAsync(sub->distance, d_dist, 8 * n_res, cudaMemcpyDeviceToHost, st));
+  }
   for (int i = 0; i < kNumOut; ++i)
     if (*out_slot(&ho, i)) CU(cudaMemcpyAsync(*out_slot(&ho, i), ctx->out[i].p, kOutElem[i] * n_res, cudaMemcpyDeviceToHost, st));
   if (d_rows) CU(cudaMemcpyAsync(h_cost_rows, d_rows, sizeof(uint32_t) * n_res * row_cap, cudaMemcpyDeviceToHost, st));
@@ -565,6 +632,16 @@ extern "C" int usv_match_templates_host(usv_ctx* ctx, const uint8_t* h_left, con
   if (!ctx) return USV_ERR_INVALID_ARG;
   if (!h_tx) return fail(ctx, USV_ERR_INVALID_ARG, "null template list");
   return match_host(ctx, h_left, h_right, frame, n_pairs, params, h_out, h_tx, h_ty, n_templates, h_cost_rows, h_score_rows, row_cap);
+}
+
+extern "C" int usv_match_dense_subpixel_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_right, const usv_frame_desc* frame,
+                                             int32_t n_pairs, const usv_search_params* params, const usv_outputs* h_out,
+                                             int32_t* h_disparity_x16, double* h_distance) {
+  if (!ctx) return USV_ERR_INVALID_ARG;
+  usv_outputs none;
+  memset(&none, 0, sizeof(none));
+  const SubpixelOut sub = {h_disparity_x16, h_distance};
+  return match_host(ctx, h_left, h_right, frame, n_pairs, params, h_out ? h_out : &none, nullptr, nullptr, 0, nullptr, nullptr, 0, &sub);
 }
 
 // ---- distance family ------------------------------------------------------------------

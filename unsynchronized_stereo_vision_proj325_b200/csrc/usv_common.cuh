@@ -67,6 +67,16 @@ __device__ inline double distance_from_disparity(int disp, int kind) {
   }
   return 0.0;
 }
+// The same formulas at a fractional disparity (the sub-pixel pass, usv_subpixel.cu). Kept apart from the int overload,
+// whose results the integer-disparity outputs pin bit for bit.
+__device__ inline double distance_from_disparity(double disp, int kind) {
+  if (kind == USV_DIST_PINHOLE) {
+    return __ddiv_rn(__ddiv_rn(201.6 * 4, __dmul_rn(disp, 0.000043)), 1000.0);
+  } else if (kind == USV_DIST_POWERLAW) {
+    return pow(__ddiv_rn(__dmul_rn(10760.0, pow(disp, -0.877)), 3.0752), (1 / 0.7791));
+  }
+  return 0.0;
+}
 
 // Correlation score from exact integer window sums; same formula and operation
 // order as oracle/block_search_oracle.c:score_from_sums (IEEE f64, no FMA).
