@@ -9,6 +9,8 @@
 #include <cstdio>
 #include <algorithm>
 #include <cstring>
+#include <initializer_list>
+#include <memory>
 #include <new>
 #include <vector>
 
@@ -64,10 +66,36 @@ namespace usv { int g_sm_count = 148; }
 
 using usv::DevJob;
 
-struct DevBuf {
+// Device memory, or pinned host memory when kPinned, that frees itself. Whoever destroys one has set its device and
+// synchronised every stream that may still use it.
+template <bool kPinned>
+struct Buf {
   void* p = nullptr;
   size_t cap = 0;
+  Buf() = default;
+  Buf(const Buf&) = delete;
+  Buf& operator=(const Buf&) = delete;
+  Buf(Buf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  ~Buf() { release(); }
+  cudaError_t release() {
+    const cudaError_t e = !p ? cudaSuccess : kPinned ? cudaFreeHost(p) : cudaFree(p);
+    p = nullptr;
+    cap = 0;
+    return e;
+  }
+  // exactly `bytes` into an empty buffer; host_flags are the cudaHostAlloc flags of pinned memory
+  cudaError_t alloc(size_t bytes, unsigned host_flags = cudaHostAllocDefault) {
+    const cudaError_t e = kPinned ? cudaHostAlloc(&p, bytes, host_flags) : cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) cap = bytes;
+    else p = nullptr;
+    return e;
+  }
 };
+using DevBuf = Buf<false>;
+using PinnedBuf = Buf<true>;
+
+static const int kNumOut = 9;
+static const size_t kOutElem[kNumOut] = {sizeof(usv_match), 4, 4, 8, 8, 4, 2, 2, 2};
 
 struct usv_ctx {
   int device = 0;
@@ -77,25 +105,21 @@ struct usv_ctx {
   const char* last_kernel = "none";
   // distance LUT cache (by kind), [lut_n] doubles. Grow-only: a LUT that is replaced by a longer one stays allocated
   // until usv_destroy (kernels in flight on other streams of this context may still read it)
-  double* lut[3] = {nullptr, nullptr, nullptr};
+  DevBuf lut[3];
   int lut_n[3] = {0, 0, 0};
-  std::vector<void*> retired;
+  std::vector<DevBuf> retired;
   // status word the kernels can raise (mapped pinned host memory: readable by the host without a copy)
-  int* h_status = nullptr;
+  PinnedBuf status;
   int* d_status = nullptr;
-  int sm_count = 148;
   int corr_kernel = USV_CORR_KERNEL_AUTO;
-  std::atomic<int> open_streams{0};
+  std::atomic<int> open_streams{0};  // usv_destroy refuses while a usv_stream of this context is alive
   // grow-only pinned staging of usv_block_search_host (frames in, match list + distances out)
-  void* pin[3] = {nullptr, nullptr, nullptr};
-  size_t pin_cap[3] = {0, 0, 0};  // usv_destroy refuses while a usv_stream of this context is alive
+  PinnedBuf pin[3];
   // grow-only scratch for the host paths
-  DevBuf in_l, in_r, tx, ty, rows_u32, rows_f64, out[9], misc[8], resolve_ws, pre_ws, corr_ws, win_ws;
+  DevBuf in_l, in_r, tx, ty, rows_u32, rows_f64, out[kNumOut], misc[8], resolve_ws, pre_ws, corr_ws, win_ws;
   DevBuf sub_ri, sub_x16, sub_dist;  // usv_match_dense_subpixel_host: winners' RightIndex, refined disparity, distance
+  ~usv_ctx() { if (stream) cudaStreamDestroy(stream); }
 };
-
-static const int kNumOut = 9;
-static const size_t kOutElem[kNumOut] = {sizeof(usv_match), 4, 4, 8, 8, 4, 2, 2, 2};
 
 static int fail(usv_ctx* c, int code, const char* fmt, ...) {
   if (c) {
@@ -112,14 +136,66 @@ static int fail(usv_ctx* c, int code, const char* fmt, ...) {
     if (e_ != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "%s: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
   } while (0)
 
-static int grow(usv_ctx* ctx, DevBuf& b, size_t bytes) {
+template <bool kPinned>
+static int grow(usv_ctx* ctx, Buf<kPinned>& b, size_t bytes) {
   if (bytes <= b.cap) return USV_OK;
-  if (b.p) CU(cudaFree(b.p));
-  b.p = nullptr; b.cap = 0;
-  size_t want = bytes + bytes / 4 + 256;
-  cudaError_t e = cudaMalloc(&b.p, want);
-  if (e != cudaSuccess) return fail(ctx, USV_ERR_NOMEM, "cudaMalloc(%zu): %s", want, cudaGetErrorString(e));
-  b.cap = want;
+  CU(b.release());
+  const size_t want = bytes + bytes / 4 + (kPinned ? 4096 : 256);
+  const cudaError_t e = b.alloc(want);
+  if (e != cudaSuccess)
+    return fail(ctx, USV_ERR_NOMEM, "%s(%zu): %s", kPinned ? "cudaHostAlloc" : "cudaMalloc", want, cudaGetErrorString(e));
+  return USV_OK;
+}
+
+// pair scratch of a dense sweep: room for every pair up to this cap (at least one pair); the sweeps run the pairs in
+// chunks of what it holds
+static const size_t kPairScratchCap = (size_t)3 << 29;  // 1.5 GB
+
+static int grow_pair_scratch(usv_ctx* ctx, DevBuf& ws, size_t per_pair, int32_t n_pairs) {
+  size_t want = per_pair * (size_t)n_pairs;
+  if (want > kPairScratchCap) want = std::max(per_pair, kPairScratchCap / per_pair * per_pair);
+  return grow(ctx, ws, want);
+}
+
+// every array of `arrs` that is null (not asked for by the caller) is pointed at its share of scratch `ws`
+struct ArrayOrScratch {
+  void** arr;
+  size_t bytes;
+};
+static int or_scratch(usv_ctx* ctx, DevBuf& ws, std::initializer_list<ArrayOrScratch> arrs) {
+  size_t total = 0;
+  for (const ArrayOrScratch& a : arrs) total += *a.arr ? 0 : a.bytes;
+  const int rc = grow(ctx, ws, total);
+  if (rc) return rc;
+  uint8_t* q = (uint8_t*)ws.p;
+  for (const ArrayOrScratch& a : arrs)
+    if (!*a.arr) { *a.arr = q; q += a.bytes; }
+  return USV_OK;
+}
+
+// device layout of host frames: rows at a 128-byte pitch, frames packed
+static usv_frame_desc device_frame_desc(const usv_frame_desc* f) {
+  usv_frame_desc d = *f;
+  d.row_stride = (f->width * f->channels + 127) & ~127;
+  d.frame_stride = (int64_t)d.row_stride * f->height;
+  return d;
+}
+
+// H2D of `n` consecutive host frames (layout `hf`) into consecutive device frames (layout `df`) from `dst` on: one copy
+// when the layouts agree, one 2D copy when the host frames are packed, one 2D copy per frame otherwise
+static int copy_frames(usv_ctx* ctx, uint8_t* dst, const usv_frame_desc& df, const uint8_t* src, const usv_frame_desc* hf, int32_t n,
+                       cudaStream_t st) {
+  const int row_bytes = hf->width * hf->channels;
+  const bool packed = n == 1 || hf->frame_stride == (int64_t)hf->row_stride * hf->height;
+  if (packed && hf->row_stride == df.row_stride) {
+    CU(cudaMemcpyAsync(dst, src, (size_t)df.frame_stride * n, cudaMemcpyHostToDevice, st));
+  } else if (packed) {
+    CU(cudaMemcpy2DAsync(dst, df.row_stride, src, hf->row_stride, row_bytes, (size_t)hf->height * n, cudaMemcpyHostToDevice, st));
+  } else {
+    for (int i = 0; i < n; ++i)
+      CU(cudaMemcpy2DAsync(dst + (size_t)i * df.frame_stride, df.row_stride, src + (size_t)i * hf->frame_stride, hf->row_stride,
+                           row_bytes, hf->height, cudaMemcpyHostToDevice, st));
+  }
   return USV_OK;
 }
 
@@ -181,9 +257,10 @@ static int check_direct(usv_ctx* ctx, const DevJob& J) {
 
 // a kernel gave up (today: a tcgen05 completion wait beyond its wall-clock bound): report it once, as an error
 static int check_dev_status(usv_ctx* ctx) {
-  if (ctx->h_status && *(volatile int*)ctx->h_status != 0) {
-    const int s = *(volatile int*)ctx->h_status;
-    *(volatile int*)ctx->h_status = 0;
+  volatile int* h_status = (volatile int*)ctx->status.p;
+  if (h_status && *h_status != 0) {
+    const int s = *h_status;
+    *h_status = 0;
     return fail(ctx, USV_ERR_CUDA, "device status %d: a kernel abandoned a wait (results of the affected call are invalid)", s);
   }
   return USV_OK;
@@ -214,15 +291,15 @@ static int ensure_lut(usv_ctx* ctx, int kind, int width, cudaStream_t st, const 
   if (kind == USV_DIST_NONE) return USV_OK;
   if (ctx->lut_n[kind] < width) {
     // (re)build on the device with the same device function the kernels use
-    if (ctx->lut[kind]) { ctx->retired.push_back(ctx->lut[kind]); ctx->lut[kind] = nullptr; ctx->lut_n[kind] = 0; }
+    if (ctx->lut[kind].p) { ctx->retired.push_back(std::move(ctx->lut[kind])); ctx->lut_n[kind] = 0; }
     int n = width < 4096 ? 4096 : width;
-    CU(cudaMalloc((void**)&ctx->lut[kind], sizeof(double) * n));
-    CU(usv::launch_build_distance_lut(ctx->lut[kind], n, kind, st));
+    CU(ctx->lut[kind].alloc(sizeof(double) * n));
+    CU(usv::launch_build_distance_lut((double*)ctx->lut[kind].p, n, kind, st));
     CU(cudaStreamSynchronize(st));  // one-time; other streams of this context may read it next
     ctx->launches++;
     ctx->lut_n[kind] = n;
   }
-  *lut = ctx->lut[kind];
+  *lut = (const double*)ctx->lut[kind].p;
   return USV_OK;
 }
 
@@ -247,17 +324,14 @@ extern "C" int usv_create(int device, usv_ctx** out) {
   usv_ctx* c = new (std::nothrow) usv_ctx();
   if (!c) return USV_ERR_NOMEM;
   c->device = device;
-  c->sm_count = prop.multiProcessorCount;
   usv::g_sm_count = prop.multiProcessorCount;
-  if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return USV_ERR_CUDA; }
-  if (cudaHostAlloc((void**)&c->h_status, sizeof(int), cudaHostAllocMapped) != cudaSuccess ||
-      cudaHostGetDevicePointer((void**)&c->d_status, c->h_status, 0) != cudaSuccess) {
-    if (c->h_status) cudaFreeHost(c->h_status);
-    cudaStreamDestroy(c->stream);
+  if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
+      c->status.alloc(sizeof(int), cudaHostAllocMapped) != cudaSuccess ||
+      cudaHostGetDevicePointer((void**)&c->d_status, c->status.p, 0) != cudaSuccess) {
     delete c;
     return USV_ERR_CUDA;
   }
-  *c->h_status = 0;
+  *(int*)c->status.p = 0;
   *out = c;
   return USV_OK;
 }
@@ -268,20 +342,6 @@ extern "C" int usv_destroy(usv_ctx* ctx) {
     return fail(ctx, USV_ERR_INVALID_ARG, "%d usv_stream(s) of this context are still open: destroy them first", ctx->open_streams.load());
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  DevBuf* bufs[] = {&ctx->in_l, &ctx->in_r, &ctx->tx, &ctx->ty, &ctx->rows_u32, &ctx->rows_f64};
-  for (DevBuf* b : bufs) if (b->p) cudaFree(b->p);
-  for (auto& b : ctx->out) if (b.p) cudaFree(b.p);
-  for (auto& b : ctx->misc) if (b.p) cudaFree(b.p);
-  if (ctx->resolve_ws.p) cudaFree(ctx->resolve_ws.p);
-  if (ctx->pre_ws.p) cudaFree(ctx->pre_ws.p);
-  if (ctx->corr_ws.p) cudaFree(ctx->corr_ws.p);
-  if (ctx->win_ws.p) cudaFree(ctx->win_ws.p);
-  for (DevBuf* b : {&ctx->sub_ri, &ctx->sub_x16, &ctx->sub_dist}) if (b->p) cudaFree(b->p);
-  for (double* l : ctx->lut) if (l) cudaFree(l);
-  for (void* l : ctx->retired) cudaFree(l);
-  if (ctx->h_status) cudaFreeHost(ctx->h_status);
-  for (void* q : ctx->pin) if (q) cudaFreeHost(q);
-  cudaStreamDestroy(ctx->stream);
   delete ctx;
   return USV_OK;
 }
@@ -327,18 +387,14 @@ static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, bool s
   if (!sparse) {
     const char* name = nullptr;
     int nl = 0;
-    // the scratch (colour planes here, planes + window statistics below) belongs to whoever owns the stream: launches on
-    // different streams must not share it
-    DevBuf& dws = corr_ws ? *corr_ws : ctx->corr_ws;
-    if (const size_t per_pair = (J.cost_kind == USV_COST_SAD && J.corr_kernel != USV_CORR_KERNEL_ALU) ? usv::dense_scratch_bytes_per_pair(J) : 0) {
-      const size_t cap = (size_t)3 << 29;  // 1.5 GB
-      size_t want = per_pair * (size_t)n_pairs;
-      if (want > cap) want = std::max(per_pair, cap / per_pair * per_pair);
-      if ((rc = grow(ctx, dws, want))) return rc;
-    }
+    // the scratch (colour planes of the SAD sweep, planes + window statistics of the correlation sweep) belongs to
+    // whoever owns the stream: launches on different streams must not share it
+    DevBuf& ws = corr_ws ? *corr_ws : ctx->corr_ws;
+    const bool sad_sweep = J.cost_kind == USV_COST_SAD && J.corr_kernel != USV_CORR_KERNEL_ALU;
+    if ((rc = grow_pair_scratch(ctx, ws, sad_sweep ? usv::dense_scratch_bytes_per_pair(J) : 0, n_pairs))) return rc;
     cudaError_t e = (J.cost_kind == USV_COST_SAD && J.channels == 3 && J.corr_kernel == USV_CORR_KERNEL_ALU)
                         ? cudaErrorNotSupported  // test / measurement aid: colour SAD on the ALU correlation kernel
-                        : usv::launch_dense(J, n_pairs, dws.p, dws.cap, st, &name, &nl);
+                        : usv::launch_dense(J, n_pairs, ws.p, ws.cap, st, &name, &nl);
     if (e == cudaSuccess) {
       ctx->launches += nl;
       ctx->last_kernel = name;
@@ -346,24 +402,16 @@ static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, bool s
     }
     if (e != cudaErrorNotSupported) return fail(ctx, USV_ERR_CUDA, "dense launch: %s", cudaGetErrorString(e));
     (void)cudaGetLastError();
-    {
-      // sliding-window correlation kernel: planes + window statistics live in a scratch buffer, pairs run in chunks
-      const size_t per_pair = usv::corr_scratch_bytes_per_pair(J, nullptr);
-      const size_t cap = (size_t)3 << 29;  // 1.5 GB
-      size_t want = per_pair * (size_t)n_pairs;
-      if (want > cap) want = std::max(per_pair, cap / per_pair * per_pair);
-      // the scratch belongs to whoever owns the stream: launches on different streams must not share it
-      DevBuf& ws = corr_ws ? *corr_ws : ctx->corr_ws;
-      if ((rc = grow(ctx, ws, want))) return rc;
-      e = usv::launch_dense_corr(J, n_pairs, ws.p, ws.cap, st, &name, &nl);
-      if (e == cudaSuccess) {
-        ctx->launches += nl;
-        ctx->last_kernel = name;
-        return USV_OK;
-      }
-      if (e != cudaErrorNotSupported) return fail(ctx, USV_ERR_CUDA, "dense correlation launch: %s", cudaGetErrorString(e));
-      (void)cudaGetLastError();
+    // sliding-window correlation kernel
+    if ((rc = grow_pair_scratch(ctx, ws, usv::corr_scratch_bytes_per_pair(J, nullptr), n_pairs))) return rc;
+    e = usv::launch_dense_corr(J, n_pairs, ws.p, ws.cap, st, &name, &nl);
+    if (e == cudaSuccess) {
+      ctx->launches += nl;
+      ctx->last_kernel = name;
+      return USV_OK;
     }
+    if (e != cudaErrorNotSupported) return fail(ctx, USV_ERR_CUDA, "dense correlation launch: %s", cudaGetErrorString(e));
+    (void)cudaGetLastError();
   }
   if ((rc = check_direct(ctx, J))) return rc;
   cudaError_t e = usv::launch_direct(J, n_pairs, st);
@@ -371,6 +419,19 @@ static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, bool s
   ctx->launches++;
   ctx->last_kernel = "block_cost_argmin_direct";
   return USV_OK;
+}
+
+// the arrays the resolved disparity map reads the winners from
+enum WinnerSrc { kWinDisparity, kWinRightIndex, kWinMatches };
+
+static WinnerSrc winner_src(const usv_search_params* p, const usv_outputs& o) {
+  if (p->cost_kind > USV_COST_SSD) return kWinMatches;  // the value of a correlation winner is an f64 score
+  // a u16 disparity names x' only when no candidate lies on the other side of the window (search_min >= 0): negative
+  // disparities are stored modulo 2^16 and -1 would read as USV_NO_DISPARITY; such ranges resolve from RightIndex
+  const bool disp_ok = p->search_min >= 0;
+  if (disp_ok && o.disparity_u16 && (o.raw_cost_u16 || o.raw_cost)) return kWinDisparity;
+  if (o.right_index && o.raw_cost) return kWinRightIndex;
+  return disp_ok ? kWinDisparity : kWinRightIndex;
 }
 
 static int match_device(usv_ctx* ctx, const uint8_t* d_left, const uint8_t* d_right, const usv_frame_desc* f, int32_t n_pairs,
@@ -400,48 +461,36 @@ static int match_device(usv_ctx* ctx, const uint8_t* d_left, const uint8_t* d_ri
     if (rc) return rc;
   }
   // resolved disparity map: ResolveMatchList over the winners on the device (usv_resolve_rows.cu). It reads the
-  // winners' RightIndex and value: the caller's arrays when they were asked for, scratch otherwise.
+  // winners from `src`: the caller's arrays when they were asked for, scratch otherwise.
   const bool want_resolved = d_out->resolved_disparity_u16 != nullptr;
+  const WinnerSrc src = winner_src(p, J.out);
   if (want_resolved) {
     if (sparse) return fail(ctx, USV_ERR_UNSUPPORTED, "resolved_disparity_u16 is an output of the dense sweep");
     if (!usv::resolve_rows_supported(J.nx, J.nxc)) return fail(ctx, USV_ERR_UNSUPPORTED, "resolved_disparity_u16: rows wider than 2048 windows");
-    const bool integer = p->cost_kind <= USV_COST_SSD;
     const size_t n_res = (size_t)J.n_templates * n_pairs;
-    // a u16 disparity names x' only when no candidate lies on the other side of the window (search_min >= 0): negative
-    // disparities are stored modulo 2^16 and -1 would read as USV_NO_DISPARITY; such ranges resolve from RightIndex
-    const bool disp_ok = p->search_min >= 0;
-    const bool have_int = integer && ((disp_ok && J.out.disparity_u16 && (J.out.raw_cost_u16 || J.out.raw_cost)) || (J.out.right_index && J.out.raw_cost));
-    if (!have_int && !(J.out.matches && !integer)) {
-      DevBuf& ws = win_ws ? *win_ws : ctx->win_ws;
-      if (integer && disp_ok) {  // disparity (2 B) + cost (4 B, or what the caller already asked for)
-        const bool need_cost = !J.out.raw_cost && !J.out.raw_cost_u16;
-        if ((rc = grow(ctx, ws, n_res * (need_cost ? 6 : 2) + 16))) return rc;
-        if (need_cost) J.out.raw_cost = (uint32_t*)ws.p;
-        if (!J.out.disparity_u16) J.out.disparity_u16 = (uint16_t*)((uint32_t*)ws.p + (need_cost ? n_res : 0));
-      } else if (integer) {      // RightIndex (4 B) + cost (4 B)
-        const bool need_cost = !J.out.raw_cost, need_ri = !J.out.right_index;
-        if ((rc = grow(ctx, ws, n_res * 4 * ((need_cost ? 1 : 0) + (need_ri ? 1 : 0)) + 16))) return rc;
-        if (need_cost) J.out.raw_cost = (uint32_t*)ws.p;
-        if (need_ri) J.out.right_index = (uint32_t*)ws.p + (need_cost ? n_res : 0);
-      } else {
-        if ((rc = grow(ctx, ws, n_res * sizeof(usv_match)))) return rc;
-        J.out.matches = (usv_match*)ws.p;
-      }
-    }
+    DevBuf& ws = win_ws ? *win_ws : ctx->win_ws;
+    usv_outputs& o = J.out;
+    if (src == kWinDisparity)  // either cost array serves; raw_cost is added when the caller asked for neither
+      rc = or_scratch(ctx, ws, {{o.raw_cost_u16 ? (void**)&o.raw_cost_u16 : (void**)&o.raw_cost, 4 * n_res},
+                                {(void**)&o.disparity_u16, 2 * n_res}});
+    else if (src == kWinRightIndex)
+      rc = or_scratch(ctx, ws, {{(void**)&o.raw_cost, 4 * n_res}, {(void**)&o.right_index, 4 * n_res}});
+    else
+      rc = or_scratch(ctx, ws, {{(void**)&o.matches, sizeof(usv_match) * n_res}});
+    if (rc) return rc;
   }
   if ((rc = dispatch_match(ctx, J, n_pairs, sparse, st, corr_ws))) return rc;
   if (want_resolved) {
-    const bool integer = p->cost_kind <= USV_COST_SSD;
     usv::ResolveRowsSrc S;
     memset(&S, 0, sizeof(S));
-    if (integer && p->search_min >= 0 && J.out.disparity_u16 && (J.out.raw_cost_u16 || J.out.raw_cost)) {
+    if (src == kWinDisparity) {
       S.disparity_u16 = J.out.disparity_u16; S.raw_cost_u16 = J.out.raw_cost_u16; S.raw_cost = J.out.raw_cost;
-    } else if (integer && J.out.right_index && J.out.raw_cost) {
+    } else if (src == kWinRightIndex) {
       S.right_index = J.out.right_index; S.raw_cost = J.out.raw_cost;
     } else {
       S.matches = J.out.matches;
     }
-    cudaError_t e = usv::launch_resolve_rows(S, S.matches == nullptr, J.nx, J.ny, J.sx, J.nxc, J.n_templates, J.camera_side, n_pairs,
+    cudaError_t e = usv::launch_resolve_rows(S, src != kWinMatches, J.nx, J.ny, J.sx, J.nxc, J.n_templates, J.camera_side, n_pairs,
                                              d_out->resolved_disparity_u16, st);
     if (e != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "resolve rows launch: %s", cudaGetErrorString(e));
     ctx->launches++;
@@ -506,24 +555,6 @@ struct SubpixelOut {
   double* distance;
 };
 
-static int upload_frames(usv_ctx* ctx, DevBuf& dst, const uint8_t* h, const usv_frame_desc* f, int n_pairs, usv_frame_desc* df,
-                         cudaStream_t st) {
-  const int row_bytes = f->width * f->channels;
-  const int pitch = (row_bytes + 127) & ~127;
-  df->width = f->width; df->height = f->height; df->channels = f->channels;
-  df->row_stride = pitch; df->frame_stride = (int64_t)pitch * f->height;
-  int rc = grow(ctx, dst, (size_t)df->frame_stride * n_pairs);
-  if (rc) return rc;
-  if (n_pairs == 1 || f->frame_stride == (int64_t)f->row_stride * f->height) {
-    CU(cudaMemcpy2DAsync(dst.p, pitch, h, f->row_stride, row_bytes, (size_t)f->height * n_pairs, cudaMemcpyHostToDevice, st));
-  } else {
-    for (int i = 0; i < n_pairs; ++i)
-      CU(cudaMemcpy2DAsync((uint8_t*)dst.p + (size_t)i * df->frame_stride, pitch, h + (size_t)i * f->frame_stride, f->row_stride,
-                           row_bytes, f->height, cudaMemcpyHostToDevice, st));
-  }
-  return USV_OK;
-}
-
 static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_right, const usv_frame_desc* f, int32_t n_pairs,
                       const usv_search_params* p, const usv_outputs* h_out, const int32_t* h_tx, const int32_t* h_ty,
                       int32_t n_templates, uint32_t* h_cost_rows, double* h_score_rows, int32_t row_cap,
@@ -554,9 +585,10 @@ static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_righ
     n_win = (int64_t)nx * ny;
   }
   const int64_t n_res = n_win * n_pairs;
-  usv_frame_desc df;
-  if ((rc = upload_frames(ctx, ctx->in_l, h_left, f, n_pairs, &df, st))) return rc;
-  if ((rc = upload_frames(ctx, ctx->in_r, h_right, f, n_pairs, &df, st))) return rc;
+  const usv_frame_desc df = device_frame_desc(f);
+  const size_t fbytes = (size_t)df.frame_stride * n_pairs;
+  if ((rc = grow(ctx, ctx->in_l, fbytes)) || (rc = copy_frames(ctx, (uint8_t*)ctx->in_l.p, df, h_left, f, n_pairs, st))) return rc;
+  if ((rc = grow(ctx, ctx->in_r, fbytes)) || (rc = copy_frames(ctx, (uint8_t*)ctx->in_r.p, df, h_right, f, n_pairs, st))) return rc;
   usv_outputs d_out;
   memset(&d_out, 0, sizeof(d_out));
   usv_outputs ho = *h_out;
@@ -587,10 +619,7 @@ static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_righ
     }
   }
   // the refinement reads the winners' RightIndex: the caller's array when it was asked for, scratch otherwise
-  if (sub && !d_out.right_index) {
-    if ((rc = grow(ctx, ctx->sub_ri, 4 * n_res))) return rc;
-    d_out.right_index = (uint32_t*)ctx->sub_ri.p;
-  }
+  if (sub && (rc = or_scratch(ctx, ctx->sub_ri, {{(void**)&d_out.right_index, 4 * (size_t)n_res}}))) return rc;
   rc = match_device(ctx, (const uint8_t*)ctx->in_l.p, (const uint8_t*)ctx->in_r.p, &df, n_pairs, p, &d_out, d_tx, d_ty, n_templates,
                     d_rows, d_srows, row_cap, st);
   if (rc) return rc;
@@ -700,16 +729,6 @@ extern "C" int usv_resolve_match_list(usv_ctx* ctx, const usv_match* h_in, int64
 }
 
 // ---- generate -> resolve -> distance in one call, host buffers (the reference's call order, P/Main.cpp:1115-1143) ----
-static int grow_pinned(usv_ctx* ctx, int k, size_t bytes) {
-  if (bytes <= ctx->pin_cap[k]) return USV_OK;
-  if (ctx->pin[k]) { CU(cudaFreeHost(ctx->pin[k])); ctx->pin[k] = nullptr; ctx->pin_cap[k] = 0; }
-  const size_t want = bytes + bytes / 4 + 4096;
-  cudaError_t e = cudaHostAlloc(&ctx->pin[k], want, cudaHostAllocDefault);
-  if (e != cudaSuccess) return fail(ctx, USV_ERR_NOMEM, "cudaHostAlloc(%zu): %s", want, cudaGetErrorString(e));
-  ctx->pin_cap[k] = want;
-  return USV_OK;
-}
-
 extern "C" int usv_block_search_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_right, const usv_frame_desc* f,
                                      const usv_search_params* p, usv_match* h_matches, double* h_distance, int64_t cap, int64_t* n_out) {
   if (!ctx) return USV_ERR_INVALID_ARG;
@@ -724,10 +743,11 @@ extern "C" int usv_block_search_host(usv_ctx* ctx, const uint8_t* h_left, const 
   cudaStream_t st = ctx->stream;
   // frames: caller memory -> pinned staging at the device pitch (one host pass; the H2D is then one asynchronous copy
   // per camera) -> HBM
-  const int row_bytes = f->width * f->channels, pitch = (row_bytes + 127) & ~127;
-  const size_t fbytes = (size_t)pitch * f->height;
-  if ((rc = grow_pinned(ctx, 0, 2 * fbytes))) return rc;
-  uint8_t* stage = (uint8_t*)ctx->pin[0];
+  const usv_frame_desc df = device_frame_desc(f);
+  const int row_bytes = f->width * f->channels, pitch = df.row_stride;
+  const size_t fbytes = (size_t)df.frame_stride;
+  if ((rc = grow(ctx, ctx->pin[0], 2 * fbytes))) return rc;
+  uint8_t* stage = (uint8_t*)ctx->pin[0].p;
   for (int k = 0; k < 2; ++k) {
     const uint8_t* src = k ? h_right : h_left;
     uint8_t* dst = stage + k * fbytes;
@@ -737,8 +757,6 @@ extern "C" int usv_block_search_host(usv_ctx* ctx, const uint8_t* h_left, const 
   if ((rc = grow(ctx, ctx->in_l, fbytes)) || (rc = grow(ctx, ctx->in_r, fbytes))) return rc;
   CU(cudaMemcpyAsync(ctx->in_l.p, stage, fbytes, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(ctx->in_r.p, stage + fbytes, fbytes, cudaMemcpyHostToDevice, st));
-  usv_frame_desc df = *f;
-  df.row_stride = pitch; df.frame_stride = (int64_t)fbytes;
   // generate (+ per-window first minimum): the winners stay in HBM
   if ((rc = grow(ctx, ctx->out[0], sizeof(usv_match) * n_win))) return rc;
   usv_outputs d_out;
@@ -764,17 +782,17 @@ extern "C" int usv_block_search_host(usv_ctx* ctx, const uint8_t* h_left, const 
   }
   ctx->last_kernel = match_kernel;
   // results: count first, then exactly the surviving records through pinned staging
-  if ((rc = grow_pinned(ctx, 1, sizeof(usv_match) * n_win + 64)) || (rc = grow_pinned(ctx, 2, sizeof(double) * n_win + 64))) return rc;
-  int64_t* h_n = (int64_t*)((uint8_t*)ctx->pin[1] + sizeof(usv_match) * n_win);
+  if ((rc = grow(ctx, ctx->pin[1], sizeof(usv_match) * n_win + 64)) || (rc = grow(ctx, ctx->pin[2], sizeof(double) * n_win + 64))) return rc;
+  int64_t* h_n = (int64_t*)((uint8_t*)ctx->pin[1].p + sizeof(usv_match) * n_win);
   CU(cudaMemcpyAsync(h_n, ctx->misc[2].p, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   const int64_t total = *h_n, m = total < cap ? total : cap;
   if (m > 0) {
-    CU(cudaMemcpyAsync(ctx->pin[1], ctx->misc[1].p, sizeof(usv_match) * (size_t)m, cudaMemcpyDeviceToHost, st));
-    if (want_dist) CU(cudaMemcpyAsync(ctx->pin[2], ctx->misc[3].p, sizeof(double) * (size_t)m, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(ctx->pin[1].p, ctx->misc[1].p, sizeof(usv_match) * (size_t)m, cudaMemcpyDeviceToHost, st));
+    if (want_dist) CU(cudaMemcpyAsync(ctx->pin[2].p, ctx->misc[3].p, sizeof(double) * (size_t)m, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    memcpy(h_matches, ctx->pin[1], sizeof(usv_match) * (size_t)m);
-    if (want_dist) memcpy(h_distance, ctx->pin[2], sizeof(double) * (size_t)m);
+    memcpy(h_matches, ctx->pin[1].p, sizeof(usv_match) * (size_t)m);
+    if (want_dist) memcpy(h_distance, ctx->pin[2].p, sizeof(double) * (size_t)m);
     else if (h_distance) memset(h_distance, 0, sizeof(double) * (size_t)m);
   }
   *n_out = total;
@@ -1051,43 +1069,41 @@ extern "C" int64_t usv_pair_nearest(const double* tl, int64_t nl, const double* 
 struct Slot {
   cudaStream_t st = nullptr;
   cudaEvent_t done = nullptr;
-  uint8_t *h_l = nullptr, *h_r = nullptr, *d_l = nullptr, *d_r = nullptr;
-  usv_outputs h_out, d_out;
+  PinnedBuf h_l, h_r;
+  DevBuf d_l, d_r;
+  PinnedBuf h_arr[kNumOut];  // the arrays of the output mask; h_out and d_out point at them
+  DevBuf d_arr[kNumOut];
+  usv_outputs h_out{}, d_out{};
   DevBuf corr_ws;  // planes + window statistics of the sliding correlation kernel: per slot, the slots run concurrently
   DevBuf win_ws;   // winners (RightIndex + value) for the resolved disparity map when the caller did not ask for them
+  Slot() = default;
+  Slot(const Slot&) = delete;
+  Slot& operator=(const Slot&) = delete;
+  ~Slot() {
+    if (done) cudaEventDestroy(done);
+    if (st) cudaStreamDestroy(st);
+  }
 };
 
 struct usv_stream {
   usv_ctx* ctx = nullptr;
   int device = 0;
-  usv_frame_desc hf, df;
+  usv_frame_desc fd;  // layout of the slots' pinned frames and of their device frames (the same: one copy per camera)
   usv_search_params params;
   int32_t pairs_per_slot = 0, n_slots = 0;
   uint32_t mask = 0;
   int64_t n_win = 0;
-  std::vector<Slot> slots;
+  std::unique_ptr<Slot[]> slots;
 };
 
 extern "C" int usv_stream_destroy(usv_stream* s) {
   if (!s) return USV_ERR_INVALID_ARG;
   cudaSetDevice(s->device);
-  for (Slot& sl : s->slots) {
-    if (sl.st) cudaStreamSynchronize(sl.st);
-    if (sl.h_l) cudaFreeHost(sl.h_l);
-    if (sl.h_r) cudaFreeHost(sl.h_r);
-    if (sl.d_l) cudaFree(sl.d_l);
-    if (sl.d_r) cudaFree(sl.d_r);
-    if (sl.corr_ws.p) cudaFree(sl.corr_ws.p);
-    if (sl.win_ws.p) cudaFree(sl.win_ws.p);
-    for (int i = 0; i < kNumOut; ++i) {
-      if (*out_slot(&sl.h_out, i)) cudaFreeHost(*out_slot(&sl.h_out, i));
-      if (*out_slot(&sl.d_out, i)) cudaFree(*out_slot(&sl.d_out, i));
-    }
-    if (sl.done) cudaEventDestroy(sl.done);
-    if (sl.st) cudaStreamDestroy(sl.st);
-  }
-  if (s->ctx) s->ctx->open_streams--;
+  for (int i = 0; i < s->n_slots; ++i)
+    if (s->slots[i].st) cudaStreamSynchronize(s->slots[i].st);
+  usv_ctx* ctx = s->ctx;
   delete s;
+  if (ctx) ctx->open_streams--;
   return USV_OK;
 }
 
@@ -1106,32 +1122,27 @@ extern "C" int usv_stream_create(usv_ctx* ctx, const usv_frame_desc* frame, cons
   if (!s) return fail(ctx, USV_ERR_NOMEM, "out of host memory");
   s->ctx = ctx; s->device = ctx->device; ctx->open_streams++; s->params = *params; s->pairs_per_slot = pairs_per_slot; s->n_slots = n_slots; s->mask = output_mask;
   s->n_win = (int64_t)nx * ny;
-  // pinned staging keeps the frames tightly packed at a 128-byte pitch, the same layout as in HBM,
-  // so each slot needs exactly one cudaMemcpyAsync per camera
-  const int pitch = (frame->width * frame->channels + 127) & ~127;
-  s->hf = *frame; s->hf.row_stride = pitch; s->hf.frame_stride = (int64_t)pitch * frame->height;
-  s->df = s->hf;
-  s->slots.resize(n_slots);
-  const size_t fbytes = (size_t)s->hf.frame_stride * pairs_per_slot;
+  // pinned staging keeps the frames tightly packed at the device layout, so each slot needs exactly one
+  // cudaMemcpyAsync per camera
+  s->fd = device_frame_desc(frame);
+  s->slots.reset(new Slot[n_slots]);
+  const size_t fbytes = (size_t)s->fd.frame_stride * pairs_per_slot;
   const size_t n_res = (size_t)s->n_win * pairs_per_slot;
   cudaError_t e = cudaSuccess;
-  for (Slot& sl : s->slots) {
-    memset(&sl.h_out, 0, sizeof(sl.h_out));
-    memset(&sl.d_out, 0, sizeof(sl.d_out));
+  for (int k = 0; k < n_slots && e == cudaSuccess; ++k) {
+    Slot& sl = s->slots[k];
     if ((e = cudaStreamCreateWithFlags(&sl.st, cudaStreamNonBlocking)) != cudaSuccess) break;
     if ((e = cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming)) != cudaSuccess) break;
-    if ((e = cudaHostAlloc((void**)&sl.h_l, fbytes, cudaHostAllocDefault)) != cudaSuccess) break;
-    if ((e = cudaHostAlloc((void**)&sl.h_r, fbytes, cudaHostAllocDefault)) != cudaSuccess) break;
-    if ((e = cudaMalloc((void**)&sl.d_l, fbytes)) != cudaSuccess) break;
-    if ((e = cudaMalloc((void**)&sl.d_r, fbytes)) != cudaSuccess) break;
-    memset(sl.h_l, 0, fbytes);
-    memset(sl.h_r, 0, fbytes);
-    for (int i = 0; i < kNumOut && e == cudaSuccess; ++i) {
+    if ((e = sl.h_l.alloc(fbytes)) != cudaSuccess || (e = sl.h_r.alloc(fbytes)) != cudaSuccess) break;
+    if ((e = sl.d_l.alloc(fbytes)) != cudaSuccess || (e = sl.d_r.alloc(fbytes)) != cudaSuccess) break;
+    memset(sl.h_l.p, 0, fbytes);
+    memset(sl.h_r.p, 0, fbytes);
+    for (int i = 0; i < kNumOut; ++i) {
       if (!(output_mask & (1u << i))) continue;
-      if ((e = cudaHostAlloc(out_slot(&sl.h_out, i), kOutElem[i] * n_res, cudaHostAllocDefault)) != cudaSuccess) break;
-      e = cudaMalloc(out_slot(&sl.d_out, i), kOutElem[i] * n_res);
+      if ((e = sl.h_arr[i].alloc(kOutElem[i] * n_res)) != cudaSuccess || (e = sl.d_arr[i].alloc(kOutElem[i] * n_res)) != cudaSuccess) break;
+      *out_slot(&sl.h_out, i) = sl.h_arr[i].p;
+      *out_slot(&sl.d_out, i) = sl.d_arr[i].p;
     }
-    if (e != cudaSuccess) break;
   }
   if (e != cudaSuccess) {
     fail(ctx, USV_ERR_NOMEM, "stream allocation: %s", cudaGetErrorString(e));
@@ -1144,38 +1155,20 @@ extern "C" int usv_stream_create(usv_ctx* ctx, const usv_frame_desc* frame, cons
 
 extern "C" int usv_stream_slot(usv_stream* s, int32_t slot, uint8_t** h_left, uint8_t** h_right, usv_outputs* h_out) {
   if (!s || slot < 0 || slot >= s->n_slots) return USV_ERR_INVALID_ARG;
-  if (h_left) *h_left = s->slots[slot].h_l;
-  if (h_right) *h_right = s->slots[slot].h_r;
+  if (h_left) *h_left = (uint8_t*)s->slots[slot].h_l.p;
+  if (h_right) *h_right = (uint8_t*)s->slots[slot].h_r.p;
   if (h_out) *h_out = s->slots[slot].h_out;
   return USV_OK;
 }
 
 extern "C" int usv_stream_frame_desc(const usv_stream* s, usv_frame_desc* out) {
   if (!s || !out) return USV_ERR_INVALID_ARG;
-  *out = s->hf;
-  return USV_OK;
-}
-
-// kernels + D2H + completion event of a slot whose frames are already enqueued on its stream
-// (h_dst: the caller's own result arrays instead of the slot's pinned ones — usv_stream_submit_io)
-static int enqueue_match_and_results(usv_stream* s, Slot& sl, int32_t n_pairs, usv_outputs* h_dst = nullptr) {
-  usv_ctx* ctx = s->ctx;
-  if (n_pairs > 0) {
-    int rc = match_device(ctx, sl.d_l, sl.d_r, &s->df, n_pairs, &s->params, &sl.d_out, nullptr, nullptr, 0, nullptr, nullptr, 0, sl.st,
-                          &sl.corr_ws, &sl.win_ws);
-    if (rc) return rc;
-    const size_t n_res = (size_t)s->n_win * n_pairs;
-    for (int i = 0; i < kNumOut; ++i)
-      if (*out_slot(&sl.h_out, i))
-        CU(cudaMemcpyAsync(h_dst ? *out_slot(h_dst, i) : *out_slot(&sl.h_out, i), *out_slot(&sl.d_out, i), kOutElem[i] * n_res,
-                           cudaMemcpyDeviceToHost, sl.st));
-  }
-  CU(cudaEventRecord(sl.done, sl.st));
+  *out = s->fd;
   return USV_OK;
 }
 
 static int check_host_frame(usv_stream* s, const usv_frame_desc* hf) {
-  if (hf->width != s->hf.width || hf->height != s->hf.height || hf->channels != s->hf.channels ||
+  if (hf->width != s->fd.width || hf->height != s->fd.height || hf->channels != s->fd.channels ||
       hf->row_stride < hf->width * hf->channels)
     return fail(s->ctx, USV_ERR_INVALID_ARG, "frame geometry differs from the stream's");
   if (hf->frame_stride < (int64_t)hf->row_stride * hf->height)
@@ -1183,102 +1176,86 @@ static int check_host_frame(usv_stream* s, const usv_frame_desc* hf) {
   return USV_OK;
 }
 
-// H2D of `n` consecutive host frames (layout `hf`) into consecutive device frames starting at `dst`
-static int enqueue_frames(usv_stream* s, Slot& sl, uint8_t* dst, const uint8_t* src, const usv_frame_desc* hf, int32_t n) {
+// the frames of one submit: pair i is frame idx_left[i] of `left` and frame idx_right[i] of `right` (frame i of each
+// without index arrays), laid out per `hf`
+struct FrameSrc {
+  const uint8_t* left;
+  const uint8_t* right;
+  const usv_frame_desc* hf;
+  const int32_t* idx_left = nullptr;
+  const int32_t* idx_right = nullptr;
+  int64_t n_store = 0;  // frames of each store, with index arrays
+};
+
+// frames H2D, kernels, results D2H (into the caller's h_dst instead of the slot's pinned arrays when given) and the
+// completion event of one slot, all on its stream
+static int submit(usv_stream* s, int32_t slot, int32_t n_pairs, const FrameSrc& src, const usv_outputs* h_dst) {
   usv_ctx* ctx = s->ctx;
-  const int row_bytes = hf->width * hf->channels;
-  if (hf->row_stride == s->df.row_stride && (n == 1 || hf->frame_stride == s->df.frame_stride)) {
-    const size_t bytes = n == 1 ? (size_t)hf->row_stride * hf->height : (size_t)s->df.frame_stride * n;
-    CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, sl.st));
-  } else if (n == 1 || hf->frame_stride == (int64_t)hf->row_stride * hf->height) {
-    CU(cudaMemcpy2DAsync(dst, s->df.row_stride, src, hf->row_stride, row_bytes, (size_t)hf->height * n, cudaMemcpyHostToDevice, sl.st));
-  } else {
-    for (int i = 0; i < n; ++i)
-      CU(cudaMemcpy2DAsync(dst + (size_t)i * s->df.frame_stride, s->df.row_stride, src + (size_t)i * hf->frame_stride, hf->row_stride,
-                           row_bytes, hf->height, cudaMemcpyHostToDevice, sl.st));
+  if (n_pairs < 0 || n_pairs > s->pairs_per_slot) return fail(ctx, USV_ERR_INVALID_ARG, "n_pairs %d exceeds the slot", n_pairs);
+  int rc = check_host_frame(s, src.hf);
+  if (rc) return rc;
+  const int32_t* idx[2] = {src.idx_left, src.idx_right};
+  if (idx[0])
+    for (int i = 0; i < n_pairs; ++i)
+      if (idx[0][i] < 0 || idx[0][i] >= src.n_store || idx[1][i] < 0 || idx[1][i] >= src.n_store)
+        return fail(ctx, USV_ERR_INVALID_ARG, "pair %d: frame index outside the store", i);
+  Slot& sl = s->slots[slot];
+  usv_outputs dst = h_dst ? *h_dst : sl.h_out;
+  if (h_dst)
+    for (int i = 0; i < kNumOut; ++i)
+      if (((s->mask >> i) & 1u) && !*out_slot(&dst, i)) return fail(ctx, USV_ERR_INVALID_ARG, "destination of output %d of the stream's mask is null", i);
+  CU(cudaSetDevice(ctx->device));
+  const uint8_t* store[2] = {src.left, src.right};
+  uint8_t* d_frames[2] = {(uint8_t*)sl.d_l.p, (uint8_t*)sl.d_r.p};
+  for (int k = 0; k < 2; ++k) {
+    // runs of consecutive store frames travel as one copy (paired unsynchronised streams are mostly consecutive)
+    for (int i = 0; i < n_pairs;) {
+      int j = i + 1;
+      while (j < n_pairs && (!idx[k] || idx[k][j] == idx[k][j - 1] + 1)) ++j;
+      const uint8_t* first = store[k] + (size_t)(idx[k] ? idx[k][i] : i) * src.hf->frame_stride;
+      if ((rc = copy_frames(ctx, d_frames[k] + (size_t)i * s->fd.frame_stride, s->fd, first, src.hf, j - i, sl.st))) return rc;
+      i = j;
+    }
   }
+  if (n_pairs > 0) {
+    rc = match_device(ctx, d_frames[0], d_frames[1], &s->fd, n_pairs, &s->params, &sl.d_out, nullptr, nullptr, 0, nullptr, nullptr, 0,
+                      sl.st, &sl.corr_ws, &sl.win_ws);
+    if (rc) return rc;
+    const size_t n_res = (size_t)s->n_win * n_pairs;
+    for (int i = 0; i < kNumOut; ++i)
+      if (*out_slot(&sl.h_out, i))
+        CU(cudaMemcpyAsync(*out_slot(&dst, i), *out_slot(&sl.d_out, i), kOutElem[i] * n_res, cudaMemcpyDeviceToHost, sl.st));
+  }
+  CU(cudaEventRecord(sl.done, sl.st));
   return USV_OK;
 }
 
 extern "C" int usv_stream_submit(usv_stream* s, int32_t slot, int32_t n_pairs) {
   if (!s || slot < 0 || slot >= s->n_slots) return USV_ERR_INVALID_ARG;
-  usv_ctx* ctx = s->ctx;
-  if (n_pairs < 0 || n_pairs > s->pairs_per_slot) return fail(ctx, USV_ERR_INVALID_ARG, "n_pairs %d exceeds the slot", n_pairs);
-  CU(cudaSetDevice(ctx->device));
-  Slot& sl = s->slots[slot];
-  if (n_pairs > 0) {
-    const size_t fbytes = (size_t)s->hf.frame_stride * n_pairs;
-    CU(cudaMemcpyAsync(sl.d_l, sl.h_l, fbytes, cudaMemcpyHostToDevice, sl.st));
-    CU(cudaMemcpyAsync(sl.d_r, sl.h_r, fbytes, cudaMemcpyHostToDevice, sl.st));
-  }
-  return enqueue_match_and_results(s, sl, n_pairs);
+  const Slot& sl = s->slots[slot];
+  return submit(s, slot, n_pairs, {(const uint8_t*)sl.h_l.p, (const uint8_t*)sl.h_r.p, &s->fd}, nullptr);
 }
 
 extern "C" int usv_stream_submit_from(usv_stream* s, int32_t slot, const uint8_t* h_left, const uint8_t* h_right,
                                       const usv_frame_desc* hf, int32_t n_pairs) {
   if (!s || slot < 0 || slot >= s->n_slots) return USV_ERR_INVALID_ARG;
-  usv_ctx* ctx = s->ctx;
-  if (!h_left || !h_right || !hf) return fail(ctx, USV_ERR_INVALID_ARG, "null pointer");
-  if (n_pairs < 0 || n_pairs > s->pairs_per_slot) return fail(ctx, USV_ERR_INVALID_ARG, "n_pairs %d exceeds the slot", n_pairs);
-  int rc = check_host_frame(s, hf);
-  if (rc) return rc;
-  CU(cudaSetDevice(ctx->device));
-  Slot& sl = s->slots[slot];
-  if (n_pairs > 0) {
-    if ((rc = enqueue_frames(s, sl, sl.d_l, h_left, hf, n_pairs))) return rc;
-    if ((rc = enqueue_frames(s, sl, sl.d_r, h_right, hf, n_pairs))) return rc;
-  }
-  return enqueue_match_and_results(s, sl, n_pairs);
+  if (!h_left || !h_right || !hf) return fail(s->ctx, USV_ERR_INVALID_ARG, "null pointer");
+  return submit(s, slot, n_pairs, {h_left, h_right, hf}, nullptr);
 }
 
 extern "C" int usv_stream_submit_gather(usv_stream* s, int32_t slot, const uint8_t* left_store, const int32_t* idx_left,
                                         const uint8_t* right_store, const int32_t* idx_right, int64_t n_store_frames,
                                         const usv_frame_desc* hf, int32_t n_pairs) {
   if (!s || slot < 0 || slot >= s->n_slots) return USV_ERR_INVALID_ARG;
-  usv_ctx* ctx = s->ctx;
-  if (!left_store || !right_store || !idx_left || !idx_right || !hf) return fail(ctx, USV_ERR_INVALID_ARG, "null pointer");
-  if (n_pairs < 0 || n_pairs > s->pairs_per_slot) return fail(ctx, USV_ERR_INVALID_ARG, "n_pairs %d exceeds the slot", n_pairs);
-  int rc = check_host_frame(s, hf);
-  if (rc) return rc;
-  for (int i = 0; i < n_pairs; ++i)
-    if (idx_left[i] < 0 || idx_left[i] >= n_store_frames || idx_right[i] < 0 || idx_right[i] >= n_store_frames)
-      return fail(ctx, USV_ERR_INVALID_ARG, "pair %d: frame index outside the store", i);
-  CU(cudaSetDevice(ctx->device));
-  Slot& sl = s->slots[slot];
-  const uint8_t* store[2] = {left_store, right_store};
-  const int32_t* idx[2] = {idx_left, idx_right};
-  uint8_t* dst[2] = {sl.d_l, sl.d_r};
-  for (int k = 0; k < 2; ++k) {
-    // runs of consecutive store frames travel as one copy (paired unsynchronised streams are mostly consecutive)
-    for (int i = 0; i < n_pairs;) {
-      int j = i + 1;
-      while (j < n_pairs && idx[k][j] == idx[k][j - 1] + 1) ++j;
-      if ((rc = enqueue_frames(s, sl, dst[k] + (size_t)i * s->df.frame_stride, store[k] + (size_t)idx[k][i] * hf->frame_stride, hf, j - i)))
-        return rc;
-      i = j;
-    }
-  }
-  return enqueue_match_and_results(s, sl, n_pairs);
+  if (!left_store || !right_store || !idx_left || !idx_right || !hf) return fail(s->ctx, USV_ERR_INVALID_ARG, "null pointer");
+  return submit(s, slot, n_pairs, {left_store, right_store, hf, idx_left, idx_right, n_store_frames}, nullptr);
 }
 
 extern "C" int usv_stream_submit_io(usv_stream* s, int32_t slot, const uint8_t* h_left, const uint8_t* h_right, const usv_frame_desc* hf,
                                     int32_t n_pairs, const usv_outputs* h_dst) {
   if (!s || slot < 0 || slot >= s->n_slots) return USV_ERR_INVALID_ARG;
-  usv_ctx* ctx = s->ctx;
-  if (!h_left || !h_right || !hf || !h_dst) return fail(ctx, USV_ERR_INVALID_ARG, "null pointer");
-  if (n_pairs < 0 || n_pairs > s->pairs_per_slot) return fail(ctx, USV_ERR_INVALID_ARG, "n_pairs %d exceeds the slot", n_pairs);
-  int rc = check_host_frame(s, hf);
-  if (rc) return rc;
-  usv_outputs dst = *h_dst;
-  for (int i = 0; i < kNumOut; ++i)
-    if (((s->mask >> i) & 1u) && !*out_slot(&dst, i)) return fail(ctx, USV_ERR_INVALID_ARG, "destination of output %d of the stream's mask is null", i);
-  CU(cudaSetDevice(ctx->device));
-  Slot& sl = s->slots[slot];
-  if (n_pairs > 0) {
-    if ((rc = enqueue_frames(s, sl, sl.d_l, h_left, hf, n_pairs))) return rc;
-    if ((rc = enqueue_frames(s, sl, sl.d_r, h_right, hf, n_pairs))) return rc;
-  }
-  return enqueue_match_and_results(s, sl, n_pairs, &dst);
+  if (!h_left || !h_right || !hf || !h_dst) return fail(s->ctx, USV_ERR_INVALID_ARG, "null pointer");
+  return submit(s, slot, n_pairs, {h_left, h_right, hf}, h_dst);
 }
 
 extern "C" int usv_host_register(usv_ctx* ctx, void* p, size_t bytes) {
@@ -1305,7 +1282,7 @@ extern "C" int usv_stream_wait(usv_stream* s, int32_t slot) {
 
 extern "C" int usv_stream_bytes_per_pair(const usv_stream* s, int64_t* h2d, int64_t* d2h) {
   if (!s) return USV_ERR_INVALID_ARG;
-  if (h2d) *h2d = 2 * s->hf.frame_stride;
+  if (h2d) *h2d = 2 * s->fd.frame_stride;
   int64_t o = 0;
   for (int i = 0; i < kNumOut; ++i)
     if (s->mask & (1u << i)) o += (int64_t)kOutElem[i] * s->n_win;

@@ -39,6 +39,9 @@ struct DevJob {
 
 constexpr int kDevStatusUmmaTimeout = 1;
 
+// row pitch of the planes that interleaved colour frames are split into for the dense sweeps (usv_dense_corr.cu)
+inline int colour_plane_pitch(const DevJob& J) { return ((J.width + 15) & ~15) + 16; }
+
 __device__ __forceinline__ unsigned long long global_timer_ns() {
   unsigned long long t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));

@@ -54,11 +54,9 @@ static int ceil_log2(long long v) {
 // usv_dense_corr.cu: interleaved colour frames -> planes [pair][plane][H][pitch] of both cameras
 cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst_l, uint8_t* dst_r, int pitch, cudaStream_t st);
 
-static int dense_plane_pitch(const DevJob& J) { return ((J.width + 15) & ~15) + 16; }
-
 // scratch the colour sweep needs per pair (planes of both cameras); 0 for one-plane frames
 size_t dense_scratch_bytes_per_pair(const DevJob& J) {
-  return J.channels == 3 ? 2ull * 3 * J.height * dense_plane_pitch(J) : 0;
+  return J.channels == 3 ? 2ull * 3 * J.height * colour_plane_pitch(J) : 0;
 }
 
 cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
@@ -97,7 +95,7 @@ cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t s
   cfg.bh = (J.nyc + n_bands - 1) / n_bands;
   cfg.n_bands = (J.nyc + cfg.bh - 1) / cfg.bh;
   const size_t smem = (size_t)cfg.ring_words * 4 + (size_t)cfg.bh * 512;
-  const int pitch = npl == 1 ? J.row_stride : dense_plane_pitch(J);
+  const int pitch = npl == 1 ? J.row_stride : colour_plane_pitch(J);
   cfg.pitch = pitch;
   cfg.plane_stride = npl == 1 ? 0 : (long long)J.height * pitch;
   cfg.pair_stride = npl == 1 ? J.frame_stride : cfg.plane_stride * npl;

@@ -435,7 +435,8 @@ __global__ void corr_stats_kernel(const uint2* __restrict__ rs, int height, int 
   }
 }
 
-// for the colour SAD sweep of usv_dense.cu (kernels are launched from the translation unit that defines them)
+// colour planes of both cameras for the sweep below and for the colour SAD sweep of usv_dense.cu (kernels are launched
+// from the translation unit that defines them)
 cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst_l, uint8_t* dst_r, int pitch, cudaStream_t st) {
   const long long plane_stride = (long long)J.height * pitch, pair_stride = plane_stride * J.channels;
   const dim3 g((pitch + 255) / 256, J.height, np);
@@ -447,7 +448,7 @@ cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst
 }
 
 size_t corr_scratch_bytes_per_pair(const DevJob& J, int* pitch_out) {
-  const int pitch = ((J.width + 15) & ~15) + 16;
+  const int pitch = colour_plane_pitch(J);
   if (pitch_out) *pitch_out = pitch;
   const size_t planes = J.channels > 1 ? 2ull * J.channels * J.height * pitch : 0;
   return planes + 2ull * J.nyc * J.nxc * sizeof(double2) + (size_t)J.height * J.nxc * sizeof(uint2) + 512 + corr_mma_best_bytes_per_pair(J);
@@ -506,9 +507,8 @@ cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, siz
       uint8_t* pl_l = base;
       uint8_t* pl_r = base + (size_t)np * cfg.pair_stride;
       base += 2 * (size_t)np * cfg.pair_stride;
-      const dim3 g((pitch + 255) / 256, J.height, np);
-      corr_planes_kernel<<<g, 256, 0, st>>>(fl, J.frame_stride, J.row_stride, J.width, J.height, npl, pl_l, cfg.pair_stride, cfg.plane_stride, pitch);
-      corr_planes_kernel<<<g, 256, 0, st>>>(fr, J.frame_stride, J.row_stride, J.width, J.height, npl, pl_r, cfg.pair_stride, cfg.plane_stride, pitch);
+      const cudaError_t e = launch_split_planes(J, p0, np, pl_l, pl_r, pitch, st);
+      if (e != cudaSuccess) return e;
       cfg.lp = pl_l; cfg.rp = pl_r;
       *n_launches += 2;
     } else {
