@@ -23,7 +23,7 @@ bool direct_supported(const DevJob& J);
 size_t dense_scratch_bytes_per_pair(const DevJob& J);
 cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
                          int* n_launches);
-size_t corr_scratch_bytes_per_pair(const DevJob& J, int* pitch_out);
+size_t corr_scratch_bytes_per_pair(const DevJob& J);
 cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
                               int* n_launches);
 cudaError_t launch_contour_descriptors(const int* pts, const int* off, int n, double* desc, cudaStream_t st);
@@ -403,7 +403,7 @@ static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, bool s
     if (e != cudaErrorNotSupported) return fail(ctx, USV_ERR_CUDA, "dense launch: %s", cudaGetErrorString(e));
     (void)cudaGetLastError();
     // sliding-window correlation kernel
-    if ((rc = grow_pair_scratch(ctx, ws, usv::corr_scratch_bytes_per_pair(J, nullptr), n_pairs))) return rc;
+    if ((rc = grow_pair_scratch(ctx, ws, usv::corr_scratch_bytes_per_pair(J), n_pairs))) return rc;
     e = usv::launch_dense_corr(J, n_pairs, ws.p, ws.cap, st, &name, &nl);
     if (e == cudaSuccess) {
       ctx->launches += nl;

@@ -14,10 +14,7 @@
 // Sab slides exactly like the SAD: h(u, d, v) = sum_{b<4} L[v][u+b] * R[v][u-d+b] over the colour planes (one
 // IDP.4A.U8.U8 each; interleaved frames are split into planes first, so that a packed word holds four pixels of one
 // channel), V(u, d, y) = sum of h over the th rows of the window kept in a register and slid down the rows,
-// Sab(x, d, y) = sum_{k < tw/4} V(x + 4k, d, y). Per candidate, in f64:
-//   n*Sab      = fma(n, 2^52 + Sab, -n*2^52)        (2^52 + Sab is the u32 -> f64 conversion by bit pattern; exact)
-//   num        = fma(-Sa, Sb, n*Sab)                 (exact: all integers below 2^53)
-//   score      = (num * ra) * rb,  v = 1 - score     (the oracle's three roundings)
+// Sab(x, d, y) = sum_{k < tw/4} V(x + 4k, d, y). Per candidate, v = 1 - score in f64 (usv_corr.cuh: corr_score),
 // and the candidate replaces the running best iff v < best (ties: the smaller x', P/Main.cpp:451). Candidates outside
 // the frame carry rb = NaN and disparities outside [search_min, search_max] carry n = NaN: their v is NaN and loses
 // every comparison, so validity costs no instruction in the inner loop.
@@ -177,15 +174,10 @@ __device__ __forceinline__ void corr_pass(const DevJob& J, const CorrCfg& cfg, u
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const int k = DIR < 0 ? i - j + 3 : i + j;
-          const double nsab = __fma_rn(nj[j], __hiloint2double(0x43300000, (int)T[j]), c0j[j]);  // n * Sab, exact
-          // ZNCC / NCC: n Sab - Sa Sb (exact), then the oracle's two roundings. SSD: "score" = -(Saa + Sbb - 2 Sab), an
-          // exact integer, so v = 1 - score = 1 + SSD orders the candidates by their integer cost
-          const double num = SSD ? __dadd_rn(__dadd_rn(La[i].x, Rs[k].x), nsab) : __fma_rn(La[i].x, Rs[k].x, nsab);
-          const double sc = SSD ? num : __dmul_rn(__dmul_rn(num, La[i].y), Rs[k].y);
-          const double v = __dsub_rn(1.0, sc);
+          const CorrCand c = corr_score<OP>(nj[j], c0j[j], (int)T[j], La[i], Rs[k]);
           // j ascending = x' descending (LeftCam) / ascending (RightCam): on a tie the smaller x' stays
-          const bool take = DIR < 0 ? v <= best_v : v < best_v;
-          if (take) { best_v = v; best_sc = sc; best_x = xrb + 4 * k; }
+          const bool take = DIR < 0 ? c.v <= best_v : c.v < best_v;
+          if (take) { best_v = c.v; best_sc = c.sc; best_x = xrb + 4 * k; }
           if (i < 7) T[j] += (i + NW < 8 ? V[i + NW][j] : Hx[i + NW - 8][j]) - V[i][j];
         }
         bsc[i] = best_sc; bx[i] = best_x;
@@ -284,15 +276,7 @@ __global__ void __launch_bounds__(kCThreads, 3) dense_corr_argmin_kernel(const D
     if (a >= n_pos || X0 + xo < 0) continue;
     const int e = (yy * 4 + pp) * 32 + a;
     const double sc = s_bsc[e];
-    const int xr = s_bx[e];
-    const int x = X0 + xo, y = y0 + yy;
-    const long long w = (long long)y * J.nx + x;
-    const long long g = (long long)(cfg.pair0 + pair) * J.n_templates + w;
-    if (xr == kNoX) write_result(J, g, (uint32_t)w, x, y, -1, 0xffffffffu, 0.0, __longlong_as_double(0x7ff0000000000000ll));
-    else if (OP != kOpCorr) {
-      const uint32_t raw = (uint32_t)(-sc);
-      write_result(J, g, (uint32_t)w, x, y, xr, raw, 0.0, normalised_cost(raw, OP == kOpSad ? USV_COST_SAD : USV_COST_SSD, J.n_elems));
-    } else write_result(J, g, (uint32_t)w, x, y, xr, 0xffffffffu, __dadd_rn(sc, 0.0), __dsub_rn(1.0, sc));  // -0.0 -> 0.0 (flat windows)
+    corr_emit<OP>(J, cfg.pair0 + pair, X0 + xo, y0 + yy, s_bx[e], __dsub_rn(1.0, sc), sc);
   }
 }
 
@@ -447,14 +431,95 @@ cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst
   return cudaGetLastError();
 }
 
-size_t corr_scratch_bytes_per_pair(const DevJob& J, int* pitch_out) {
-  const int pitch = colour_plane_pitch(J);
-  if (pitch_out) *pitch_out = pitch;
-  const size_t planes = J.channels > 1 ? 2ull * J.channels * J.height * pitch : 0;
-  return planes + 2ull * J.nyc * J.nxc * sizeof(double2) + (size_t)J.height * J.nxc * sizeof(uint2) + 512 + corr_mma_best_bytes_per_pair(J);
+// Pair scratch of launch_dense_corr for a chunk of np pairs: the colour planes of both cameras (colour frames only);
+// 256-byte aligned, the window statistics of both cameras and the row sums they are made from; 256-byte aligned, the
+// tensor-pipe sweeps' running best (v, score, x'). per_pair sets the chunk sizes. Its 1 280 bytes of slack cover the two
+// alignments (at most 510 bytes a chunk), so np * per_pair bytes hold a chunk of np pairs.
+struct CorrScratch {
+  size_t per_pair;
+  size_t planes_r, stat_l, stat_r, rsum, best_v, best_sc, best_x;  // offsets inside the chunk (left planes at 0)
+};
+static CorrScratch corr_scratch(const DevJob& J, size_t np) {
+  const size_t planes = J.channels > 1 ? (size_t)J.channels * J.height * colour_plane_pitch(J) : 0;  // of one camera
+  const size_t win = (size_t)J.nyc * J.nxc, rows = (size_t)J.height * J.nxc;
+  auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  CorrScratch s;
+  s.per_pair = 2 * planes + 2 * win * sizeof(double2) + rows * sizeof(uint2) + win * (2 * sizeof(double) + sizeof(int)) + 1280;
+  s.planes_r = np * planes;
+  s.stat_l = align(2 * np * planes);
+  s.stat_r = s.stat_l + np * win * sizeof(double2);
+  s.rsum = s.stat_r + np * win * sizeof(double2);
+  s.best_v = align(s.rsum + np * rows * sizeof(uint2));
+  s.best_sc = s.best_v + np * win * sizeof(double);
+  s.best_x = s.best_sc + np * win * sizeof(double);
+  return s;
 }
 
-// Returns cudaErrorNotSupported when the job is outside the kernel's coverage (the caller then runs the direct form).
+size_t corr_scratch_bytes_per_pair(const DevJob& J) { return corr_scratch(J, 1).per_pair; }
+
+// coverage of both tensor-pipe sweeps
+static bool corr_tensor_supported(const DevJob& J, int op) {
+  if (op == kOpSad) return false;               // |a - b| is not a product
+  if (J.tw < 1 || J.tw > 32) return false;      // K = 32 bytes of one product; narrower templates zero the unused bytes of A
+  return 255ll * 255 * J.n_elems < (1ll << 31);  // Sab must fit the s32 accumulators
+}
+
+void corr_bands(const DevJob& J, CorrCfg& cfg, int np, int slots, double warm_weight, int bh_cap) {
+  double best_eff = -1.0;
+  int best_nb = (J.nyc + bh_cap - 1) / bh_cap;
+  for (int nb = best_nb; nb <= std::max(best_nb, J.nyc / 8); ++nb) {
+    const int bh = (J.nyc + nb - 1) / nb, nbb = (J.nyc + bh - 1) / bh;
+    if (bh > bh_cap) continue;
+    const long long ctas = (long long)nbb * cfg.n_xtiles * np;
+    const long long waves = (ctas + slots - 1) / slots;
+    const double eff = (double)ctas / (double)(waves * slots) * bh / (bh + warm_weight * (J.th - 1));
+    if (eff > best_eff * 1.005) { best_eff = eff; best_nb = nbb; }
+  }
+  cfg.bh = (J.nyc + best_nb - 1) / best_nb;
+  cfg.n_bands = (J.nyc + cfg.bh - 1) / cfg.bh;
+}
+
+template <int DIR, int NW, int NPL>
+static CorrKernel alu_kernel_op(int op) {
+  return op == kOpSsd ? dense_corr_argmin_kernel<DIR, NW, NPL, kOpSsd>
+       : op == kOpSad ? dense_corr_argmin_kernel<DIR, NW, NPL, kOpSad>
+                      : dense_corr_argmin_kernel<DIR, NW, NPL, kOpCorr>;
+}
+template <int DIR, int NPL>
+static CorrKernel alu_kernel(int nw, int op) {
+  switch (nw) {
+    case 2: return alu_kernel_op<DIR, 2, NPL>(op);
+    case 3: return alu_kernel_op<DIR, 3, NPL>(op);
+    case 4: return alu_kernel_op<DIR, 4, NPL>(op);
+    case 6: return alu_kernel_op<DIR, 6, NPL>(op);
+    default: return alu_kernel_op<DIR, 8, NPL>(op);
+  }
+}
+
+constexpr size_t kCSmemBudget = 74 * 1024;  // three CTAs per SM
+static_assert((kCSmemBudget - (size_t)4 * kCRB * 3 * kCRowWords * 4) / (128 * 12) >= 8, "bands of at least 8 rows");
+
+// The ALU sweep: x-tiles of 4 * (33 - tw / 4) windows; as many bands as shared memory requires, more while the grid of
+// the whole batch (n_pairs) fills fewer than two CTAs per SM
+static cudaError_t launch_corr_alu(const DevJob& J, CorrCfg cfg, int op, int np, int n_pairs, cudaStream_t st) {
+  const int nw = J.tw / 4, npl = J.channels;
+  cfg.stride_px = 4 * (32 - nw + 1);
+  cfg.n_xtiles = (J.nxc + cfg.stride_px - 1) / cfg.stride_px;
+  cfg.x_off = J.camera_side == USV_LEFT_CAM ? ((cfg.n_xtiles * cfg.stride_px - J.nxc) & ~3) : 0;
+  const size_t ring_bytes = (size_t)4 * kCRB * npl * kCRowWords * 4;
+  const int bh_max = (int)((kCSmemBudget - ring_bytes) / (128 * 12));
+  int n_bands = (J.nyc + bh_max - 1) / bh_max;
+  while ((long long)n_bands * cfg.n_xtiles * n_pairs < g_sm_count * 2 && n_bands < (J.nyc + 15) / 16) ++n_bands;
+  cfg.bh = (J.nyc + n_bands - 1) / n_bands;
+  cfg.n_bands = (J.nyc + cfg.bh - 1) / cfg.bh;
+  const size_t smem = ring_bytes + (size_t)cfg.bh * 128 * 12;
+  const CorrKernel k = J.camera_side == USV_LEFT_CAM ? (npl == 1 ? alu_kernel<-1, 1>(nw, op) : alu_kernel<-1, 3>(nw, op))
+                                                     : (npl == 1 ? alu_kernel<1, 1>(nw, op) : alu_kernel<1, 3>(nw, op));
+  return launch_corr_kernel(k, dim3(cfg.n_xtiles, cfg.n_bands, np), dim3(kCThreads), smem, st, J, cfg);
+}
+
+// Returns cudaErrorNotSupported when the job is outside the coverage of the three sweeps (the caller then runs the
+// direct form).
 cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
                               int* n_launches) {
   *n_launches = 0;
@@ -462,130 +527,76 @@ cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, siz
   if (J.cost_kind != USV_COST_NCC && J.cost_kind != USV_COST_ZNCC && J.cost_kind != USV_COST_SSD && J.cost_kind != USV_COST_SAD)
     return cudaErrorNotSupported;
   if (J.channels != 1 && J.channels != 3) return cudaErrorNotSupported;
-  const int nw = J.tw / 4;
   if (J.cost_rows || J.score_rows) return cudaErrorNotSupported;
   const int op = J.cost_kind == USV_COST_SSD ? kOpSsd : J.cost_kind == USV_COST_SAD ? kOpSad : kOpCorr;
-  // the two sweeps: ALU kernel (this file; widths 8 / 12 / 16 / 24 / 32, th <= 64) and tensor-pipe kernel
-  // (usv_dense_mma.cu; any width up to 32, any height, not SAD), which is preferred where both apply
+  // the sweep: a tensor-pipe kernel wherever one covers the job (any width up to 32, any height, not SAD): tcgen05 for
+  // one-plane NCC / ZNCC on frames at least 128 windows wide, mma.sync otherwise; else the ALU kernel (widths
+  // 8 / 12 / 16 / 24 / 32, th <= 64). J.corr_kernel (usv_set_option USV_OPT_CORR_KERNEL, a test / measurement aid):
+  // 0 = this choice, otherwise the named sweep wherever it covers the job
+  const int nw = J.tw / 4;
   const bool alu_ok = J.tw % 4 == 0 && (nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) && J.th <= 64 &&
                       255ll * 255 * J.n_elems < (1ll << 32);  // Sab must fit the u32 accumulators
-  // J.corr_kernel (usv_set_option USV_OPT_CORR_KERNEL, a test / measurement aid): 0 = the dispatch below, otherwise the
-  // named sweep wherever it covers the job
-  const bool mma_ok = J.corr_kernel != USV_CORR_KERNEL_ALU && corr_mma_supported(J, op);
-  if (!alu_ok && !mma_ok) return cudaErrorNotSupported;
-  int pitch;
-  const size_t per_pair = corr_scratch_bytes_per_pair(J, &pitch);
-  const int chunk = (int)std::min<size_t>((size_t)n_pairs, std::max<size_t>(1, scratch_bytes / per_pair));
+  const bool tensor_ok = J.corr_kernel != USV_CORR_KERNEL_ALU && corr_tensor_supported(J, op);
+  if (!alu_ok && !tensor_ok) return cudaErrorNotSupported;
+  const bool umma = J.corr_kernel == USV_CORR_KERNEL_TCGEN05 ||
+                    (J.corr_kernel == USV_CORR_KERNEL_AUTO && J.channels == 1 && op == kOpCorr && J.nxc >= 128);
+  enum Sweep { kAlu, kMma, kUmma };
+  const Sweep sweep = !tensor_ok ? kAlu : umma ? kUmma : kMma;
+
+  const size_t per_pair = corr_scratch_bytes_per_pair(J);
   if (scratch_bytes < per_pair) return cudaErrorNotSupported;
+  const int chunk = (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / per_pair);
 
-  CorrCfg cfg;
-  cfg.stride_px = 4 * (32 - nw + 1);
-  cfg.n_xtiles = (J.nxc + cfg.stride_px - 1) / cfg.stride_px;
-  cfg.x_off = J.camera_side == USV_LEFT_CAM ? ((cfg.n_xtiles * cfg.stride_px - J.nxc) & ~3) : 0;
+  CorrCfg cfg = {};
   cfg.n_eff = J.cost_kind == USV_COST_ZNCC ? (double)J.n_elems : J.cost_kind == USV_COST_SSD ? 2.0 : J.cost_kind == USV_COST_SAD ? -1.0 : 1.0;
-  const int npl = J.channels;
-  const size_t ring_bytes = (size_t)4 * kCRB * npl * kCRowWords * 4;
-  const size_t smem_budget = 74 * 1024;  // three CTAs per SM
-  int bh_max = (int)((smem_budget - ring_bytes) / (128 * 12));
-  if (bh_max < 8) return cudaErrorNotSupported;
-  int n_bands = (J.nyc + bh_max - 1) / bh_max;
-  while ((long long)n_bands * cfg.n_xtiles * n_pairs < g_sm_count * 2 && n_bands < (J.nyc + 15) / 16) ++n_bands;
-  cfg.bh = (J.nyc + n_bands - 1) / n_bands;
-  cfg.n_bands = (J.nyc + cfg.bh - 1) / cfg.bh;
-  const size_t smem = ring_bytes + (size_t)cfg.bh * 128 * 12;
-
-  bool used_mma = false, used_umma = false;
   for (int p0 = 0; p0 < n_pairs; p0 += chunk) {
     const int np = std::min(chunk, n_pairs - p0);
-    uint8_t* base = (uint8_t*)d_scratch;
-    const uint8_t* fl = J.left + (long long)p0 * J.frame_stride;
-    const uint8_t* fr = J.right + (long long)p0 * J.frame_stride;
-    if (npl > 1) {
-      cfg.plane_stride = (long long)J.height * pitch;
-      cfg.pair_stride = cfg.plane_stride * npl;
-      cfg.pitch = pitch;
-      uint8_t* pl_l = base;
-      uint8_t* pl_r = base + (size_t)np * cfg.pair_stride;
-      base += 2 * (size_t)np * cfg.pair_stride;
-      const cudaError_t e = launch_split_planes(J, p0, np, pl_l, pl_r, pitch, st);
+    const CorrScratch s = corr_scratch(J, np);
+    uint8_t* const base = (uint8_t*)d_scratch;  // 256-byte aligned (cudaMalloc)
+    cfg.pair0 = p0;
+    if (J.channels > 1) {
+      cfg.pitch = colour_plane_pitch(J);
+      cfg.plane_stride = (long long)J.height * cfg.pitch;
+      cfg.pair_stride = cfg.plane_stride * J.channels;
+      cfg.lp = base;
+      cfg.rp = base + s.planes_r;
+      const cudaError_t e = launch_split_planes(J, p0, np, base, base + s.planes_r, cfg.pitch, st);
       if (e != cudaSuccess) return e;
-      cfg.lp = pl_l; cfg.rp = pl_r;
       *n_launches += 2;
     } else {
-      cfg.lp = fl; cfg.rp = fr;
+      cfg.lp = J.left + (long long)p0 * J.frame_stride;
+      cfg.rp = J.right + (long long)p0 * J.frame_stride;
       cfg.pitch = J.row_stride; cfg.plane_stride = 0; cfg.pair_stride = J.frame_stride;
     }
-    base = (uint8_t*)(((uintptr_t)base + 255) & ~(uintptr_t)255);
-    double2* st_l = (double2*)base;
-    double2* st_r = st_l + (size_t)np * J.nyc * J.nxc;
-    uint2* rsum = (uint2*)(st_r + (size_t)np * J.nyc * J.nxc);  // [np][H][nxc], reused for the right camera
-    {
-      const int band_rows = 32;  // short bands: the kernel is latency-bound (one dependent load chain per thread)
-      const dim3 g1(((J.nxc + 31) / 32 + 63) / 64, J.height, np);
-      const dim3 g2((J.nxc + 127) / 128, (J.nyc + band_rows - 1) / band_rows, np);
-      // row sums: prefix-sum kernel when the row fits one block's registers, else the sliding one
-      const bool scan = (J.width * J.channels + 3) / 4 <= kScanThreads * kScanWords;
-      const dim3 gs(J.height, np);
-      const size_t smem_scan = (size_t)(J.width + 1) * sizeof(uint2);
-      if (scan) corr_rowsum_scan_kernel<<<gs, kScanThreads, smem_scan, st>>>(fl, J.frame_stride, J.row_stride, J.channels, J.tw, J.nxc, J.width, J.height, rsum);
-      else corr_rowsum_kernel<<<g1, 64, 0, st>>>(fl, J.frame_stride, J.row_stride, J.channels, J.tw, J.nxc, J.height, rsum);
-      corr_stats_kernel<<<g2, 128, 0, st>>>(rsum, J.height, J.tw, J.th, J.channels, J.nxc, J.nyc, J.cost_kind, 1, band_rows, st_l);
-      if (scan) corr_rowsum_scan_kernel<<<gs, kScanThreads, smem_scan, st>>>(fr, J.frame_stride, J.row_stride, J.channels, J.tw, J.nxc, J.width, J.height, rsum);
-      else corr_rowsum_kernel<<<g1, 64, 0, st>>>(fr, J.frame_stride, J.row_stride, J.channels, J.tw, J.nxc, J.height, rsum);
-      corr_stats_kernel<<<g2, 128, 0, st>>>(rsum, J.height, J.tw, J.th, J.channels, J.nxc, J.nyc, J.cost_kind, 0, band_rows, st_r);
-      *n_launches += 4;
+    // window statistics of each camera: row sums into rsum ([np][H][nxc], by prefix sums when the row fits one block's
+    // registers, else sliding), then their vertical sliding sums
+    uint2* rsum = (uint2*)(base + s.rsum);
+    double2* stat[2] = {(double2*)(base + s.stat_l), (double2*)(base + s.stat_r)};
+    const int band_rows = 32;  // short bands: the kernel is latency-bound (one dependent load chain per thread)
+    const dim3 g1(((J.nxc + 31) / 32 + 63) / 64, J.height, np);
+    const dim3 g2((J.nxc + 127) / 128, (J.nyc + band_rows - 1) / band_rows, np);
+    const bool scan = (J.width * J.channels + 3) / 4 <= kScanThreads * kScanWords;
+    const dim3 gs(J.height, np);
+    const size_t smem_scan = (size_t)(J.width + 1) * sizeof(uint2);
+    for (int cam = 0; cam < 2; ++cam) {
+      const uint8_t* f = (cam ? J.right : J.left) + (long long)p0 * J.frame_stride;
+      if (scan) corr_rowsum_scan_kernel<<<gs, kScanThreads, smem_scan, st>>>(f, J.frame_stride, J.row_stride, J.channels, J.tw, J.nxc, J.width, J.height, rsum);
+      else corr_rowsum_kernel<<<g1, 64, 0, st>>>(f, J.frame_stride, J.row_stride, J.channels, J.tw, J.nxc, J.height, rsum);
+      corr_stats_kernel<<<g2, 128, 0, st>>>(rsum, J.height, J.tw, J.th, J.channels, J.nxc, J.nyc, J.cost_kind, cam == 0, band_rows, stat[cam]);
     }
-    cfg.stat_l = st_l; cfg.stat_r = st_r;
-    cfg.pair0 = p0;
-    {
-      // NCC / ZNCC / SSD with 16- or 32-px templates: the row products run on the integer tensor pipe (usv_dense_mma.cu)
-      uint8_t* bb = (uint8_t*)(rsum + (size_t)np * J.height * J.nxc);
-      bb = (uint8_t*)(((uintptr_t)bb + 255) & ~(uintptr_t)255);
-      cfg.best_v = (double*)bb;
-      cfg.best_sc = cfg.best_v + (size_t)np * J.nyc * J.nxc;
-      cfg.best_x = (int*)(cfg.best_sc + (size_t)np * J.nyc * J.nxc);
-      cudaError_t e = cudaErrorNotSupported;
-      const bool umma_auto = J.channels == 1 && op == kOpCorr && J.nxc >= 128;
-      if (mma_ok && (J.corr_kernel == USV_CORR_KERNEL_TCGEN05 || (J.corr_kernel == USV_CORR_KERNEL_AUTO && umma_auto)) && corr_umma_supported(J, op)) {
-        e = launch_corr_umma(J, cfg, op, np, st);
-        if (e == cudaSuccess) used_umma = true;
-      }
-      if (e == cudaErrorNotSupported) e = mma_ok ? launch_corr_mma(J, cfg, op, np, st) : cudaErrorNotSupported;
-      if (e == cudaSuccess) {
-        *n_launches += 1;
-        used_mma = true;
-        continue;
-      }
-      if (e != cudaErrorNotSupported || !alu_ok) return e;
-      (void)cudaGetLastError();
-    }
-    const dim3 grid(cfg.n_xtiles, cfg.n_bands, np), block(kCThreads);
-#define USV_CORR_LAUNCH(D, NWW, NPLL)                                                                      \
-  {                                                                                                        \
-    auto kfn = op == kOpSsd ? dense_corr_argmin_kernel<D, NWW, NPLL, kOpSsd>                               \
-             : op == kOpSad ? dense_corr_argmin_kernel<D, NWW, NPLL, kOpSad>                               \
-                            : dense_corr_argmin_kernel<D, NWW, NPLL, kOpCorr>;                             \
-    cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-    if (e != cudaSuccess) return e;                                                                        \
-    kfn<<<grid, block, smem, st>>>(J, cfg);                                                                \
-  }
-#define USV_CORR_BY_NW(D, NPLL)                                                                            \
-  switch (nw) {                                                                                            \
-    case 2: USV_CORR_LAUNCH(D, 2, NPLL) break;                                                             \
-    case 3: USV_CORR_LAUNCH(D, 3, NPLL) break;                                                             \
-    case 4: USV_CORR_LAUNCH(D, 4, NPLL) break;                                                             \
-    case 6: USV_CORR_LAUNCH(D, 6, NPLL) break;                                                             \
-    default: USV_CORR_LAUNCH(D, 8, NPLL) break;                                                            \
-  }
-    if (J.camera_side == USV_LEFT_CAM) { if (npl == 1) USV_CORR_BY_NW(-1, 1) else USV_CORR_BY_NW(-1, 3) }
-    else { if (npl == 1) USV_CORR_BY_NW(1, 1) else USV_CORR_BY_NW(1, 3) }
-#undef USV_CORR_BY_NW
-#undef USV_CORR_LAUNCH
-    *n_launches += 1;
-    cudaError_t e = cudaGetLastError();
+    *n_launches += 4;
+    cfg.stat_l = stat[0];
+    cfg.stat_r = stat[1];
+    cfg.best_v = (double*)(base + s.best_v);
+    cfg.best_sc = (double*)(base + s.best_sc);
+    cfg.best_x = (int*)(base + s.best_x);
+    const cudaError_t e = sweep == kAlu   ? launch_corr_alu(J, cfg, op, np, n_pairs, st)
+                          : sweep == kMma ? launch_corr_mma(J, cfg, op, np, st)
+                                          : launch_corr_umma(J, cfg, op, np, st);
     if (e != cudaSuccess) return e;
+    *n_launches += 1;
   }
-  *kernel_name = used_umma ? "dense_corr_umma_kernel" : used_mma ? "dense_corr_mma_kernel" : "dense_corr_argmin_kernel";
+  *kernel_name = sweep == kAlu ? "dense_corr_argmin_kernel" : sweep == kMma ? "dense_corr_mma_kernel" : "dense_corr_umma_kernel";
   return cudaSuccess;
 }
 

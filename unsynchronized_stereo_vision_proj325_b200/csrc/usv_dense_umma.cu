@@ -66,11 +66,9 @@ __device__ __forceinline__ void u_ld8(uint32_t taddr, uint32_t (&v)[8]) {
                : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
                : "r"(taddr) : "memory");
 }
-__device__ __forceinline__ bool u_better(double v_o, int x_o, double v_m, int x_m) { return v_o < v_m || (v_o == v_m && x_o < x_m); }
 
 template <int NPL, int OP, bool WS>
 __global__ void __launch_bounds__(u_threads(NPL), u_ctas(NPL)) dense_corr_umma_kernel(const DevJob J, const CorrCfg cfg) {
-  constexpr bool SSD = OP != kOpCorr;
   constexpr int kUThreads = u_threads(NPL), kUCols = u_cols(NPL), kUNQ = kUThreads / 128, kUQCols = kUCols / kUNQ, kUTile = u_tile(NPL);
   constexpr uint32_t kUTmemCols = u_ctas(NPL) == 2 ? 256 : 512, kUAccL = kUTmemCols / 2;
   extern __shared__ __align__(1024) uint8_t usmem[];
@@ -103,10 +101,8 @@ __global__ void __launch_bounds__(u_threads(NPL), u_ctas(NPL)) dense_corr_umma_k
   const double inf = __longlong_as_double(0x7ff0000000000000ll);
   const uint32_t dspan = (uint32_t)(J.dmax - J.dmin);
 
-  const int x_last = min(xm + kUWin - 1, nxc - 1);
   int c_lo, c_hi;
-  if (leftcam) { c_lo = max(0, xm - J.dmax); c_hi = min(nxc - 1, x_last - J.dmin); }
-  else { c_lo = max(0, xm + J.dmin); c_hi = min(nxc - 1, x_last + J.dmax); }
+  corr_cand_cols(J, leftcam, xm, kUWin, c_lo, c_hi);
   const int col_base = c_lo & ~3;
   const int n_pass = c_hi >= c_lo ? (c_hi - col_base) / kUCols + 1 : 1;
 
@@ -292,12 +288,9 @@ __global__ void __launch_bounds__(u_threads(NPL), u_ctas(NPL)) dense_corr_umma_k
             for (int i = 0; i < 8; ++i) {  // ascending x': a later equal candidate never replaces (P/Main.cpp:451)
               const uint32_t sab = e[i] - l[i];
               const double2 Rr = rs[8 * ch + i];
-              const double nsab = __fma_rn(n_eff, __hiloint2double(0x43300000, (int)sab), c0);  // n * Sab, exact
-              const double num = SSD ? __dadd_rn(__dadd_rn(La.x, Rr.x), nsab) : __fma_rn(La.x, Rr.x, nsab);
-              const double sc = SSD ? num : __dmul_rn(__dmul_rn(num, La.y), Rr.y);
-              const double v = __dsub_rn(1.0, sc);
+              const CorrCand c = corr_score<OP>(n_eff, c0, (int)sab, La, Rr);
               const int j = 8 * ch + i;
-              if (v < bv && (uint32_t)(ub + usgn * j) <= dspan) { bv = v; bi = j; if (WS) bs = sc; }
+              if (c.v < bv && (uint32_t)(ub + usgn * j) <= dspan) { bv = c.v; bi = j; if (WS) bs = c.sc; }
             }
           }
         const int mo = ((r & 1) * kUNQ + cq) * kUWin + m;
@@ -316,26 +309,10 @@ __global__ void __launch_bounds__(u_threads(NPL), u_ctas(NPL)) dense_corr_umma_k
         for (int qq = 1; qq < kUNQ; ++qq) {
           const double vo = s_mv[mb + qq * kUWin + tid];
           const int xo = s_mx[mb + qq * kUWin + tid];
-          if (u_better(vo, xo, v, xr)) { v = vo; xr = xo; if (WS) sc = s_msc[mb + qq * kUWin + tid]; }
+          if (corr_v_better(vo, xo, v, xr)) { v = vo; xr = xo; if (WS) sc = s_msc[mb + qq * kUWin + tid]; }
         }
-        if (xw <= nxc - 1) {
-          const long long eidx = ((long long)pair * J.nyc + yo) * nxc + xw;
-          if (pass > 0) {
-            const double vo = cfg.best_v[eidx];
-            const int xo = cfg.best_x[eidx];
-            if (!u_better(v, xr, vo, xo)) { v = vo; xr = xo; if (WS) sc = cfg.best_sc[eidx]; }
-          }
-          if (pass < n_pass - 1) { cfg.best_v[eidx] = v; cfg.best_x[eidx] = xr; if (WS) cfg.best_sc[eidx] = sc; }
-          else {
-            const long long wi = (long long)yo * J.nx + xw;
-            const long long gi = (long long)(cfg.pair0 + pair) * J.n_templates + wi;
-            if (xr == kNoX) write_result(J, gi, (uint32_t)wi, xw, yo, -1, 0xffffffffu, 0.0, inf);
-            else if (SSD) {
-              const uint32_t raw = (uint32_t)__dsub_rn(v, 1.0);
-              write_result(J, gi, (uint32_t)wi, xw, yo, xr, raw, 0.0, normalised_cost(raw, USV_COST_SSD, J.n_elems));
-            } else write_result(J, gi, (uint32_t)wi, xw, yo, xr, 0xffffffffu, __dadd_rn(sc, 0.0), v);
-          }
-        }
+        if (xw <= nxc - 1 && corr_merge_pass<WS>(cfg, ((long long)pair * J.nyc + yo) * nxc + xw, pass, n_pass, v, xr, sc))
+          corr_emit<OP>(J, cfg.pair0 + pair, xw, yo, xr, v, sc);
       }
     }
   }
@@ -344,56 +321,25 @@ __global__ void __launch_bounds__(u_threads(NPL), u_ctas(NPL)) dense_corr_umma_k
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(kUTmemCols) : "memory");
 }
 
-bool corr_umma_supported(const DevJob& J, int op) {
-  if (op == kOpSad) return false;
-  if (J.tw < 1 || J.tw > kUK) return false;
-  if (J.channels != 1 && J.channels != 3) return false;
-  return 255ll * 255 * J.n_elems < (1ll << 31);
+template <int NPL>
+static CorrKernel umma_kernel(int op, bool ws) {
+  if (op == kOpSsd) return dense_corr_umma_kernel<NPL, kOpSsd, false>;
+  return ws ? dense_corr_umma_kernel<NPL, kOpCorr, true> : dense_corr_umma_kernel<NPL, kOpCorr, false>;
 }
 
 cudaError_t launch_corr_umma(const DevJob& J, CorrCfg cfg, int op, int np, cudaStream_t st) {
-  if (!corr_umma_supported(J, op)) return cudaErrorNotSupported;
   cfg.n_xtiles = (J.nxc + kUWin - 1) / kUWin;
+  cfg.n_launch_pairs = np;
   // E and L are running sums over the rows of a band: keep them below 2^31
   const long long per_row = 65025ll * J.tw * J.channels;
   const int bh_cap = (int)std::max<long long>(1, std::min<long long>(J.nyc, ((1ll << 31) - 1) / per_row - J.th));
-  {
-    const int slots = g_sm_count * u_ctas(J.channels);
-    double best_eff = -1.0;
-    int best_nb = (J.nyc + bh_cap - 1) / bh_cap;
-    for (int nb = best_nb; nb <= std::max(best_nb, J.nyc / 8); ++nb) {
-      const int bh = (J.nyc + nb - 1) / nb, nbb = (J.nyc + bh - 1) / bh;
-      if (bh > bh_cap) continue;
-      const long long ctas = (long long)nbb * cfg.n_xtiles * np;
-      const long long waves = (ctas + slots - 1) / slots;
-      const double eff = (double)ctas / (double)(waves * slots) * bh / (bh + 0.2 * (J.th - 1));
-      if (eff > best_eff * 1.005) { best_eff = eff; best_nb = nbb; }
-    }
-    cfg.bh = (J.nyc + best_nb - 1) / best_nb;
-    cfg.n_bands = (J.nyc + cfg.bh - 1) / cfg.bh;
-  }
-  cfg.n_launch_pairs = np;
-  cfg.chunk_pairs = np;
+  corr_bands(J, cfg, np, g_sm_count * u_ctas(J.channels), 0.2, bh_cap);
   const int npl = J.channels;
   const bool ws = op == kOpCorr && J.out.score != nullptr;
   const size_t smem = (size_t)4 * npl * u_tile(npl) + 2 * u_cols(npl) * sizeof(double2) +
                       2 * (u_threads(npl) / 128) * kUWin * (2 * sizeof(double) + sizeof(int)) + 64 + (size_t)4 * npl * kURaw;
-  const dim3 grid(cfg.n_xtiles * cfg.n_bands * np), block(u_threads(npl));
-#define USV_UMMA_LAUNCH(NPLL, OPP, WSS)                                                                    \
-  {                                                                                                        \
-    auto kfn = dense_corr_umma_kernel<NPLL, OPP, WSS>;                                                     \
-    cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
-    if (e != cudaSuccess) return e;                                                                        \
-    kfn<<<grid, block, smem, st>>>(J, cfg);                                                                \
-  }
-#define USV_UMMA_BY_OP(NPLL)                                                                               \
-  if (op == kOpSsd) USV_UMMA_LAUNCH(NPLL, kOpSsd, false)                                                   \
-  else if (ws) USV_UMMA_LAUNCH(NPLL, kOpCorr, true)                                                        \
-  else USV_UMMA_LAUNCH(NPLL, kOpCorr, false)
-  if (npl == 1) USV_UMMA_BY_OP(1) else USV_UMMA_BY_OP(3)
-#undef USV_UMMA_BY_OP
-#undef USV_UMMA_LAUNCH
-  return cudaGetLastError();
+  const CorrKernel k = npl == 1 ? umma_kernel<1>(op, ws) : umma_kernel<3>(op, ws);
+  return launch_corr_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(u_threads(npl)), smem, st, J, cfg);
 }
 
 }  // namespace usv
