@@ -19,12 +19,15 @@
 namespace usv {
 cudaError_t launch_direct(const DevJob& J, int n_pairs, cudaStream_t st);
 bool direct_supported(const DevJob& J);
-// returns cudaErrorNotSupported when the dense kernels do not cover the job
+// the dense sweeps, for dense stride-1 jobs of one or three planes: coverage (usv_dense.cu: the SAD sweep, for a batch of
+// n_pairs; usv_dense_corr.cu: the correlation sweep that serves the job, Sweep::kNone if none), pair scratch, launch
+// (with at least one pair's scratch; launches add to *n_launches)
+bool dense_sad_covers(const DevJob& J, int n_pairs);
 size_t dense_scratch_bytes_per_pair(const DevJob& J);
-cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
-                         int* n_launches);
+cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, int* n_launches);
+Sweep corr_sweep(const DevJob& J);
 size_t corr_scratch_bytes_per_pair(const DevJob& J);
-cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
+cudaError_t launch_dense_corr(const DevJob& J, Sweep sweep, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st,
                               int* n_launches);
 cudaError_t launch_contour_descriptors(const int* pts, const int* off, int n, double* desc, cudaStream_t st);
 cudaError_t launch_contour_costs(const double* dl, int nl, const double* dr, int nr, double* cost, cudaStream_t st);
@@ -381,43 +384,46 @@ static int resolve_device(usv_ctx* ctx, const usv_match* d_in, int64_t n, int32_
                           int64_t* d_n_out, cudaStream_t st);
 
 // ---- matching: device pointers -----------------------------------------------------
-// the matching kernels of one call (dense sweeps first, the direct form for everything they do not cover)
-static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, bool sparse, cudaStream_t st, DevBuf* corr_ws) {
-  int rc;
-  if (!sparse) {
-    const char* name = nullptr;
-    int nl = 0;
-    // the scratch (colour planes of the SAD sweep, planes + window statistics of the correlation sweep) belongs to
+// The sweep that serves a matching call of n_pairs and the pair scratch it needs per pair, chosen before anything is
+// allocated or launched, in the order of the dispatch table of DESIGN §4
+struct MatchPlan {
+  usv::Sweep sweep;
+  size_t scratch_per_pair;
+};
+static MatchPlan plan_match(const DevJob& J, int n_pairs) {
+  using usv::Sweep;
+  const bool dense = !J.tx && J.sx == 1 && J.sy == 1 && (J.channels == 1 || J.channels == 3);
+  // USV_CORR_KERNEL_ALU also moves colour SAD to the ALU correlation kernel (a test / measurement aid)
+  const bool colour_sad_on_alu = J.cost_kind == USV_COST_SAD && J.channels == 3 && J.corr_kernel == USV_CORR_KERNEL_ALU;
+  if (dense && !colour_sad_on_alu && usv::dense_sad_covers(J, n_pairs)) return {Sweep::kSad, usv::dense_scratch_bytes_per_pair(J)};
+  const Sweep corr = dense ? usv::corr_sweep(J) : Sweep::kNone;
+  return corr != Sweep::kNone ? MatchPlan{corr, usv::corr_scratch_bytes_per_pair(J)} : MatchPlan{Sweep::kDirect, 0};
+}
+// by usv::Sweep: the kernel usv_last_kernel reports, and what a failed launch of it is called
+static const char* const kSweepKernel[] = {"dense_sad_argmin_kernel", "dense_corr_argmin_kernel", "dense_corr_mma_kernel",
+                                           "dense_corr_umma_kernel", "block_cost_argmin_direct"};
+static const char* const kSweepLaunch[] = {"dense", "dense correlation", "dense correlation", "dense correlation", "direct"};
+
+// the matching kernels of one call
+static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, cudaStream_t st, DevBuf* corr_ws) {
+  const MatchPlan plan = plan_match(J, n_pairs);
+  int rc, nl = 0;
+  cudaError_t e;
+  if (plan.sweep == usv::Sweep::kDirect) {
+    if ((rc = check_direct(ctx, J))) return rc;
+    e = usv::launch_direct(J, n_pairs, st);
+    nl = 1;
+  } else {
+    // the scratch (colour planes of the SAD sweep, planes + window statistics of the correlation sweeps) belongs to
     // whoever owns the stream: launches on different streams must not share it
     DevBuf& ws = corr_ws ? *corr_ws : ctx->corr_ws;
-    const bool sad_sweep = J.cost_kind == USV_COST_SAD && J.corr_kernel != USV_CORR_KERNEL_ALU;
-    if ((rc = grow_pair_scratch(ctx, ws, sad_sweep ? usv::dense_scratch_bytes_per_pair(J) : 0, n_pairs))) return rc;
-    cudaError_t e = (J.cost_kind == USV_COST_SAD && J.channels == 3 && J.corr_kernel == USV_CORR_KERNEL_ALU)
-                        ? cudaErrorNotSupported  // test / measurement aid: colour SAD on the ALU correlation kernel
-                        : usv::launch_dense(J, n_pairs, ws.p, ws.cap, st, &name, &nl);
-    if (e == cudaSuccess) {
-      ctx->launches += nl;
-      ctx->last_kernel = name;
-      return USV_OK;
-    }
-    if (e != cudaErrorNotSupported) return fail(ctx, USV_ERR_CUDA, "dense launch: %s", cudaGetErrorString(e));
-    (void)cudaGetLastError();
-    // sliding-window correlation kernel
-    if ((rc = grow_pair_scratch(ctx, ws, usv::corr_scratch_bytes_per_pair(J), n_pairs))) return rc;
-    e = usv::launch_dense_corr(J, n_pairs, ws.p, ws.cap, st, &name, &nl);
-    if (e == cudaSuccess) {
-      ctx->launches += nl;
-      ctx->last_kernel = name;
-      return USV_OK;
-    }
-    if (e != cudaErrorNotSupported) return fail(ctx, USV_ERR_CUDA, "dense correlation launch: %s", cudaGetErrorString(e));
-    (void)cudaGetLastError();
+    if ((rc = grow_pair_scratch(ctx, ws, plan.scratch_per_pair, n_pairs))) return rc;
+    e = plan.sweep == usv::Sweep::kSad ? usv::launch_dense(J, n_pairs, ws.p, ws.cap, st, &nl)
+                                       : usv::launch_dense_corr(J, plan.sweep, n_pairs, ws.p, ws.cap, st, &nl);
   }
-  if ((rc = check_direct(ctx, J))) return rc;
-  cudaError_t e = usv::launch_direct(J, n_pairs, st);
-  if (e != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "direct launch: %s", cudaGetErrorString(e));
-  ctx->launches++;
-  ctx->last_kernel = "block_cost_argmin_direct";
+  if (e != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "%s launch: %s", kSweepLaunch[(int)plan.sweep], cudaGetErrorString(e));
+  ctx->launches += nl;
+  ctx->last_kernel = kSweepKernel[(int)plan.sweep];
   return USV_OK;
 }
 
@@ -479,7 +485,7 @@ static int match_device(usv_ctx* ctx, const uint8_t* d_left, const uint8_t* d_ri
       rc = or_scratch(ctx, ws, {{(void**)&o.matches, sizeof(usv_match) * n_res}});
     if (rc) return rc;
   }
-  if ((rc = dispatch_match(ctx, J, n_pairs, sparse, st, corr_ws))) return rc;
+  if ((rc = dispatch_match(ctx, J, n_pairs, st, corr_ws))) return rc;
   if (want_resolved) {
     usv::ResolveRowsSrc S;
     memset(&S, 0, sizeof(S));

@@ -1,4 +1,4 @@
-// usv_common.cuh — device-side structs and helpers shared by the sm_100a kernels.
+// usv_common.cuh — device-side structs and helpers shared by the sm_100a kernels, and the host pieces the dense sweeps share.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -39,8 +39,55 @@ struct DevJob {
 
 constexpr int kDevStatusUmmaTimeout = 1;
 
-// row pitch of the planes that interleaved colour frames are split into for the dense sweeps (usv_dense_corr.cu)
+// ---- host side shared by the dense sweeps
+// the kernel that serves a matching call (usv_capi.cu: plan_match, whose name tables follow this order; DESIGN §4)
+enum class Sweep { kSad, kCorrAlu, kCorrMma, kCorrUmma, kDirect, kNone };
+
+// row pitch of the planes that interleaved colour frames are split into for the dense sweeps, and the bytes of the
+// planes of one frame (0 for one-plane frames, which are read in place)
 inline int colour_plane_pitch(const DevJob& J) { return ((J.width + 15) & ~15) + 16; }
+inline size_t colour_planes_bytes(const DevJob& J) { return J.channels > 1 ? (size_t)J.channels * J.height * colour_plane_pitch(J) : 0; }
+
+// x-tiles of the sliding-window sweeps (SAD and ALU correlation): 32 window positions per byte phase, the first
+// 33 - tw/4 of them emitted. LeftCam windows at small x have few candidates (x' in [x - dmax, x - dmin] clipped at 0):
+// the partly filled tile goes there; RightCam is the mirror image and keeps it at the high-x end.
+template <class Cfg>
+void set_x_tiles(const DevJob& J, Cfg& cfg) {
+  cfg.stride_px = 4 * (33 - J.tw / 4);
+  cfg.n_xtiles = (J.nxc + cfg.stride_px - 1) / cfg.stride_px;
+  cfg.x_off = J.camera_side == USV_LEFT_CAM ? ((cfg.n_xtiles * cfg.stride_px - J.nxc) & ~3) : 0;
+}
+
+// usv_dense_corr.cu: interleaved colour frames of pairs [pair0, pair0 + np) -> planes [pair][plane][H][pitch] of both cameras
+cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst_l, uint8_t* dst_r, int pitch, cudaStream_t st);
+
+// Where a dense sweep reads the rows of the chunk of np pairs from pair p0: the frames themselves (one plane), or their
+// colour planes, split into `planes` (left planes first, then the right ones) by two launches counted in *n_launches.
+template <class Cfg>
+cudaError_t set_chunk_rows(const DevJob& J, int p0, int np, uint8_t* planes, cudaStream_t st, Cfg& cfg, int* n_launches) {
+  if (J.channels == 1) {
+    cfg.lp = J.left + (long long)p0 * J.frame_stride;
+    cfg.rp = J.right + (long long)p0 * J.frame_stride;
+    cfg.pitch = J.row_stride; cfg.plane_stride = 0; cfg.pair_stride = J.frame_stride;
+    return cudaSuccess;
+  }
+  cfg.pitch = colour_plane_pitch(J);
+  cfg.plane_stride = (long long)J.height * cfg.pitch;
+  cfg.pair_stride = cfg.plane_stride * J.channels;
+  uint8_t* const planes_r = planes + np * colour_planes_bytes(J);
+  cfg.lp = planes; cfg.rp = planes_r;
+  *n_launches += 2;
+  return launch_split_planes(J, p0, np, planes, planes_r, cfg.pitch, st);
+}
+
+// sets the kernel's dynamic shared memory limit, then launches it
+template <class... Params, class... Args>
+cudaError_t launch_kernel(void (*k)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const Args&... args) {
+  const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  k<<<grid, block, smem, st>>>(args...);
+  return cudaGetLastError();
+}
 
 __device__ __forceinline__ unsigned long long global_timer_ns() {
   unsigned long long t;

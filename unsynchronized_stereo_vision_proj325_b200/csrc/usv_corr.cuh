@@ -86,15 +86,8 @@ __device__ __forceinline__ void corr_emit(const DevJob& J, int pair, int x, int 
   } else write_result(J, g, (uint32_t)w, x, y, xr, 0xffffffffu, __dadd_rn(sc, 0.0), v);  // -0.0 -> 0.0 (flat windows)
 }
 
-// host side of the two tensor-pipe sweeps (usv_dense_corr.cu chooses the sweep and lays out the scratch)
+// host side of the two tensor-pipe sweeps (usv_dense_corr.cu lays out the scratch; usv_capi.cu: plan_match chooses the sweep)
 using CorrKernel = void (*)(DevJob, CorrCfg);
-// sets the kernel's dynamic shared memory limit, then launches it
-inline cudaError_t launch_corr_kernel(CorrKernel k, dim3 grid, dim3 block, size_t smem, cudaStream_t st, const DevJob& J, const CorrCfg& cfg) {
-  const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  k<<<grid, block, smem, st>>>(J, cfg);
-  return cudaGetLastError();
-}
 // sets cfg.bh and cfg.n_bands for cfg.n_xtiles x-tiles of np pairs on `slots` CTA slots: the band count whose grid fills
 // its waves best, a band paying its th - 1 warm-up rows at `warm_weight` of a full row; bands of at most bh_cap rows
 void corr_bands(const DevJob& J, CorrCfg& cfg, int np, int slots, double warm_weight, int bh_cap);

@@ -39,11 +39,10 @@
 
 namespace usv {
 
-USV_DENSE_DEFINE_VARIANT(1, 4)
-// usv_dense_g8.cu, usv_dense_colour.cu
-template <> cudaError_t dense_launch_variant<1, 8>(int, int, bool, dim3, size_t, const DevJob&, const DenseCfg&, cudaStream_t);
-template <> cudaError_t dense_launch_variant<3, 4>(int, int, bool, dim3, size_t, const DevJob&, const DenseCfg&, cudaStream_t);
-template <> cudaError_t dense_launch_variant<3, 8>(int, int, bool, dim3, size_t, const DevJob&, const DenseCfg&, cudaStream_t);
+// compiled in usv_dense_g8.cu and usv_dense_colour.cu
+extern template DenseKernel dense_kernel<1, 8>(int, int, bool);
+extern template DenseKernel dense_kernel<3, 4>(int, int, bool);
+extern template DenseKernel dense_kernel<3, 8>(int, int, bool);
 
 static int ceil_log2(long long v) {
   int b = 0;
@@ -51,86 +50,83 @@ static int ceil_log2(long long v) {
   return b;
 }
 
-// usv_dense_corr.cu: interleaved colour frames -> planes [pair][plane][H][pitch] of both cameras
-cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst_l, uint8_t* dst_r, int pitch, cudaStream_t st);
-
-// scratch the colour sweep needs per pair (planes of both cameras); 0 for one-plane frames
-size_t dense_scratch_bytes_per_pair(const DevJob& J) {
-  return J.channels == 3 ? 2ull * 3 * J.height * colour_plane_pitch(J) : 0;
+// Shared memory of a CTA: the row ring, then bands of up to bh_max rows of 128 keys. 4 CTAs per SM for gray JT = 4,
+// otherwise 3 (colour: one more plane set of temporaries in registers).
+constexpr int dense_smem_budget(int npl, int jt) { return npl == 1 && jt == 4 ? 56 * 1024 : 75 * 1024; }
+constexpr int dense_ring_words(int npl, int jt, bool ring2, int th) {
+  return (ring2 ? 4 * (npl == 1 ? 4 : 2) : th + 2 * 4) * npl * row_words(jt);
 }
+constexpr int dense_bh_max(int npl, int jt, bool ring2, int th) { return (dense_smem_budget(npl, jt) - 4 * dense_ring_words(npl, jt, ring2, th)) / 512; }
+// the tallest rings: th + 8 rows of one plane (th <= 16; the two-half ring holds 16) and 8 rows of three planes
+static_assert(dense_bh_max(1, 4, false, 16) >= 8 && dense_bh_max(1, 8, false, 16) >= 8 && dense_bh_max(3, 4, true, 0) >= 8 &&
+                  dense_bh_max(3, 8, true, 0) >= 8,
+              "bands of at least 8 rows");
 
-cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
-                         int* n_launches) {
-  // coverage of the sliding-window kernels; everything else runs on the direct-form kernel
-  *n_launches = 0;
-  if (J.tx || (J.channels != 1 && J.channels != 3) || J.sx != 1 || J.sy != 1) return cudaErrorNotSupported;
-  if (J.cost_kind != USV_COST_SAD) return cudaErrorNotSupported;
-  const int nw = J.tw / 4;
-  if (J.tw % 4 != 0 || !(nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) || J.th > 64) return cudaErrorNotSupported;
-  const int npl = J.channels;
-  DenseCfg cfg;
-  cfg.stride_px = 4 * (32 - nw + 1);
-  cfg.n_xtiles = (J.nxc + cfg.stride_px - 1) / cfg.stride_px;
-  // LeftCam windows at small x have few candidates (x' in [x - dmax, x - dmin] clipped at 0): put the
-  // partly filled tile there; RightCam is the mirror image and keeps it at the high-x end
-  cfg.x_off = J.camera_side == USV_LEFT_CAM ? ((cfg.n_xtiles * cfg.stride_px - J.nxc) & ~3) : 0;
+// The SAD sweep's launch of a dense stride-1 job of one or three planes (usv_capi.cu: plan_match checks those), for a batch
+// of n_pairs; false when the sweep does not cover the job.
+struct DenseLaunch {
+  DenseCfg cfg;  // all but the pairs of a launch and where its rows come from
+  int jt;
+  bool ring2;
+  size_t smem;
+};
+static bool dense_launch_cfg(const DevJob& J, int n_pairs, DenseLaunch& L) {
+  const int nw = J.tw / 4, npl = J.channels;
+  if (J.cost_kind != USV_COST_SAD || J.tw % 4 != 0 || !(nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) || J.th > 64) return false;
+  DenseCfg& cfg = L.cfg;
+  set_x_tiles(J, cfg);
   cfg.xb = ceil_log2((long long)J.nxc + kCodeOff + 1);
-  const long long smax = 255ll * J.n_elems;
-  if (ceil_log2(smax + 1) + cfg.xb > 31) return cudaErrorNotSupported;  // bit 31 marks invalid candidates
+  if (ceil_log2(255ll * J.n_elems + 1) + cfg.xb > 31) return false;  // bit 31 marks invalid candidates
   // bands: as tall as shared memory allows (amortises the th-1 warm-up rows), but enough CTAs to fill 148 SMs
   const bool wide_range = std::min(J.dmax, J.nxc - 1) - std::max(J.dmin, -(J.nxc - 1)) + 1 >= 48;
   // 8 disparities per thread (64 per pass, 64 accumulators, three CTAs per SM) when the range is wide enough to fill such
   // passes, gray and colour alike: 24 operand words for 64 VABSDIFF4 instead of 20 for 32, half the reduce-scatter, staging and
   // barriers per candidate (measured on C2: 10.08 against 10.92 ms although the full-range triangle wastes more slots)
-  const int jt = wide_range ? 8 : 4;
-  const int smem_budget = (npl == 1 && jt == 4) ? 56 * 1024 : 75 * 1024;  // 4 CTAs / SM; colour: 3 (one more plane set of temporaries in registers)
-  const bool ring2 = npl > 1 || J.th > 16;  // measured: the short double-fetched ring pays from 24-row templates on
-  const int rb = npl == 1 ? 4 : 2;
-  cfg.ring_words = (ring2 ? 4 * rb : J.th + 2 * rb) * npl * row_words(jt);
-  int bh_max = (smem_budget - cfg.ring_words * 4) / 512;
-  if (bh_max < 8) return cudaErrorNotSupported;
-  const int ctas_per_sm = (npl == 1 && jt == 4) ? 4 : 3;
+  L.jt = wide_range ? 8 : 4;
+  L.ring2 = npl > 1 || J.th > 16;  // measured: the short double-fetched ring pays from 24-row templates on
+  cfg.ring_words = dense_ring_words(npl, L.jt, L.ring2, J.th);
+  const int bh_max = dense_bh_max(npl, L.jt, L.ring2, J.th);
+  const int ctas_per_sm = (npl == 1 && L.jt == 4) ? 4 : 3;
   int n_bands = (J.nyc + bh_max - 1) / bh_max;
   while ((long long)n_bands * cfg.n_xtiles * n_pairs < g_sm_count * (ctas_per_sm - 1) && n_bands < (J.nyc + 15) / 16) ++n_bands;
   cfg.bh = (J.nyc + n_bands - 1) / n_bands;
   cfg.n_bands = (J.nyc + cfg.bh - 1) / cfg.bh;
-  const size_t smem = (size_t)cfg.ring_words * 4 + (size_t)cfg.bh * 512;
+  L.smem = (size_t)cfg.ring_words * 4 + (size_t)cfg.bh * 512;
   const int pitch = npl == 1 ? J.row_stride : colour_plane_pitch(J);
-  cfg.pitch = pitch;
-  cfg.plane_stride = npl == 1 ? 0 : (long long)J.height * pitch;
-  cfg.pair_stride = npl == 1 ? J.frame_stride : cfg.plane_stride * npl;
   cfg.chunk_pairs = (int)std::min<long long>(64, std::max<long long>(1, (48ll << 20) / (2ll * npl * J.height * pitch)));
-  // colour: the planes of a chunk of pairs live in the caller's scratch
+  // one-dimensional grid of the whole batch. Tiles of at least 100 px and bands of at least 16 rows give a pair at most
+  // about nxc * nyc / 1600 blocks, so 2^31 of them would need some 3.4e12 pixels of resident frames per camera
+  return (long long)cfg.n_xtiles * cfg.n_bands * n_pairs <= 0x7fffffffll;
+}
+
+bool dense_sad_covers(const DevJob& J, int n_pairs) {
+  DenseLaunch L;
+  return dense_launch_cfg(J, n_pairs, L);
+}
+
+// scratch the sweep needs per pair: the colour planes of both cameras
+size_t dense_scratch_bytes_per_pair(const DevJob& J) { return 2 * colour_planes_bytes(J); }
+
+// colour: the planes of a chunk of pairs live in the caller's scratch, which holds at least one pair's
+cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, int* n_launches) {
+  DenseLaunch L;
+  if (!dense_launch_cfg(J, n_pairs, L)) return cudaErrorInvalidValue;
+  const int dir = J.camera_side == USV_LEFT_CAM ? -1 : 1, nw = J.tw / 4;
+  const DenseKernel k = J.channels == 3 ? (L.jt == 8 ? dense_kernel<3, 8>(dir, nw, L.ring2) : dense_kernel<3, 4>(dir, nw, L.ring2))
+                                        : (L.jt == 8 ? dense_kernel<1, 8>(dir, nw, L.ring2) : dense_kernel<1, 4>(dir, nw, L.ring2));
   const size_t per_pair = dense_scratch_bytes_per_pair(J);
-  if (npl > 1 && (!d_scratch || scratch_bytes < per_pair)) return cudaErrorNotSupported;
-  const int launch_pairs = npl == 1 ? n_pairs : (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / per_pair);
-  if ((long long)cfg.n_xtiles * cfg.n_bands * launch_pairs > 0x7fffffffll) return cudaErrorNotSupported;
-  for (int p0 = 0; p0 < n_pairs; p0 += launch_pairs) {
-    const int np = std::min(launch_pairs, n_pairs - p0);
+  const int chunk = per_pair ? (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / per_pair) : n_pairs;
+  DenseCfg cfg = L.cfg;
+  for (int p0 = 0; p0 < n_pairs; p0 += chunk) {
+    const int np = std::min(chunk, n_pairs - p0);
     cfg.n_pairs = np;
     cfg.pair0 = p0;
-    if (npl == 1) {
-      cfg.lp = J.left; cfg.rp = J.right;
-    } else {
-      uint8_t* pl_l = (uint8_t*)d_scratch;
-      uint8_t* pl_r = pl_l + (size_t)np * cfg.pair_stride;
-      cudaError_t e = launch_split_planes(J, p0, np, pl_l, pl_r, pitch, st);
-      if (e != cudaSuccess) return e;
-      cfg.lp = pl_l; cfg.rp = pl_r;
-      *n_launches += 2;
-    }
-    const dim3 grid(cfg.n_xtiles * cfg.n_bands * np);
-    const int dir = J.camera_side == USV_LEFT_CAM ? -1 : 1;
-    const cudaError_t e = npl == 3 ? (jt == 8 ? dense_launch_variant<3, 8>(dir, nw, ring2, grid, smem, J, cfg, st)
-                                              : dense_launch_variant<3, 4>(dir, nw, ring2, grid, smem, J, cfg, st))
-                          : jt == 8 ? dense_launch_variant<1, 8>(dir, nw, ring2, grid, smem, J, cfg, st)
-                                    : dense_launch_variant<1, 4>(dir, nw, ring2, grid, smem, J, cfg, st);
+    cudaError_t e = set_chunk_rows(J, p0, np, (uint8_t*)d_scratch, st, cfg, n_launches);
+    if (e == cudaSuccess) e = launch_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(kDenseThreads), L.smem, st, J, cfg, 0xffffffffu);
     if (e != cudaSuccess) return e;
     *n_launches += 1;
   }
-  *kernel_name = "dense_sad_argmin_kernel";
   return cudaSuccess;
 }
-
 
 }  // namespace usv

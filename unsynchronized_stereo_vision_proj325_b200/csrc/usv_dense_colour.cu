@@ -4,7 +4,7 @@
 
 namespace usv {
 
-USV_DENSE_DEFINE_VARIANT(3, 4)
-USV_DENSE_DEFINE_VARIANT(3, 8)
+template DenseKernel dense_kernel<3, 4>(int, int, bool);
+template DenseKernel dense_kernel<3, 8>(int, int, bool);
 
 }  // namespace usv

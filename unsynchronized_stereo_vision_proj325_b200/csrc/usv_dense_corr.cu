@@ -419,8 +419,8 @@ __global__ void corr_stats_kernel(const uint2* __restrict__ rs, int height, int 
   }
 }
 
-// colour planes of both cameras for the sweep below and for the colour SAD sweep of usv_dense.cu (kernels are launched
-// from the translation unit that defines them)
+// colour planes of both cameras for the sweep below and for the colour SAD sweep of usv_dense.cu (usv_common.cuh:
+// set_chunk_rows; kernels are launched from the translation unit that defines them)
 cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst_l, uint8_t* dst_r, int pitch, cudaStream_t st) {
   const long long plane_stride = (long long)J.height * pitch, pair_stride = plane_stride * J.channels;
   const dim3 g((pitch + 255) / 256, J.height, np);
@@ -437,15 +437,14 @@ cudaError_t launch_split_planes(const DevJob& J, int pair0, int np, uint8_t* dst
 // alignments (at most 510 bytes a chunk), so np * per_pair bytes hold a chunk of np pairs.
 struct CorrScratch {
   size_t per_pair;
-  size_t planes_r, stat_l, stat_r, rsum, best_v, best_sc, best_x;  // offsets inside the chunk (left planes at 0)
+  size_t stat_l, stat_r, rsum, best_v, best_sc, best_x;  // offsets inside the chunk (the planes of both cameras at 0)
 };
 static CorrScratch corr_scratch(const DevJob& J, size_t np) {
-  const size_t planes = J.channels > 1 ? (size_t)J.channels * J.height * colour_plane_pitch(J) : 0;  // of one camera
+  const size_t planes = colour_planes_bytes(J);  // of one camera
   const size_t win = (size_t)J.nyc * J.nxc, rows = (size_t)J.height * J.nxc;
   auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
   CorrScratch s;
   s.per_pair = 2 * planes + 2 * win * sizeof(double2) + rows * sizeof(uint2) + win * (2 * sizeof(double) + sizeof(int)) + 1280;
-  s.planes_r = np * planes;
   s.stat_l = align(2 * np * planes);
   s.stat_r = s.stat_l + np * win * sizeof(double2);
   s.rsum = s.stat_r + np * win * sizeof(double2);
@@ -462,6 +461,23 @@ static bool corr_tensor_supported(const DevJob& J, int op) {
   if (op == kOpSad) return false;               // |a - b| is not a product
   if (J.tw < 1 || J.tw > 32) return false;      // K = 32 bytes of one product; narrower templates zero the unused bytes of A
   return 255ll * 255 * J.n_elems < (1ll << 31);  // Sab must fit the s32 accumulators
+}
+
+static int corr_op(const DevJob& J) { return J.cost_kind == USV_COST_SSD ? kOpSsd : J.cost_kind == USV_COST_SAD ? kOpSad : kOpCorr; }
+
+// The sweep of a dense stride-1 job of one or three planes (usv_capi.cu: plan_match checks those), kNone outside the
+// coverage of all three: a tensor-pipe kernel wherever one covers the job (any width up to 32, any height, not SAD):
+// tcgen05 for one-plane NCC / ZNCC on frames at least 128 windows wide, mma.sync otherwise; else the ALU kernel (widths
+// 8 / 12 / 16 / 24 / 32, th <= 64). J.corr_kernel (usv_set_option USV_OPT_CORR_KERNEL, a test / measurement aid):
+// 0 = this choice, otherwise the named sweep wherever it covers the job.
+Sweep corr_sweep(const DevJob& J) {
+  const int op = corr_op(J), nw = J.tw / 4;
+  const bool alu_ok = J.tw % 4 == 0 && (nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) && J.th <= 64 &&
+                      255ll * 255 * J.n_elems < (1ll << 32);  // Sab must fit the u32 accumulators
+  if (J.corr_kernel == USV_CORR_KERNEL_ALU || !corr_tensor_supported(J, op)) return alu_ok ? Sweep::kCorrAlu : Sweep::kNone;
+  const bool umma = J.corr_kernel == USV_CORR_KERNEL_TCGEN05 ||
+                    (J.corr_kernel == USV_CORR_KERNEL_AUTO && J.channels == 1 && op == kOpCorr && J.nxc >= 128);
+  return umma ? Sweep::kCorrUmma : Sweep::kCorrMma;
 }
 
 void corr_bands(const DevJob& J, CorrCfg& cfg, int np, int slots, double warm_weight, int bh_cap) {
@@ -503,9 +519,7 @@ static_assert((kCSmemBudget - (size_t)4 * kCRB * 3 * kCRowWords * 4) / (128 * 12
 // the whole batch (n_pairs) fills fewer than two CTAs per SM
 static cudaError_t launch_corr_alu(const DevJob& J, CorrCfg cfg, int op, int np, int n_pairs, cudaStream_t st) {
   const int nw = J.tw / 4, npl = J.channels;
-  cfg.stride_px = 4 * (32 - nw + 1);
-  cfg.n_xtiles = (J.nxc + cfg.stride_px - 1) / cfg.stride_px;
-  cfg.x_off = J.camera_side == USV_LEFT_CAM ? ((cfg.n_xtiles * cfg.stride_px - J.nxc) & ~3) : 0;
+  set_x_tiles(J, cfg);
   const size_t ring_bytes = (size_t)4 * kCRB * npl * kCRowWords * 4;
   const int bh_max = (int)((kCSmemBudget - ring_bytes) / (128 * 12));
   int n_bands = (J.nyc + bh_max - 1) / bh_max;
@@ -515,38 +529,14 @@ static cudaError_t launch_corr_alu(const DevJob& J, CorrCfg cfg, int op, int np,
   const size_t smem = ring_bytes + (size_t)cfg.bh * 128 * 12;
   const CorrKernel k = J.camera_side == USV_LEFT_CAM ? (npl == 1 ? alu_kernel<-1, 1>(nw, op) : alu_kernel<-1, 3>(nw, op))
                                                      : (npl == 1 ? alu_kernel<1, 1>(nw, op) : alu_kernel<1, 3>(nw, op));
-  return launch_corr_kernel(k, dim3(cfg.n_xtiles, cfg.n_bands, np), dim3(kCThreads), smem, st, J, cfg);
+  return launch_kernel(k, dim3(cfg.n_xtiles, cfg.n_bands, np), dim3(kCThreads), smem, st, J, cfg);
 }
 
-// Returns cudaErrorNotSupported when the job is outside the coverage of the three sweeps (the caller then runs the
-// direct form).
-cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, const char** kernel_name,
+// The correlation sweep `sweep` (corr_sweep) over n_pairs, in chunks of the pairs the scratch holds (at least one).
+cudaError_t launch_dense_corr(const DevJob& J, Sweep sweep, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st,
                               int* n_launches) {
-  *n_launches = 0;
-  if (J.tx || J.sx != 1 || J.sy != 1) return cudaErrorNotSupported;
-  if (J.cost_kind != USV_COST_NCC && J.cost_kind != USV_COST_ZNCC && J.cost_kind != USV_COST_SSD && J.cost_kind != USV_COST_SAD)
-    return cudaErrorNotSupported;
-  if (J.channels != 1 && J.channels != 3) return cudaErrorNotSupported;
-  if (J.cost_rows || J.score_rows) return cudaErrorNotSupported;
-  const int op = J.cost_kind == USV_COST_SSD ? kOpSsd : J.cost_kind == USV_COST_SAD ? kOpSad : kOpCorr;
-  // the sweep: a tensor-pipe kernel wherever one covers the job (any width up to 32, any height, not SAD): tcgen05 for
-  // one-plane NCC / ZNCC on frames at least 128 windows wide, mma.sync otherwise; else the ALU kernel (widths
-  // 8 / 12 / 16 / 24 / 32, th <= 64). J.corr_kernel (usv_set_option USV_OPT_CORR_KERNEL, a test / measurement aid):
-  // 0 = this choice, otherwise the named sweep wherever it covers the job
-  const int nw = J.tw / 4;
-  const bool alu_ok = J.tw % 4 == 0 && (nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) && J.th <= 64 &&
-                      255ll * 255 * J.n_elems < (1ll << 32);  // Sab must fit the u32 accumulators
-  const bool tensor_ok = J.corr_kernel != USV_CORR_KERNEL_ALU && corr_tensor_supported(J, op);
-  if (!alu_ok && !tensor_ok) return cudaErrorNotSupported;
-  const bool umma = J.corr_kernel == USV_CORR_KERNEL_TCGEN05 ||
-                    (J.corr_kernel == USV_CORR_KERNEL_AUTO && J.channels == 1 && op == kOpCorr && J.nxc >= 128);
-  enum Sweep { kAlu, kMma, kUmma };
-  const Sweep sweep = !tensor_ok ? kAlu : umma ? kUmma : kMma;
-
-  const size_t per_pair = corr_scratch_bytes_per_pair(J);
-  if (scratch_bytes < per_pair) return cudaErrorNotSupported;
-  const int chunk = (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / per_pair);
-
+  const int op = corr_op(J);
+  const int chunk = (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / corr_scratch_bytes_per_pair(J));
   CorrCfg cfg = {};
   cfg.n_eff = J.cost_kind == USV_COST_ZNCC ? (double)J.n_elems : J.cost_kind == USV_COST_SSD ? 2.0 : J.cost_kind == USV_COST_SAD ? -1.0 : 1.0;
   for (int p0 = 0; p0 < n_pairs; p0 += chunk) {
@@ -554,20 +544,8 @@ cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, siz
     const CorrScratch s = corr_scratch(J, np);
     uint8_t* const base = (uint8_t*)d_scratch;  // 256-byte aligned (cudaMalloc)
     cfg.pair0 = p0;
-    if (J.channels > 1) {
-      cfg.pitch = colour_plane_pitch(J);
-      cfg.plane_stride = (long long)J.height * cfg.pitch;
-      cfg.pair_stride = cfg.plane_stride * J.channels;
-      cfg.lp = base;
-      cfg.rp = base + s.planes_r;
-      const cudaError_t e = launch_split_planes(J, p0, np, base, base + s.planes_r, cfg.pitch, st);
-      if (e != cudaSuccess) return e;
-      *n_launches += 2;
-    } else {
-      cfg.lp = J.left + (long long)p0 * J.frame_stride;
-      cfg.rp = J.right + (long long)p0 * J.frame_stride;
-      cfg.pitch = J.row_stride; cfg.plane_stride = 0; cfg.pair_stride = J.frame_stride;
-    }
+    cudaError_t e = set_chunk_rows(J, p0, np, base, st, cfg, n_launches);
+    if (e != cudaSuccess) return e;
     // window statistics of each camera: row sums into rsum ([np][H][nxc], by prefix sums when the row fits one block's
     // registers, else sliding), then their vertical sliding sums
     uint2* rsum = (uint2*)(base + s.rsum);
@@ -590,13 +568,12 @@ cudaError_t launch_dense_corr(const DevJob& J, int n_pairs, void* d_scratch, siz
     cfg.best_v = (double*)(base + s.best_v);
     cfg.best_sc = (double*)(base + s.best_sc);
     cfg.best_x = (int*)(base + s.best_x);
-    const cudaError_t e = sweep == kAlu   ? launch_corr_alu(J, cfg, op, np, n_pairs, st)
-                          : sweep == kMma ? launch_corr_mma(J, cfg, op, np, st)
-                                          : launch_corr_umma(J, cfg, op, np, st);
+    e = sweep == Sweep::kCorrAlu   ? launch_corr_alu(J, cfg, op, np, n_pairs, st)
+        : sweep == Sweep::kCorrMma ? launch_corr_mma(J, cfg, op, np, st)
+                                   : launch_corr_umma(J, cfg, op, np, st);
     if (e != cudaSuccess) return e;
     *n_launches += 1;
   }
-  *kernel_name = sweep == kAlu ? "dense_corr_argmin_kernel" : sweep == kMma ? "dense_corr_mma_kernel" : "dense_corr_umma_kernel";
   return cudaSuccess;
 }
 

@@ -3,6 +3,6 @@
 
 namespace usv {
 
-USV_DENSE_DEFINE_VARIANT(1, 8)
+template DenseKernel dense_kernel<1, 8>(int, int, bool);
 
 }  // namespace usv

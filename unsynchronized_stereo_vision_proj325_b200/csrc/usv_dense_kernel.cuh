@@ -1,5 +1,5 @@
-// usv_dense_kernel.cuh — the sliding-window SAD kernel templates (described in usv_dense.cu) and the launch of one
-// (planes, disparities per thread) variant. Included by the three translation units that instantiate the variants
+// usv_dense_kernel.cuh — the sliding-window SAD kernel templates (described in usv_dense.cu) and the choice of the kernel
+// of one (planes, disparities per thread) variant. Included by the three translation units that instantiate the variants
 // (usv_dense.cu: gray JT = 4, usv_dense_g8.cu: gray JT = 8, usv_dense_colour.cu: three planes) so that they compile in
 // parallel; nothing here is specific to one of them.
 #pragma once
@@ -456,37 +456,27 @@ dense_sad_argmin_kernel(const DevJob J, const DenseCfg cfg, const uint32_t minus
   }
 }
 
-// Launch of the <NPL, JT> variant for one direction, template width and ring kind. Explicitly instantiated once per variant.
-template <int NPL, int JT>
-cudaError_t dense_launch_variant(int dir, int nw, bool ring2, dim3 grid, size_t smem, const DevJob& J, const DenseCfg& cfg, cudaStream_t st);
-
-#define USV_DENSE_DEFINE_VARIANT(NPL, JT)                                                                                   \
-  template <int D, int NWW>                                                                                                 \
-  static cudaError_t dense_launch_one_##NPL##_##JT(bool ring2, dim3 grid, size_t smem, const DevJob& J, const DenseCfg& cfg, \
-                                                   cudaStream_t st) {                                                        \
-    auto kfn = (ring2 || NPL > 1) ? dense_sad_argmin_kernel<D, NWW, true, NPL, JT>                                          \
-                                  : dense_sad_argmin_kernel<D, NWW, NPL != 1, NPL, JT>;                                     \
-    cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);                      \
-    if (e != cudaSuccess) return e;                                                                                         \
-    kfn<<<grid, dim3(kDenseThreads), smem, st>>>(J, cfg, 0xffffffffu);                                                      \
-    return cudaGetLastError();                                                                                              \
-  }                                                                                                                         \
-  template <int D>                                                                                                          \
-  static cudaError_t dense_launch_dir_##NPL##_##JT(int nw, bool ring2, dim3 grid, size_t smem, const DevJob& J,              \
-                                                   const DenseCfg& cfg, cudaStream_t st) {                                   \
-    switch (nw) {                                                                                                           \
-      case 2: return dense_launch_one_##NPL##_##JT<D, 2>(ring2, grid, smem, J, cfg, st);                                    \
-      case 3: return dense_launch_one_##NPL##_##JT<D, 3>(ring2, grid, smem, J, cfg, st);                                    \
-      case 4: return dense_launch_one_##NPL##_##JT<D, 4>(ring2, grid, smem, J, cfg, st);                                    \
-      case 6: return dense_launch_one_##NPL##_##JT<D, 6>(ring2, grid, smem, J, cfg, st);                                    \
-      default: return dense_launch_one_##NPL##_##JT<D, 8>(ring2, grid, smem, J, cfg, st);                                   \
-    }                                                                                                                       \
-  }                                                                                                                         \
-  template <>                                                                                                               \
-  cudaError_t dense_launch_variant<NPL, JT>(int dir, int nw, bool ring2, dim3 grid, size_t smem, const DevJob& J,           \
-                                            const DenseCfg& cfg, cudaStream_t st) {                                         \
-    return dir < 0 ? dense_launch_dir_##NPL##_##JT<-1>(nw, ring2, grid, smem, J, cfg, st)                                   \
-                   : dense_launch_dir_##NPL##_##JT<1>(nw, ring2, grid, smem, J, cfg, st);                                   \
+// The kernel of the <NPL, JT> variant for one direction, template width and ring kind (colour frames always run the
+// two-half ring). dense_kernel is explicitly instantiated once per variant, in the translation unit that compiles it.
+using DenseKernel = void (*)(DevJob, DenseCfg, uint32_t);
+template <int DIR, int NW, int NPL, int JT>
+DenseKernel dense_kernel_ring(bool ring2) {
+  if constexpr (NPL > 1) return dense_sad_argmin_kernel<DIR, NW, true, NPL, JT>;
+  else return ring2 ? dense_sad_argmin_kernel<DIR, NW, true, NPL, JT> : dense_sad_argmin_kernel<DIR, NW, false, NPL, JT>;
+}
+template <int DIR, int NPL, int JT>
+DenseKernel dense_kernel_nw(int nw, bool ring2) {
+  switch (nw) {
+    case 2: return dense_kernel_ring<DIR, 2, NPL, JT>(ring2);
+    case 3: return dense_kernel_ring<DIR, 3, NPL, JT>(ring2);
+    case 4: return dense_kernel_ring<DIR, 4, NPL, JT>(ring2);
+    case 6: return dense_kernel_ring<DIR, 6, NPL, JT>(ring2);
+    default: return dense_kernel_ring<DIR, 8, NPL, JT>(ring2);
   }
+}
+template <int NPL, int JT>
+DenseKernel dense_kernel(int dir, int nw, bool ring2) {
+  return dir < 0 ? dense_kernel_nw<-1, NPL, JT>(nw, ring2) : dense_kernel_nw<1, NPL, JT>(nw, ring2);
+}
 
 }  // namespace usv

@@ -403,7 +403,7 @@ cudaError_t launch_corr_mma(const DevJob& J, CorrCfg cfg, int op, int np, cudaSt
                       2 * 4 * kMWin * (2 * sizeof(double) + sizeof(int));
   const CorrKernel k = J.tw > 16 ? (npl == 1 ? mma_kernel<32, 1>(op, ws, ssd_int) : mma_kernel<32, 3>(op, ws, ssd_int))
                                  : (npl == 1 ? mma_kernel<16, 1>(op, ws, ssd_int) : mma_kernel<16, 3>(op, ws, ssd_int));
-  return launch_corr_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(kMThreads), smem, st, J, cfg);
+  return launch_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(kMThreads), smem, st, J, cfg);
 }
 
 }  // namespace usv

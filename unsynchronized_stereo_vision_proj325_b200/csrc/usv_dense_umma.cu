@@ -339,7 +339,7 @@ cudaError_t launch_corr_umma(const DevJob& J, CorrCfg cfg, int op, int np, cudaS
   const size_t smem = (size_t)4 * npl * u_tile(npl) + 2 * u_cols(npl) * sizeof(double2) +
                       2 * (u_threads(npl) / 128) * kUWin * (2 * sizeof(double) + sizeof(int)) + 64 + (size_t)4 * npl * kURaw;
   const CorrKernel k = npl == 1 ? umma_kernel<1>(op, ws) : umma_kernel<3>(op, ws);
-  return launch_corr_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(u_threads(npl)), smem, st, J, cfg);
+  return launch_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(u_threads(npl)), smem, st, J, cfg);
 }
 
 }  // namespace usv

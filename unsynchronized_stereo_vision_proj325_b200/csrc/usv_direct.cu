@@ -13,8 +13,8 @@
 // Match record, disparity and distance (P/Main.cpp:681-694, P/DistanceCalculator.cpp:84).
 //
 // This is the general path (sparse template lists, any stride / template size /
-// channel count, optional dump of every candidate's cost). Dense stride-1 sweeps
-// dispatch to the sliding-window kernels in usv_dense.cu.
+// channel count, optional dump of every candidate's cost). Dense stride-1 jobs that a
+// sliding-window sweep covers go to that sweep instead (DESIGN §4, usv_capi.cu: plan_match).
 #include "usv_common.cuh"
 
 namespace usv {
@@ -291,26 +291,12 @@ bool direct_supported(const DevJob& J) { return direct_layout(J).smem != 0; }
 template <int KIND>
 static cudaError_t launch_direct_c(const DevJob& J, int n_pairs, cudaStream_t st) {
   const DirectLayout d = direct_layout(J);
-  if (d.smem == 0) return cudaErrorInvalidValue;
-  const size_t smem = d.smem;
-  const int tmpl_pitch_words = d.tmpl_pitch_words, strip_pitch_words = d.strip_pitch_words, rows = d.rows;
-  dim3 grid(J.n_templates, n_pairs), block(kDirectThreads);
-#define USV_LAUNCH_C(CC)                                                                              \
-  {                                                                                                   \
-    auto kfn = block_cost_argmin_direct<KIND, CC>;                                                    \
-    cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    if (e != cudaSuccess) return e;                                                                   \
-    kfn<<<grid, block, smem, st>>>(J, tmpl_pitch_words, strip_pitch_words, rows);                      \
-    return cudaGetLastError();                                                                        \
-  }
-  switch (J.channels) {
-    case 1: USV_LAUNCH_C(1)
-    case 2: USV_LAUNCH_C(2)
-    case 3: USV_LAUNCH_C(3)
-    case 4: USV_LAUNCH_C(4)
-    default: return cudaErrorInvalidValue;
-  }
-#undef USV_LAUNCH_C
+  if (d.smem == 0 || J.channels < 1 || J.channels > 4) return cudaErrorInvalidValue;
+  const auto k = J.channels == 1 ? block_cost_argmin_direct<KIND, 1>
+               : J.channels == 2 ? block_cost_argmin_direct<KIND, 2>
+               : J.channels == 3 ? block_cost_argmin_direct<KIND, 3>
+                                 : block_cost_argmin_direct<KIND, 4>;
+  return launch_kernel(k, dim3(J.n_templates, n_pairs), dim3(kDirectThreads), d.smem, st, J, d.tmpl_pitch_words, d.strip_pitch_words, d.rows);
 }
 
 cudaError_t launch_direct(const DevJob& J, int n_pairs, cudaStream_t st) {
