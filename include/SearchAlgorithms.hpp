@@ -29,7 +29,7 @@ struct ColourSearchParameters {
 // What to score and where to look (the reference hard-codes its equivalents: accept 0.75 at
 // P/Main.cpp:417, 640x480 at P/DistanceCalculator.hpp:22-23).
 struct BlockSearchSpec {
-  enum CostKind { SAD = 0, SSD = 1, NCC = 2, ZNCC = 3 };
+  enum CostKind { SAD = 0, SSD = 1, NCC = 2, ZNCC = 3, CENSUS = 4 };  // USV_COST_* of usv_b200.h
   enum DistanceKind { NoDistance = 0, Pinhole = 1, PowerLaw = 2 };
   int TemplateWidth = 16, TemplateHeight = 16;
   int SearchMin = 0, SearchMax = 1 << 20;  // disparity range, clipped to the frame
@@ -86,7 +86,7 @@ int BlockSearch(bool CameraSide, const usv::ImageView* ImportGrayThisCamera, con
 // thread per device, each with its own context, pinned ring and CUDA streams; pair p goes to device floor(p * G / N)
 // (contiguous blocks, no inter-GPU exchange); every worker lands its results in its own disjoint slice of the caller's
 // arrays. Per window: ResolvedDisparity = d of the window's winner if its record survives ResolveMatchList
-// (generate -> accept -> resolve all on the device), else 0xFFFF; RawCost (optional, SAD with 255 * n < 65535) = the
+// (generate -> accept -> resolve all on the device), else 0xFFFF; RawCost (optional, SAD with 255 * n or CENSUS with 8 * n < 65535) = the
 // winner's integer cost. Distance = DistanceTable(...)[d]. Page-lock the frame and result arrays once with
 // BlockSearchPinHostBuffer for asynchronous copies (pageable memory works, slower).
 struct BlockSearchBatchStats {

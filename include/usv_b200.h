@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define USV_ABI_VERSION 4
+#define USV_ABI_VERSION 5
 
 /* ---- status codes ------------------------------------------------------ */
 #define USV_OK 0
@@ -53,6 +53,17 @@ extern "C" {
 #define USV_COST_SSD 1  /* sum (a-b)^2        exact u32                       */
 #define USV_COST_NCC 2  /* 1 - sum ab / sqrt(sum a^2 * sum b^2)        f64     */
 #define USV_COST_ZNCC 3 /* 1 - zero-mean NCC from exact integer sums   f64     */
+#define USV_COST_CENSUS 4 /* Hamming distance of 3x3 census bytes      exact u32   */
+/* USV_COST_CENSUS. Every byte of a frame (pixel (x, y), channel c; channels are independent) becomes
+ *   ct(x, y, c) = sum_{k<8} 2^k [I(n_k) < I(x, y, c)]
+ * over the neighbours n_k of the same channel at (dx, dy) = (-1,-1), (0,-1), (+1,-1), (-1,0), (+1,0), (-1,+1), (0,+1),
+ * (+1,+1) in that order. A neighbour outside [0, width) x [0, height) contributes bit 0; row padding is never read.
+ * A window at x against a candidate at x' on row y costs
+ *   H = sum_{dy<th, dx<tw, c<C} popcount(ctL(x+dx, y+dy, c) XOR ctR(x'+dx, y+dy, c))   (exact u32, at most 8 n)
+ * with n = tmpl_w * tmpl_h * channels: raw_cost = H, MatchValue = H / (8 n), score unused (0). Candidates, the
+ * first-minimum rule, accept test, indices, disparity, distance and the resolved map are those of the other costs.
+ * The cost is unchanged by any strictly increasing intensity map applied to either frame: cameras that expose or
+ * equalise each frame on its own still match. The sub-pixel entry points refuse it (USV_ERR_UNSUPPORTED). */
 
 #define USV_DIST_NONE 0
 #define USV_DIST_PINHOLE 1  /* ((201.6*4)/(disp*0.000043))/1000  P/Main.cpp:694 */
@@ -111,15 +122,16 @@ typedef struct usv_frame_desc {
 typedef struct usv_outputs {
   usv_match *matches;      /* 16-B reference records                          */
   uint32_t *right_index;   /* as usv_match.RightIndex                         */
-  uint32_t *raw_cost;      /* exact integer cost of the winner (SAD/SSD)      */
+  uint32_t *raw_cost;      /* exact integer cost of the winner (SAD/SSD/CENSUS) */
   double *score;           /* NCC / ZNCC correlation of the winner            */
   double *distance;        /* cm, f64 (reference type)                        */
   float *distance_f32;     /* cm, f32 copy for bandwidth-bound consumers      */
   uint16_t *disparity_u16; /* d of the winner or USV_NO_DISPARITY. Meant for search_min >= 0: a negative d
                             * (candidate on the other side of the window) is stored modulo 2^16, and -1 then
                             * reads as USV_NO_DISPARITY — take right_index or matches for such ranges */
-  uint16_t *raw_cost_u16;  /* raw_cost as u16 (0xFFFF = no candidate): SAD only,
-                              and only when 255*tmpl_w*tmpl_h*channels < 0xFFFF,
+  uint16_t *raw_cost_u16;  /* raw_cost as u16 (0xFFFF = no candidate): SAD or
+                              CENSUS only, and only when 255*tmpl_w*tmpl_h*channels
+                              (CENSUS: 8*tmpl_w*tmpl_h*channels) < 0xFFFF,
                               so that no real cost reads as "no candidate"
                               (else USV_ERR_UNSUPPORTED); lossless             */
   uint16_t *resolved_disparity_u16;
@@ -201,7 +213,8 @@ int usv_match_dense_host(usv_ctx *ctx, const uint8_t *h_left,
  * For the sweep's own winners den > 0 always (the first minimum in ascending x' has c(x*-1) > c(x*) <= c(x*+1)); a tie
  * c(x*+1) == c(x*) gives q = +8, the midpoint of the tied pair. The other outputs (distance, disparity_u16, matches,
  * resolved_disparity_u16) keep the integer disparity. To combine with the resolved map, take disparity_x16 where
- * resolved_disparity_u16 != USV_NO_DISPARITY. Frames wider than 2^26 pixels are refused (USV_ERR_UNSUPPORTED).
+ * resolved_disparity_u16 != USV_NO_DISPARITY. Frames wider than 2^26 pixels are refused (USV_ERR_UNSUPPORTED), and
+ * so is USV_COST_CENSUS (the pass reads frame bytes, not census bytes).
  * At least one of the two output pointers must be non-NULL. */
 /* Device pointers (frames as usv_match_dense_device), enqueued on cuda_stream. */
 int usv_refine_subpixel_device(usv_ctx *ctx, const uint8_t *d_left, const uint8_t *d_right,
@@ -218,7 +231,7 @@ int usv_match_dense_subpixel_host(usv_ctx *ctx, const uint8_t *h_left, const uin
 
 /* ---- sparse templates: explicit (x, y) list, shared by all pairs -------- */
 /* cost_rows (optional): [n_pairs][n_templates][row_cap] u32 costs of every
- * candidate in scan order (SAD/SSD); score_rows likewise f64 (NCC/ZNCC).
+ * candidate in scan order (SAD/SSD/CENSUS); score_rows likewise f64 (NCC/ZNCC).
  * Entries past a template's candidate count are left untouched.
  * A template must fit the frame: 0 <= x <= width - tmpl_w, 0 <= y <= height -
  * tmpl_h. The *_host entry point rejects a list that violates this

@@ -3,10 +3,10 @@ import ctypes as C
 
 import numpy as np
 
-USV_ABI_VERSION = 4
+USV_ABI_VERSION = 5
 USV_OK, USV_ERR_INVALID_ARG, USV_ERR_CUDA, USV_ERR_NO_DEVICE, USV_ERR_UNSUPPORTED, USV_ERR_NOMEM = 0, -1, -2, -3, -4, -5
-COST_SAD, COST_SSD, COST_NCC, COST_ZNCC = 0, 1, 2, 3
-COST_NAMES = {"sad": COST_SAD, "ssd": COST_SSD, "ncc": COST_NCC, "zncc": COST_ZNCC}
+COST_SAD, COST_SSD, COST_NCC, COST_ZNCC, COST_CENSUS = 0, 1, 2, 3, 4
+COST_NAMES = {"sad": COST_SAD, "ssd": COST_SSD, "ncc": COST_NCC, "zncc": COST_ZNCC, "census": COST_CENSUS}
 DIST_NONE, DIST_PINHOLE, DIST_POWERLAW = 0, 1, 2
 LEFT_CAM, RIGHT_CAM = 1, 0
 NO_MATCH = 0xFFFFFFFF

@@ -190,7 +190,7 @@ class Context:
         ty = np.ascontiguousarray(ty, np.int32)
         arrs, st = _alloc_host_outputs(n * nt, mask)
         cap = f.width
-        integer = params.cost_kind <= _abi.COST_SSD
+        integer = params.cost_kind not in (_abi.COST_NCC, _abi.COST_ZNCC)
         cost_rows = np.full((n, nt, cap), 0xFFFFFFFF, np.uint32) if rows and integer else None
         score_rows = np.full((n, nt, cap), np.nan, np.float64) if rows and not integer else None
         rc = lib().usv_match_templates_host(self._h, _ptr(left), _ptr(right), C.byref(f), C.c_int32(n), _ptr(tx), _ptr(ty),

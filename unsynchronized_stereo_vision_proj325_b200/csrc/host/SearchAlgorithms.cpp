@@ -112,7 +112,7 @@ void GenerateMatchingList(const usv::ImageView& ThisCamera, const usv::ImageView
   const int nt = (int)Templates.size(), cap = f.width;
   std::vector<int32_t> tx(nt), ty(nt);
   for (int i = 0; i < nt; ++i) { tx[i] = Templates[i].x; ty[i] = Templates[i].y; }
-  const bool integer = p.cost_kind <= USV_COST_SSD;
+  const bool integer = p.cost_kind != USV_COST_NCC && p.cost_kind != USV_COST_ZNCC;
   std::vector<uint32_t> cost_rows(integer ? (size_t)nt * cap : 0);
   std::vector<double> score_rows(integer ? 0 : (size_t)nt * cap);
   usv_outputs out;
@@ -122,7 +122,7 @@ void GenerateMatchingList(const usv::ImageView& ThisCamera, const usv::ImageView
   if (!tc.check(ctx, rc, "usv_match_templates_host")) return;
   const int nxc = f.width - p.tmpl_w + 1;
   const double n_elems = (double)p.tmpl_w * p.tmpl_h * f.channels;
-  const double den = p.cost_kind == USV_COST_SAD ? 255.0 * n_elems : 65025.0 * n_elems;
+  const double den = (p.cost_kind == USV_COST_SAD ? 255.0 : p.cost_kind == USV_COST_CENSUS ? 8.0 : 65025.0) * n_elems;
   for (int i = 0; i < nt; ++i) {  // template-major (P/Main.cpp:408)
     int lo, hi;
     if (p.camera_side == USV_LEFT_CAM) { lo = tx[i] - p.search_max; hi = tx[i] - p.search_min; }

@@ -17,7 +17,8 @@
 #include "usv_common.cuh"
 
 namespace usv {
-cudaError_t launch_direct(const DevJob& J, int n_pairs, cudaStream_t st);
+// the direct form; census runs in chunks of pairs whose census frames the scratch holds (at least one pair's)
+cudaError_t launch_direct(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, int* n_launches);
 bool direct_supported(const DevJob& J);
 // the dense sweeps, for dense stride-1 jobs of one or three planes: coverage (usv_dense.cu: the SAD sweep, for a batch of
 // n_pairs; usv_dense_corr.cu: the correlation sweep that serves the job, Sweep::kNone if none), pair scratch, launch
@@ -235,17 +236,19 @@ static int check_common(usv_ctx* ctx, const usv_frame_desc* f, const usv_search_
   if (p->stride_x <= 0 || p->stride_y <= 0) return fail(ctx, USV_ERR_INVALID_ARG, "stride must be positive");
   if (p->search_min > p->search_max) return fail(ctx, USV_ERR_INVALID_ARG, "search_min > search_max");
   if (p->search_min < -(1 << 24) || p->search_max > (1 << 24)) return fail(ctx, USV_ERR_INVALID_ARG, "search range beyond +-2^24");
-  if (p->cost_kind < USV_COST_SAD || p->cost_kind > USV_COST_ZNCC) return fail(ctx, USV_ERR_INVALID_ARG, "unknown cost_kind %d", p->cost_kind);
+  if (p->cost_kind < USV_COST_SAD || p->cost_kind > USV_COST_CENSUS) return fail(ctx, USV_ERR_INVALID_ARG, "unknown cost_kind %d", p->cost_kind);
   if (p->distance_kind < USV_DIST_NONE || p->distance_kind > USV_DIST_POWERLAW)
     return fail(ctx, USV_ERR_INVALID_ARG, "unknown distance_kind %d", p->distance_kind);
   if (p->camera_side != USV_LEFT_CAM && p->camera_side != USV_RIGHT_CAM) return fail(ctx, USV_ERR_INVALID_ARG, "camera_side must be 0 or 1");
   return USV_OK;
 }
 
-// raw_cost_u16 is lossless or refused: every SAD of the template must fit 16 bits below 0xFFFF, the "no candidate" value
+// raw_cost_u16 is lossless or refused: every SAD or census cost of the template must fit 16 bits below 0xFFFF, the
+// "no candidate" value
 static int check_cost_u16(usv_ctx* ctx, const usv_frame_desc* f, const usv_search_params* p) {
-  if (p->cost_kind != USV_COST_SAD || 255ll * p->tmpl_w * p->tmpl_h * f->channels >= 0xFFFFll)
-    return fail(ctx, USV_ERR_UNSUPPORTED, "raw_cost_u16 needs SAD with 255*tmpl_w*tmpl_h*channels < 65535");
+  const long long unit = p->cost_kind == USV_COST_SAD ? 255 : p->cost_kind == USV_COST_CENSUS ? 8 : 0;
+  if (unit == 0 || unit * p->tmpl_w * p->tmpl_h * f->channels >= 0xFFFFll)
+    return fail(ctx, USV_ERR_UNSUPPORTED, "raw_cost_u16 needs SAD with 255*tmpl_w*tmpl_h*channels < 65535 or CENSUS with 8*... < 65535");
   return USV_OK;
 }
 
@@ -393,34 +396,33 @@ struct MatchPlan {
 static MatchPlan plan_match(const DevJob& J, int n_pairs) {
   using usv::Sweep;
   const bool dense = !J.tx && J.sx == 1 && J.sy == 1 && (J.channels == 1 || J.channels == 3);
-  // USV_CORR_KERNEL_ALU also moves colour SAD to the ALU correlation kernel (a test / measurement aid)
+  // USV_CORR_KERNEL_ALU also moves colour SAD to the ALU correlation kernel (a test / measurement aid); census stays
   const bool colour_sad_on_alu = J.cost_kind == USV_COST_SAD && J.channels == 3 && J.corr_kernel == USV_CORR_KERNEL_ALU;
-  if (dense && !colour_sad_on_alu && usv::dense_sad_covers(J, n_pairs)) return {Sweep::kSad, usv::dense_scratch_bytes_per_pair(J)};
+  if (dense && !colour_sad_on_alu && usv::dense_sad_covers(J, n_pairs))
+    return {J.cost_kind == USV_COST_CENSUS ? Sweep::kCensus : Sweep::kSad, usv::dense_scratch_bytes_per_pair(J)};
   const Sweep corr = dense ? usv::corr_sweep(J) : Sweep::kNone;
-  return corr != Sweep::kNone ? MatchPlan{corr, usv::corr_scratch_bytes_per_pair(J)} : MatchPlan{Sweep::kDirect, 0};
+  return corr != Sweep::kNone ? MatchPlan{corr, usv::corr_scratch_bytes_per_pair(J)}
+                              : MatchPlan{Sweep::kDirect, usv::census_scratch_bytes_per_pair(J)};
 }
 // by usv::Sweep: the kernel usv_last_kernel reports, and what a failed launch of it is called
-static const char* const kSweepKernel[] = {"dense_sad_argmin_kernel", "dense_corr_argmin_kernel", "dense_corr_mma_kernel",
-                                           "dense_corr_umma_kernel", "block_cost_argmin_direct"};
-static const char* const kSweepLaunch[] = {"dense", "dense correlation", "dense correlation", "dense correlation", "direct"};
+static const char* const kSweepKernel[] = {"dense_sad_argmin_kernel", "dense_census_argmin_kernel", "dense_corr_argmin_kernel",
+                                           "dense_corr_mma_kernel", "dense_corr_umma_kernel", "block_cost_argmin_direct"};
+static const char* const kSweepLaunch[] = {"dense", "dense census", "dense correlation", "dense correlation", "dense correlation", "direct"};
 
 // the matching kernels of one call
 static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, cudaStream_t st, DevBuf* corr_ws) {
   const MatchPlan plan = plan_match(J, n_pairs);
   int rc, nl = 0;
-  cudaError_t e;
-  if (plan.sweep == usv::Sweep::kDirect) {
-    if ((rc = check_direct(ctx, J))) return rc;
-    e = usv::launch_direct(J, n_pairs, st);
-    nl = 1;
-  } else {
-    // the scratch (colour planes of the SAD sweep, planes + window statistics of the correlation sweeps) belongs to
-    // whoever owns the stream: launches on different streams must not share it
-    DevBuf& ws = corr_ws ? *corr_ws : ctx->corr_ws;
-    if ((rc = grow_pair_scratch(ctx, ws, plan.scratch_per_pair, n_pairs))) return rc;
-    e = plan.sweep == usv::Sweep::kSad ? usv::launch_dense(J, n_pairs, ws.p, ws.cap, st, &nl)
-                                       : usv::launch_dense_corr(J, plan.sweep, n_pairs, ws.p, ws.cap, st, &nl);
-  }
+  if (plan.sweep == usv::Sweep::kDirect && (rc = check_direct(ctx, J))) return rc;
+  // the scratch (census frames, colour planes of the SAD sweep, planes + window statistics of the correlation sweeps)
+  // belongs to whoever owns the stream: launches on different streams must not share it. Jobs that need none (the direct
+  // form of the costs other than census, gray SAD) grow nothing.
+  DevBuf& ws = corr_ws ? *corr_ws : ctx->corr_ws;
+  if ((rc = grow_pair_scratch(ctx, ws, plan.scratch_per_pair, n_pairs))) return rc;
+  const cudaError_t e = plan.sweep == usv::Sweep::kDirect ? usv::launch_direct(J, n_pairs, ws.p, ws.cap, st, &nl)
+                        : plan.sweep == usv::Sweep::kSad || plan.sweep == usv::Sweep::kCensus
+                            ? usv::launch_dense(J, n_pairs, ws.p, ws.cap, st, &nl)
+                            : usv::launch_dense_corr(J, plan.sweep, n_pairs, ws.p, ws.cap, st, &nl);
   if (e != cudaSuccess) return fail(ctx, USV_ERR_CUDA, "%s launch: %s", kSweepLaunch[(int)plan.sweep], cudaGetErrorString(e));
   ctx->launches += nl;
   ctx->last_kernel = kSweepKernel[(int)plan.sweep];
@@ -431,7 +433,7 @@ static int dispatch_match(usv_ctx* ctx, const DevJob& J, int32_t n_pairs, cudaSt
 enum WinnerSrc { kWinDisparity, kWinRightIndex, kWinMatches };
 
 static WinnerSrc winner_src(const usv_search_params* p, const usv_outputs& o) {
-  if (p->cost_kind > USV_COST_SSD) return kWinMatches;  // the value of a correlation winner is an f64 score
+  if (p->cost_kind == USV_COST_NCC || p->cost_kind == USV_COST_ZNCC) return kWinMatches;  // the value of a correlation winner is an f64 score
   // a u16 disparity names x' only when no candidate lies on the other side of the window (search_min >= 0): negative
   // disparities are stored modulo 2^16 and -1 would read as USV_NO_DISPARITY; such ranges resolve from RightIndex
   const bool disp_ok = p->search_min >= 0;
@@ -522,8 +524,10 @@ extern "C" int usv_match_templates_device(usv_ctx* ctx, const uint8_t* d_left, c
 }
 
 // ---- sub-pixel refinement of dense winners (usv_subpixel.cu) --------------------------
-static int check_subpixel(usv_ctx* ctx, const usv_frame_desc* f, const void* x16, const void* dist) {
+static int check_subpixel(usv_ctx* ctx, const usv_frame_desc* f, const usv_search_params* p, const void* x16, const void* dist) {
   if (!x16 && !dist) return fail(ctx, USV_ERR_INVALID_ARG, "sub-pixel refinement: both output pointers are NULL");
+  // the refinement scores the winner's neighbours from frame bytes; census would need the census frames
+  if (p->cost_kind == USV_COST_CENSUS) return fail(ctx, USV_ERR_UNSUPPORTED, "sub-pixel refinement: not available for USV_COST_CENSUS");
   // 16 * d must fit int32
   if (f->width > (1 << 26)) return fail(ctx, USV_ERR_UNSUPPORTED, "sub-pixel refinement: frame wider than 2^26 pixels");
   return USV_OK;
@@ -532,7 +536,7 @@ static int check_subpixel(usv_ctx* ctx, const usv_frame_desc* f, const void* x16
 static int refine_device(usv_ctx* ctx, const uint8_t* d_left, const uint8_t* d_right, const usv_frame_desc* f, int32_t n_pairs,
                          const usv_search_params* p, const uint32_t* d_ri, int32_t* d_x16, double* d_dist, cudaStream_t st) {
   int rc = check_common(ctx, f, p, n_pairs);
-  if (rc || (rc = check_subpixel(ctx, f, d_x16, d_dist))) return rc;
+  if (rc || (rc = check_subpixel(ctx, f, p, d_x16, d_dist))) return rc;
   if (!d_left || !d_right || !d_ri) return fail(ctx, USV_ERR_INVALID_ARG, "null device pointer");
   if (!aligned16(d_left) || !aligned16(d_right) || (f->row_stride & 15) || (f->frame_stride & 15))
     return fail(ctx, USV_ERR_INVALID_ARG, "device frames need 16-byte aligned base, row_stride and frame_stride");
@@ -568,7 +572,7 @@ static int match_host(usv_ctx* ctx, const uint8_t* h_left, const uint8_t* h_righ
   int rc = check_common(ctx, f, p, n_pairs);
   if (rc) return rc;
   if (!h_left || !h_right || !h_out) return fail(ctx, USV_ERR_INVALID_ARG, "null host pointer");
-  if (sub && (rc = check_subpixel(ctx, f, sub->disparity_x16, sub->distance))) return rc;
+  if (sub && (rc = check_subpixel(ctx, f, p, sub->disparity_x16, sub->distance))) return rc;
   if (n_pairs == 0) return USV_OK;
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;

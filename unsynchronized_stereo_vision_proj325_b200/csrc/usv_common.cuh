@@ -41,12 +41,21 @@ constexpr int kDevStatusUmmaTimeout = 1;
 
 // ---- host side shared by the dense sweeps
 // the kernel that serves a matching call (usv_capi.cu: plan_match, whose name tables follow this order; DESIGN §4)
-enum class Sweep { kSad, kCorrAlu, kCorrMma, kCorrUmma, kDirect, kNone };
+enum class Sweep { kSad, kCensus, kCorrAlu, kCorrMma, kCorrUmma, kDirect, kNone };
 
 // row pitch of the planes that interleaved colour frames are split into for the dense sweeps, and the bytes of the
 // planes of one frame (0 for one-plane frames, which are read in place)
 inline int colour_plane_pitch(const DevJob& J) { return ((J.width + 15) & ~15) + 16; }
 inline size_t colour_planes_bytes(const DevJob& J) { return J.channels > 1 ? (size_t)J.channels * J.height * colour_plane_pitch(J) : 0; }
+
+// census frames (usv_census.cu): interleaved like the frames, rows at a compact 16-byte pitch, padding zeroed. A census
+// job's pair scratch starts with those of both cameras for every pair of a chunk (left frames, then right frames).
+inline int census_pitch(const DevJob& J) { return (J.width * J.channels + 15) & ~15; }
+inline size_t census_frame_bytes(const DevJob& J) { return (size_t)census_pitch(J) * J.height; }
+inline size_t census_scratch_bytes_per_pair(const DevJob& J) { return J.cost_kind == USV_COST_CENSUS ? 2 * census_frame_bytes(J) : 0; }
+// census frames of pairs [p0, p0 + np) of both cameras into `scratch` (one launch, counted in *n_launches), and in Jc the
+// job J on them: pair 0 of Jc is pair p0 of J
+cudaError_t census_chunk(const DevJob& J, int p0, int np, uint8_t* scratch, cudaStream_t st, DevJob& Jc, int* n_launches);
 
 // x-tiles of the sliding-window sweeps (SAD and ALU correlation): 32 window positions per byte phase, the first
 // 33 - tw/4 of them emitted. LeftCam windows at small x have few candidates (x' in [x - dmax, x - dmin] clipped at 0):
@@ -147,9 +156,10 @@ __device__ inline double zncc_score(long long n, long long sab, long long sa, lo
 }
 
 // Normalised MatchValue of an integer cost (0 = perfect; keeps the reference's
-// "accept < 0.75" meaningful, P/Main.cpp:400-401,417).
+// "accept < 0.75" meaningful, P/Main.cpp:400-401,417): the cost over its largest value.
 __device__ inline double normalised_cost(uint32_t raw, int kind, int n_elems) {
-  double den = kind == USV_COST_SAD ? (double)(255ll * n_elems) : (double)(65025ll * n_elems);
+  const long long unit = kind == USV_COST_SAD ? 255ll : kind == USV_COST_CENSUS ? 8ll : 65025ll;
+  double den = (double)(unit * n_elems);
   return __ddiv_rn((double)raw, den);
 }
 
@@ -185,6 +195,9 @@ __device__ __forceinline__ uint32_t sad4_acc(uint32_t a, uint32_t b, uint32_t c)
   asm("vabsdiff4.u32.u32.u32.add %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
   return d;
 }
+
+// c + the Hamming distance of four census bytes -> LOP3 + POPC + IADD
+__device__ __forceinline__ uint32_t hamming4_acc(uint32_t a, uint32_t b, uint32_t c) { return __popc(a ^ b) + c; }
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   unsigned s = (unsigned)__cvta_generic_to_shared(smem);

@@ -35,14 +35,22 @@
 // lanes/clk/SM on the ALU pipe, IMAD at 64 lanes/clk/SM on the FMA pipe in parallel,
 // VIMNMX at 128. The old-row subtraction and the key slide are IMADs on purpose, to keep
 // them off the ALU pipe that bounds this kernel.
+//
+// USV_COST_CENSUS runs the same sweep over census frames (usv_census.cu), transformed into the pair scratch once per chunk
+// of pairs, as dense_census_argmin_kernel: h(u, d, v) = popc(L ^ R) of one packed word (LOP3 + POPC + IADD instead of
+// one VABSDIFF4), at most 8 per byte where SAD has 255.
 #include "usv_dense_kernel.cuh"
 
 namespace usv {
 
-// compiled in usv_dense_g8.cu and usv_dense_colour.cu
+// compiled in usv_dense_g8.cu, usv_dense_colour.cu, usv_dense_census.cu and usv_dense_census_colour.cu
 extern template DenseKernel dense_kernel<1, 8>(int, int, bool);
 extern template DenseKernel dense_kernel<3, 4>(int, int, bool);
 extern template DenseKernel dense_kernel<3, 8>(int, int, bool);
+extern template DenseKernel dense_kernel<1, 4, true>(int, int, bool);
+extern template DenseKernel dense_kernel<1, 8, true>(int, int, bool);
+extern template DenseKernel dense_kernel<3, 4, true>(int, int, bool);
+extern template DenseKernel dense_kernel<3, 8, true>(int, int, bool);
 
 static int ceil_log2(long long v) {
   int b = 0;
@@ -62,8 +70,8 @@ static_assert(dense_bh_max(1, 4, false, 16) >= 8 && dense_bh_max(1, 8, false, 16
                   dense_bh_max(3, 8, true, 0) >= 8,
               "bands of at least 8 rows");
 
-// The SAD sweep's launch of a dense stride-1 job of one or three planes (usv_capi.cu: plan_match checks those), for a batch
-// of n_pairs; false when the sweep does not cover the job.
+// The SAD sweep's launch of a dense stride-1 SAD or census job of one or three planes (usv_capi.cu: plan_match checks
+// those), for a batch of n_pairs; false when the sweep does not cover the job.
 struct DenseLaunch {
   DenseCfg cfg;  // all but the pairs of a launch and where its rows come from
   int jt;
@@ -72,11 +80,13 @@ struct DenseLaunch {
 };
 static bool dense_launch_cfg(const DevJob& J, int n_pairs, DenseLaunch& L) {
   const int nw = J.tw / 4, npl = J.channels;
-  if (J.cost_kind != USV_COST_SAD || J.tw % 4 != 0 || !(nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) || J.th > 64) return false;
+  const bool census = J.cost_kind == USV_COST_CENSUS;
+  if ((J.cost_kind != USV_COST_SAD && !census) || J.tw % 4 != 0 || !(nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) || J.th > 64) return false;
   DenseCfg& cfg = L.cfg;
   set_x_tiles(J, cfg);
   cfg.xb = ceil_log2((long long)J.nxc + kCodeOff + 1);
-  if (ceil_log2(255ll * J.n_elems + 1) + cfg.xb > 31) return false;  // bit 31 marks invalid candidates
+  // bit 31 marks invalid candidates. Census (at most 8 a byte): at th <= 64 any frame narrower than 2^15 px fits
+  if (ceil_log2((census ? 8ll : 255ll) * J.n_elems + 1) + cfg.xb > 31) return false;
   // bands: as tall as shared memory allows (amortises the th-1 warm-up rows), but enough CTAs to fill 148 SMs
   const bool wide_range = std::min(J.dmax, J.nxc - 1) - std::max(J.dmin, -(J.nxc - 1)) + 1 >= 48;
   // 8 disparities per thread (64 per pass, 64 accumulators, three CTAs per SM) when the range is wide enough to fill such
@@ -104,16 +114,20 @@ bool dense_sad_covers(const DevJob& J, int n_pairs) {
   return dense_launch_cfg(J, n_pairs, L);
 }
 
-// scratch the sweep needs per pair: the colour planes of both cameras
-size_t dense_scratch_bytes_per_pair(const DevJob& J) { return 2 * colour_planes_bytes(J); }
+// scratch the sweep needs per pair: the census frames (census) and the colour planes of both cameras
+size_t dense_scratch_bytes_per_pair(const DevJob& J) { return census_scratch_bytes_per_pair(J) + 2 * colour_planes_bytes(J); }
 
-// colour: the planes of a chunk of pairs live in the caller's scratch, which holds at least one pair's
+// census frames and colour planes of a chunk of pairs live in the caller's scratch, which holds at least one pair's
 cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, int* n_launches) {
   DenseLaunch L;
   if (!dense_launch_cfg(J, n_pairs, L)) return cudaErrorInvalidValue;
   const int dir = J.camera_side == USV_LEFT_CAM ? -1 : 1, nw = J.tw / 4;
-  const DenseKernel k = J.channels == 3 ? (L.jt == 8 ? dense_kernel<3, 8>(dir, nw, L.ring2) : dense_kernel<3, 4>(dir, nw, L.ring2))
-                                        : (L.jt == 8 ? dense_kernel<1, 8>(dir, nw, L.ring2) : dense_kernel<1, 4>(dir, nw, L.ring2));
+  const bool census = J.cost_kind == USV_COST_CENSUS;
+  const DenseKernel k =
+      census ? (J.channels == 3 ? (L.jt == 8 ? dense_kernel<3, 8, true>(dir, nw, L.ring2) : dense_kernel<3, 4, true>(dir, nw, L.ring2))
+                                : (L.jt == 8 ? dense_kernel<1, 8, true>(dir, nw, L.ring2) : dense_kernel<1, 4, true>(dir, nw, L.ring2)))
+             : (J.channels == 3 ? (L.jt == 8 ? dense_kernel<3, 8>(dir, nw, L.ring2) : dense_kernel<3, 4>(dir, nw, L.ring2))
+                                : (L.jt == 8 ? dense_kernel<1, 8>(dir, nw, L.ring2) : dense_kernel<1, 4>(dir, nw, L.ring2)));
   const size_t per_pair = dense_scratch_bytes_per_pair(J);
   const int chunk = per_pair ? (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / per_pair) : n_pairs;
   DenseCfg cfg = L.cfg;
@@ -121,8 +135,16 @@ cudaError_t launch_dense(const DevJob& J, int n_pairs, void* d_scratch, size_t s
     const int np = std::min(chunk, n_pairs - p0);
     cfg.n_pairs = np;
     cfg.pair0 = p0;
-    cudaError_t e = set_chunk_rows(J, p0, np, (uint8_t*)d_scratch, st, cfg, n_launches);
-    if (e == cudaSuccess) e = launch_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(kDenseThreads), L.smem, st, J, cfg, 0xffffffffu);
+    // census: the chunk's census frames first (the sweep then reads them from pair 0 of Jc), its colour planes after them
+    DevJob Jc = J;
+    uint8_t* planes = (uint8_t*)d_scratch;
+    cudaError_t e = cudaSuccess;
+    if (census) {
+      e = census_chunk(J, p0, np, planes, st, Jc, n_launches);
+      planes += np * census_scratch_bytes_per_pair(J);
+    }
+    if (e == cudaSuccess) e = set_chunk_rows(Jc, census ? 0 : p0, np, planes, st, cfg, n_launches);
+    if (e == cudaSuccess) e = launch_kernel(k, dim3(cfg.n_xtiles * cfg.n_bands * np), dim3(kDenseThreads), L.smem, st, Jc, cfg, 0xffffffffu);
     if (e != cudaSuccess) return e;
     *n_launches += 1;
   }

@@ -471,6 +471,7 @@ static int corr_op(const DevJob& J) { return J.cost_kind == USV_COST_SSD ? kOpSs
 // 8 / 12 / 16 / 24 / 32, th <= 64). J.corr_kernel (usv_set_option USV_OPT_CORR_KERNEL, a test / measurement aid):
 // 0 = this choice, otherwise the named sweep wherever it covers the job.
 Sweep corr_sweep(const DevJob& J) {
+  if (J.cost_kind == USV_COST_CENSUS) return Sweep::kNone;  // an integer cost of census frames: the SAD sweep or the direct form
   const int op = corr_op(J), nw = J.tw / 4;
   const bool alu_ok = J.tw % 4 == 0 && (nw == 2 || nw == 3 || nw == 4 || nw == 6 || nw == 8) && J.th <= 64 &&
                       255ll * 255 * J.n_elems < (1ll << 32);  // Sab must fit the u32 accumulators

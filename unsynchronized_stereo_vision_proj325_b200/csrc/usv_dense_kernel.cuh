@@ -1,7 +1,12 @@
 // usv_dense_kernel.cuh — the sliding-window SAD kernel templates (described in usv_dense.cu) and the choice of the kernel
-// of one (planes, disparities per thread) variant. Included by the three translation units that instantiate the variants
-// (usv_dense.cu: gray JT = 4, usv_dense_g8.cu: gray JT = 8, usv_dense_colour.cu: three planes) so that they compile in
-// parallel; nothing here is specific to one of them.
+// of one (planes, disparities per thread, cost) variant. Included by the translation units that instantiate the variants
+// (usv_dense.cu: gray JT = 4, usv_dense_g8.cu: gray JT = 8, usv_dense_colour.cu: three planes; usv_dense_census.cu and
+// usv_dense_census_colour.cu: the same for census frames) so that they compile in parallel; nothing here is specific to
+// one of them.
+//
+// CENSUS: the Hamming arm. The frames are census frames (usv_census.cu) and a packed word of four bytes costs
+// popc(a ^ b) (LOP3 + POPC) instead of sum |a - b| (VABSDIFF4); everything else (ring, byte-shifted copies, sliding V
+// sums, keys, BIG columns, fold, thin pass, epilogue) is the same code.
 #pragma once
 #include <algorithm>
 #include <type_traits>
@@ -38,6 +43,13 @@ struct DenseCfg {
   int pair0;        // first pair of this launch inside the caller's batch (outputs are indexed by the global pair)
 };
 
+// c + the cost of four packed bytes of the sweep's cost
+template <bool CENSUS>
+__device__ __forceinline__ uint32_t cost4_acc(uint32_t a, uint32_t b, uint32_t c) {
+  if constexpr (CENSUS) return hamming4_acc(a, b, c);
+  else return sad4_acc(a, b, c);
+}
+
 __device__ __forceinline__ uint32_t imad_u32(uint32_t a, uint32_t b, uint32_t c) {
   uint32_t d;
   asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
@@ -55,7 +67,7 @@ __device__ __forceinline__ uint32_t imad_u32(uint32_t a, uint32_t b, uint32_t c)
 // i0-1, i0-1-NW, ... and i1+NW-1, i1+2NW-1, ... start at BIG = 2^(31-xb) instead of 0. Every invalid
 // window then contains exactly one BIG column and its key carries bit 31 (true keys stay below 2^31,
 // checked on the host), every valid window contains none. No per-element masks, no second code path.
-template <int DIR, int NW, bool FOLD, bool RING2, int NPL, int JT, int NJ = JT>
+template <int DIR, int NW, bool FOLD, bool RING2, int NPL, int JT, bool CENSUS, int NJ = JT>
 __device__ __forceinline__ void dense_pass(const DevJob& J, const DenseCfg& cfg, uint32_t* s_ring, uint32_t* s_best,
                                            const uint32_t* __restrict__ Lg, const uint32_t* __restrict__ Rg, const int X0,
                                            const int XR0, const int run, const int dbase, const int r_shift,
@@ -200,7 +212,7 @@ __device__ __forceinline__ void dense_pass(const DevJob& J, const DenseCfg& cfg,
 #pragma unroll
         for (int i = 0; i < 8; ++i)
 #pragma unroll
-          for (int j = 0; j < NJ; ++j) V[i][j] = sad4_acc(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], V[i][j]);
+          for (int j = 0; j < NJ; ++j) V[i][j] = cost4_acc<CENSUS>(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], V[i][j]);
       }
     }
     if (HAS_OLD) {
@@ -218,7 +230,7 @@ __device__ __forceinline__ void dense_pass(const DevJob& J, const DenseCfg& cfg,
         for (int i = 0; i < 8; ++i)
 #pragma unroll
           for (int j = 0; j < NJ; ++j) {
-            const uint32_t t = sad4_acc(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], 0u);
+            const uint32_t t = cost4_acc<CENSUS>(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], 0u);
             V[i][j] = imad_u32(t, minus_one, V[i][j]);  // V -= t on the FMA pipe
           }
       } else {
@@ -239,12 +251,12 @@ __device__ __forceinline__ void dense_pass(const DevJob& J, const DenseCfg& cfg,
 #pragma unroll
             for (int i = 0; i < 8; ++i)
 #pragma unroll
-              for (int j = 0; j < NJ; ++j) T[i][NJ <= 4 ? j : 0] = sad4_acc(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], pl == 0 ? 0u : T[i][NJ <= 4 ? j : 0]);
+              for (int j = 0; j < NJ; ++j) T[i][NJ <= 4 ? j : 0] = cost4_acc<CENSUS>(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], pl == 0 ? 0u : T[i][NJ <= 4 ? j : 0]);
           } else {
 #pragma unroll
             for (int i = 0; i < 8; ++i)
 #pragma unroll
-              for (int j = 0; j < NJ; ++j) V[i][j] = imad_u32(sad4_acc(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], 0u), minus_one, V[i][j]);
+              for (int j = 0; j < NJ; ++j) V[i][j] = imad_u32(cost4_acc<CENSUS>(Lw[i], Rw[DIR < 0 ? i - j + JT : i + j], 0u), minus_one, V[i][j]);
           }
         }
         if (NJ <= 4) {
@@ -340,11 +352,11 @@ __device__ __forceinline__ void dense_pass(const DevJob& J, const DenseCfg& cfg,
   }
 }
 
+// The body of the sweep's kernels (dense_sad_argmin_kernel, dense_census_argmin_kernel).
 // DIR = -1: LeftCam (x' = x - d); DIR = +1: RightCam (x' = x + d).
 // NW = tw / 4 packed words per window (2..8: the halo columns come from one neighbouring lane).
-template <int DIR, int NW, bool RING2, int NPL, int JT>
-__global__ void __launch_bounds__(kDenseThreads, NPL == 1 && JT == 4 ? 4 : 3)
-dense_sad_argmin_kernel(const DevJob J, const DenseCfg cfg, const uint32_t minus_one) {
+template <int DIR, int NW, bool RING2, int NPL, int JT, bool CENSUS>
+__device__ __forceinline__ void dense_argmin(const DevJob& J, const DenseCfg& cfg, const uint32_t minus_one) {
   constexpr int PD = 8 * JT;  // disparities a warp covers per pass
   extern __shared__ __align__(16) uint32_t smem_u32[];
   uint32_t* s_ring = smem_u32;                                  // RING2 ? [2][2*kRB][kRowWords] : [th + 2*kRB][kRowWords]
@@ -422,14 +434,14 @@ dense_sad_argmin_kernel(const DevJob J, const DenseCfg cfg, const uint32_t minus
     // first byte of the R copies for this pass: R copy q word w = bytes [XR0 + q + 4w, +4)
     const int XR0 = DIR < 0 ? X0 - D0 - PD : X0 + D0;
     const int r_shift = DIR < 0 ? -((D0_mine - D0) >> 2) : ((D0_mine - D0) >> 2);
-    if (fold_pass) dense_pass<DIR, NW, true, RING2, NPL, JT>(J, cfg, s_ring, s_best, Lg, Rg, X0, XR0, run, dbase, r_shift, rows_in, minus_one);
-    else dense_pass<DIR, NW, false, RING2, NPL, JT>(J, cfg, s_ring, s_best, Lg, Rg, X0, XR0, run, dbase, r_shift, rows_in, minus_one);
+    if (fold_pass) dense_pass<DIR, NW, true, RING2, NPL, JT, CENSUS>(J, cfg, s_ring, s_best, Lg, Rg, X0, XR0, run, dbase, r_shift, rows_in, minus_one);
+    else dense_pass<DIR, NW, false, RING2, NPL, JT, CENSUS>(J, cfg, s_ring, s_best, Lg, Rg, X0, XR0, run, dbase, r_shift, rows_in, minus_one);
   }
   if (thin) {
     const int D0 = d_lo + PD * n_pass;
     const int dbase = D0 + 4 * JT * (dl >> 2) + (DIR < 0 ? (p - (dl & 3)) : ((dl & 3) - p));
     const int XR0 = DIR < 0 ? X0 - D0 - PD : X0 + D0;
-    dense_pass<DIR, NW, false, RING2, NPL, JT, 1>(J, cfg, s_ring, s_best, Lg, Rg, X0, XR0, ul, dbase, 0, rows_in, minus_one);
+    dense_pass<DIR, NW, false, RING2, NPL, JT, CENSUS, 1>(J, cfg, s_ring, s_best, Lg, Rg, X0, XR0, ul, dbase, 0, rows_in, minus_one);
   }
   __syncthreads();
 
@@ -451,32 +463,48 @@ dense_sad_argmin_kernel(const DevJob J, const DenseCfg cfg, const uint32_t minus
       const uint32_t raw = key >> xb;
       const int c = (int)(key & code_mask) - kCodeOff;  // = x0 -/+ d of the owning thread column 0
       const int xr = c + 4 * (a & 7);
-      write_result(J, g, (uint32_t)w, x, y, xr, raw, 0.0, normalised_cost(raw, USV_COST_SAD, J.n_elems));
+      write_result(J, g, (uint32_t)w, x, y, xr, raw, 0.0, normalised_cost(raw, CENSUS ? USV_COST_CENSUS : USV_COST_SAD, J.n_elems));
     }
   }
 }
 
-// The kernel of the <NPL, JT> variant for one direction, template width and ring kind (colour frames always run the
-// two-half ring). dense_kernel is explicitly instantiated once per variant, in the translation unit that compiles it.
-using DenseKernel = void (*)(DevJob, DenseCfg, uint32_t);
-template <int DIR, int NW, int NPL, int JT>
-DenseKernel dense_kernel_ring(bool ring2) {
-  if constexpr (NPL > 1) return dense_sad_argmin_kernel<DIR, NW, true, NPL, JT>;
-  else return ring2 ? dense_sad_argmin_kernel<DIR, NW, true, NPL, JT> : dense_sad_argmin_kernel<DIR, NW, false, NPL, JT>;
+template <int DIR, int NW, bool RING2, int NPL, int JT>
+__global__ void __launch_bounds__(kDenseThreads, NPL == 1 && JT == 4 ? 4 : 3)
+dense_sad_argmin_kernel(const DevJob J, const DenseCfg cfg, const uint32_t minus_one) {
+  dense_argmin<DIR, NW, RING2, NPL, JT, false>(J, cfg, minus_one);
 }
-template <int DIR, int NPL, int JT>
+template <int DIR, int NW, bool RING2, int NPL, int JT>
+__global__ void __launch_bounds__(kDenseThreads, NPL == 1 && JT == 4 ? 4 : 3)
+dense_census_argmin_kernel(const DevJob J, const DenseCfg cfg, const uint32_t minus_one) {
+  dense_argmin<DIR, NW, RING2, NPL, JT, true>(J, cfg, minus_one);
+}
+
+// The kernel of the <NPL, JT, CENSUS> variant for one direction, template width and ring kind (colour frames always run
+// the two-half ring). dense_kernel is explicitly instantiated once per variant, in the translation unit that compiles it.
+using DenseKernel = void (*)(DevJob, DenseCfg, uint32_t);
+template <int DIR, int NW, bool RING2, int NPL, int JT, bool CENSUS>
+DenseKernel dense_kernel_cost() {
+  if constexpr (CENSUS) return dense_census_argmin_kernel<DIR, NW, RING2, NPL, JT>;
+  else return dense_sad_argmin_kernel<DIR, NW, RING2, NPL, JT>;
+}
+template <int DIR, int NW, int NPL, int JT, bool CENSUS>
+DenseKernel dense_kernel_ring(bool ring2) {
+  if constexpr (NPL > 1) return dense_kernel_cost<DIR, NW, true, NPL, JT, CENSUS>();
+  else return ring2 ? dense_kernel_cost<DIR, NW, true, NPL, JT, CENSUS>() : dense_kernel_cost<DIR, NW, false, NPL, JT, CENSUS>();
+}
+template <int DIR, int NPL, int JT, bool CENSUS>
 DenseKernel dense_kernel_nw(int nw, bool ring2) {
   switch (nw) {
-    case 2: return dense_kernel_ring<DIR, 2, NPL, JT>(ring2);
-    case 3: return dense_kernel_ring<DIR, 3, NPL, JT>(ring2);
-    case 4: return dense_kernel_ring<DIR, 4, NPL, JT>(ring2);
-    case 6: return dense_kernel_ring<DIR, 6, NPL, JT>(ring2);
-    default: return dense_kernel_ring<DIR, 8, NPL, JT>(ring2);
+    case 2: return dense_kernel_ring<DIR, 2, NPL, JT, CENSUS>(ring2);
+    case 3: return dense_kernel_ring<DIR, 3, NPL, JT, CENSUS>(ring2);
+    case 4: return dense_kernel_ring<DIR, 4, NPL, JT, CENSUS>(ring2);
+    case 6: return dense_kernel_ring<DIR, 6, NPL, JT, CENSUS>(ring2);
+    default: return dense_kernel_ring<DIR, 8, NPL, JT, CENSUS>(ring2);
   }
 }
-template <int NPL, int JT>
+template <int NPL, int JT, bool CENSUS = false>
 DenseKernel dense_kernel(int dir, int nw, bool ring2) {
-  return dir < 0 ? dense_kernel_nw<-1, NPL, JT>(nw, ring2) : dense_kernel_nw<1, NPL, JT>(nw, ring2);
+  return dir < 0 ? dense_kernel_nw<-1, NPL, JT, CENSUS>(nw, ring2) : dense_kernel_nw<1, NPL, JT, CENSUS>(nw, ring2);
 }
 
 }  // namespace usv

@@ -7,6 +7,7 @@
 //   SAD : __vsadu4            -> VABSDIFF4.U8.ACC
 //   SSD : __vabsdiffu4+__dp4a -> VABSDIFF4.U8 + IDP.4A.U8.U8
 //   NCC / ZNCC: three __dp4a  -> exact integer sum(ab), sum(b), sum(b^2)
+//   CENSUS: __popc(a ^ b)     -> LOP3 + POPC, over census frames (usv_census.cu) transformed into the pair scratch
 // Selection is a warp-shuffle + block argmin on a packed (cost, scan index) key,
 // so "smallest cost, then earliest candidate" (P/Main.cpp:451) is one unsigned
 // min and cannot depend on reduction order. The epilogue turns the winner into a
@@ -15,6 +16,8 @@
 // This is the general path (sparse template lists, any stride / template size /
 // channel count, optional dump of every candidate's cost). Dense stride-1 jobs that a
 // sliding-window sweep covers go to that sweep instead (DESIGN §4, usv_capi.cu: plan_match).
+#include <algorithm>
+
 #include "usv_common.cuh"
 
 namespace usv {
@@ -106,9 +109,12 @@ block_cost_argmin_direct(const DevJob J, int tmpl_pitch_words, int strip_pitch_w
     __syncthreads();
   }
 
+  // integer costs (SAD, SSD, census) select on a packed (cost, index) key, correlation costs on an f64 value
+  constexpr bool kInteger = KIND == USV_COST_SAD || KIND == USV_COST_SSD || KIND == USV_COST_CENSUS;
+
   // ---- template sums (NCC / ZNCC only)
   long long t_sa = 0, t_saa = 0;
-  if (KIND >= USV_COST_NCC) {
+  if (!kInteger) {
     unsigned a1 = 0, a2 = 0;
     for (int i = tid; i < J.th * nw; i += kDirectThreads) {
       int r = i / nw, k = i - r * nw;
@@ -194,6 +200,8 @@ block_cost_argmin_direct(const DevJob J, int tmpl_pitch_words, int strip_pitch_w
             } else if (KIND == USV_COST_SSD) {
               uint32_t d = __vabsdiffu4(a, b);
               acc[i] = __dp4a(d, d, acc[i]);
+            } else if (KIND == USV_COST_CENSUS) {
+              acc[i] = hamming4_acc(a, b, acc[i]);
             } else {
               acc[i] = __dp4a(a, b, acc[i]);
               accb[i] = __dp4a(b, 0x01010101u, accb[i]);
@@ -209,7 +217,7 @@ block_cost_argmin_direct(const DevJob J, int tmpl_pitch_words, int strip_pitch_w
     for (int i = 0; i < kCandPerThread; ++i) {
       const int j = jb + 4 * i;
       if (j >= c1) continue;
-      if (KIND <= USV_COST_SSD) {
+      if (kInteger) {
         unsigned long long key = ((unsigned long long)acc[i] << 32) | (unsigned)j;
         best_key = key < best_key ? key : best_key;
         if (J.cost_rows && j < J.row_cap) J.cost_rows[g * J.row_cap + j] = acc[i];
@@ -227,7 +235,7 @@ block_cost_argmin_direct(const DevJob J, int tmpl_pitch_words, int strip_pitch_w
   }
 
   // ---- block argmin (deterministic: pure min on the packed key)
-  if (KIND <= USV_COST_SSD) {
+  if (kInteger) {
     unsigned long long k = warp_min_u64(best_key);
     if (lane == 0) s_red[warp] = k;
     __syncthreads();
@@ -299,7 +307,38 @@ static cudaError_t launch_direct_c(const DevJob& J, int n_pairs, cudaStream_t st
   return launch_kernel(k, dim3(J.n_templates, n_pairs), dim3(kDirectThreads), d.smem, st, J, d.tmpl_pitch_words, d.strip_pitch_words, d.rows);
 }
 
-cudaError_t launch_direct(const DevJob& J, int n_pairs, cudaStream_t st) {
+// census: the pairs run in chunks of what the scratch holds (at least one pair's census frames, usv_common.cuh:
+// census_scratch_bytes_per_pair); each chunk is transformed, then scored with its outputs offset to its first pair
+static cudaError_t launch_direct_census(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st,
+                                        int* n_launches) {
+  const int chunk = (int)std::min<size_t>((size_t)n_pairs, scratch_bytes / census_scratch_bytes_per_pair(J));
+  if (chunk < 1) return cudaErrorInvalidValue;
+  for (int p0 = 0; p0 < n_pairs; p0 += chunk) {
+    const int np = std::min(chunk, n_pairs - p0);
+    DevJob Jc;
+    cudaError_t e = census_chunk(J, p0, np, (uint8_t*)d_scratch, st, Jc, n_launches);
+    if (e != cudaSuccess) return e;
+    const long long off = (long long)p0 * J.n_templates;
+    usv_outputs& o = Jc.out;
+    if (o.matches) o.matches += off;
+    if (o.right_index) o.right_index += off;
+    if (o.raw_cost) o.raw_cost += off;
+    if (o.raw_cost_u16) o.raw_cost_u16 += off;
+    if (o.score) o.score += off;
+    if (o.distance) o.distance += off;
+    if (o.distance_f32) o.distance_f32 += off;
+    if (o.disparity_u16) o.disparity_u16 += off;
+    if (Jc.cost_rows) Jc.cost_rows += off * Jc.row_cap;
+    if (Jc.score_rows) Jc.score_rows += off * Jc.row_cap;
+    if ((e = launch_direct_c<USV_COST_CENSUS>(Jc, np, st)) != cudaSuccess) return e;
+    *n_launches += 1;
+  }
+  return cudaSuccess;
+}
+
+cudaError_t launch_direct(const DevJob& J, int n_pairs, void* d_scratch, size_t scratch_bytes, cudaStream_t st, int* n_launches) {
+  if (J.cost_kind == USV_COST_CENSUS) return launch_direct_census(J, n_pairs, d_scratch, scratch_bytes, st, n_launches);
+  *n_launches += 1;
   switch (J.cost_kind) {
     case USV_COST_SAD: return launch_direct_c<USV_COST_SAD>(J, n_pairs, st);
     case USV_COST_SSD: return launch_direct_c<USV_COST_SSD>(J, n_pairs, st);

@@ -25,15 +25,16 @@ constexpr int kChains = 8;  // independent dependency chains per thread (ILP)
 enum Probe {
   P_SAD4_ACC, P_ABSDIFF4, P_DP4A, P_IADD3, P_IMAD, P_LOP3, P_SHF, P_PRMT, P_VIMNMX, P_LEA,
   P_SAD4_IMAD, P_SAD4_IADD, P_SAD4_VIMNMX, P_DP4A_SAD4, P_DP4A_IMAD, P_SAD4_SHF, P_IADD_IMAD,
-  P_SHFL, P_LDS32, P_LDS128, P_SAD4_LDS, P_DMUL, P_SAD4_DMUL, P_REDUX, P_REDUX_STRIDED, P_SAD4_REDUX, P_COUNT
+  P_SHFL, P_LDS32, P_LDS128, P_SAD4_LDS, P_DMUL, P_SAD4_DMUL, P_REDUX, P_REDUX_STRIDED, P_SAD4_REDUX, P_POPC, P_HAMMING4, P_COUNT
 };
 static const char* kNames[P_COUNT] = {
   "VABSDIFF4.U8.ACC", "VABSDIFF4.U8", "IDP.4A.U8.U8", "IADD3", "IMAD", "LOP3", "SHF.R.W(funnel)", "PRMT", "VIMNMX.U32", "LEA",
   "VABSDIFF4.ACC+IMAD", "VABSDIFF4.ACC+IADD3", "VABSDIFF4.ACC+VIMNMX", "IDP.4A+VABSDIFF4.ACC", "IDP.4A+IMAD", "VABSDIFF4.ACC+SHF",
   "IADD3+IMAD", "SHFL.BFLY", "LDS.32", "LDS.128", "VABSDIFF4.ACC+LDS.32", "DMUL", "VABSDIFF4.ACC+DMUL",
-  "REDUX.MIN.U32(full mask)", "REDUX.MIN.U32(8 lanes, stride 4)", "VABSDIFF4.ACC+REDUX.MIN(stride 4)"};
+  "REDUX.MIN.U32(full mask)", "REDUX.MIN.U32(8 lanes, stride 4)", "VABSDIFF4.ACC+REDUX.MIN(stride 4)", "POPC",
+  "LOP3+POPC+IADD3(census word)"};
 // tested instructions per chain step (for the mixed probes both are counted)
-static const int kOpsPerStep[P_COUNT] = {1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 2, 2, 2, 2, 2, 2, 2, 1, 1, 1, 2, 1, 2, 1, 1, 2};
+static const int kOpsPerStep[P_COUNT] = {1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 2, 2, 2, 2, 2, 2, 2, 1, 1, 1, 2, 1, 2, 1, 1, 2, 1, 3};
 
 __device__ __forceinline__ uint32_t sad4(uint32_t a, uint32_t b, uint32_t c) {
   uint32_t d;
@@ -58,6 +59,11 @@ __device__ __forceinline__ uint32_t iadd3(uint32_t a, uint32_t b, uint32_t c) {
 __device__ __forceinline__ uint32_t lop3(uint32_t a, uint32_t b, uint32_t c) {
   uint32_t d;
   asm volatile("lop3.b32 %0, %1, %2, %3, 0x96;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+  return d;
+}
+__device__ __forceinline__ uint32_t popc(uint32_t a) {
+  uint32_t d;
+  asm volatile("popc.b32 %0, %1;" : "=r"(d) : "r"(a));
   return d;
 }
 __device__ __forceinline__ uint32_t shf(uint32_t a, uint32_t b, uint32_t c) {
@@ -128,6 +134,9 @@ __global__ void __launch_bounds__(kThreads) probe_kernel(uint32_t* out, long lon
       if (P == P_REDUX) x[c] = __reduce_min_sync(0xffffffffu, x[c] + it);
       if (P == P_REDUX_STRIDED) x[c] = __reduce_min_sync(0x11111111u << (threadIdx.x & 3), x[c] + it);
       if (P == P_SAD4_REDUX) { y[c] = sad4(a, b, y[c]); x[c] = __reduce_min_sync(0x11111111u << (threadIdx.x & 3), x[c] + it); }
+      if (P == P_POPC) x[c] = popc(x[c]);
+      // the census sweep's candidate slot (usv_common.cuh: hamming4_acc): c + popc(a ^ b)
+      if (P == P_HAMMING4) x[c] = iadd3(popc(lop3(x[c], a, b)), x[c], a);
       if (P == P_DMUL) dx[c] = __dmul_rn(dx[c], dm);
       if (P == P_SAD4_DMUL) { x[c] = sad4(a, b, x[c]); dx[c] = __dmul_rn(dx[c], dm); }
     }
