@@ -289,7 +289,9 @@ int usv_match_contours(usv_ctx *ctx, const int32_t *pts_this,
  *   BGR2GRAY                                                               :921
  * OpenCV's arithmetic, bit for bit (oracle/preprocess_oracle.py states what is pinned against cv2 and how).
  * maps: the fixed-point pair cv::initUndistortRectifyMap(..., CV_16SC2, ...) / cv::convertMaps produce, shared
- * by all frames of the call; map1 == NULL skips the rectification. */
+ * by all frames of the call; map1 == NULL skips the rectification. Both calls write only the width x height
+ * bytes of each gray frame: row padding and the gaps between frames keep what the caller put there (a gray ROI
+ * inside a larger image is safe), and the host call reads only the 3 * width x height bytes of each BGR frame. */
 #define USV_PRE_OPENCV3 3 /* the reference's library: 14-bit gray coefficients, unfused HSV2BGR products */
 #define USV_PRE_OPENCV4 4 /* cv2 4.13: 15-bit gray coefficients, fused `1 - s*h` (what the tests pin) */
 typedef struct usv_preprocess_params {

@@ -47,10 +47,13 @@ def test_batches_random_maps_and_odd_sizes(ctx, flavour, lighting):
 
 
 def test_hsv2bgr_all_hues(ctx):
-    """Every (H, S, V) of a dense sample goes through the device HSV2BGR: frames are built so that BGR2HSV returns the
-    wanted triple (oracle round trip) and the equalisation is the identity (flat histogram of V)."""
+    """Random frames whose pixels take every hue H in [0, 180) at many saturations and values go through the device
+    HSV2BGR, under the equalisation LUT of each frame. (Every BGR triple, and so every (H, S, V) that BGR2HSV can give,
+    goes through the chain in test_preprocess_limits.py.)"""
     rng = np.random.default_rng(5)
     src = rng.integers(0, 256, (4, 256, 256, 3), dtype=np.uint8)
+    for k in range(4):
+        assert len(np.unique(po.bgr2hsv(src[k])[..., 0])) == 180
     for fl in (_abi.PRE_OPENCV3, _abi.PRE_OPENCV4):
         got = ctx.preprocess(src, lighting=True, flavour=fl)
         for k in range(4):

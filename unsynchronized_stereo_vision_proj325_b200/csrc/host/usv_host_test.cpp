@@ -4,6 +4,7 @@
 // and results so that tests/test_host_cpp.py can compare them with the CPU oracle.
 //   usv_host_test <dump-file>
 //   usv_host_test --bench <pairs> <n_devices> <steps> <warmup>     (one JSON line: the C++ drop-in's throughput)
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -204,6 +205,36 @@ int main(int argc, char** argv) {
       const int b = bgr[3 * k], g = bgr[3 * k + 1], r = bgr[3 * k + 2];
       CHECK(g3[k] == ((b * 1868 + g * 9617 + r * 4899 + (1 << 13)) >> 14));
       CHECK(g4[k] == ((b * 3735 + g * 19235 + r * 9798 + (1 << 14)) >> 15));
+    }
+  }
+  // ---- pre-pass on ROIs (a cv::Mat window: step > row bytes): the source is a 13x7 window of a 23x11 BGR image, the
+  // output a 13x7 window of a 31x11 gray image. Every gray pixel outside the output window keeps its value; with lighting
+  // off the window holds the gray formula of the source window.
+  {
+    const int IW = 23, IH = 11, GW = 31, RW = 13, RH = 7, X0 = 5, Y0 = 2;  // odd width and step: the byte-store path
+    const uint8_t kSentinel = 0xA5;
+    std::vector<uint8_t> img(3 * IW * IH), gray(GW * IH);
+    for (size_t k = 0; k < img.size(); ++k) img[k] = (uint8_t)(53 * k + 7);
+    usv::ImageView roi(img.data() + (size_t)Y0 * 3 * IW + 3 * X0, RW, RH, 3, 3 * IW);
+    for (int lighting = 0; lighting < 2; ++lighting) {
+      for (int opencv3 = 0; opencv3 < 2; ++opencv3) {
+        std::fill(gray.begin(), gray.end(), kSentinel);
+        CHECK(RectifyLightingGray(roi, nullptr, nullptr, lighting != 0, gray.data() + (size_t)Y0 * GW + X0, GW, opencv3 != 0) == 0);
+        int outside_changed = 0, inside_wrong = 0;
+        for (int y = 0; y < IH; ++y)
+          for (int x = 0; x < GW; ++x) {
+            const bool in = y >= Y0 && y < Y0 + RH && x >= X0 && x < X0 + RW;
+            const uint8_t got = gray[(size_t)y * GW + x];
+            if (!in) { outside_changed += got != kSentinel; continue; }
+            if (lighting) continue;
+            const uint8_t* px = img.data() + (size_t)y * 3 * IW + 3 * x;
+            const int b = px[0], g = px[1], r = px[2];
+            inside_wrong += got != (opencv3 ? (b * 1868 + g * 9617 + r * 4899 + (1 << 13)) >> 14
+                                            : (b * 3735 + g * 19235 + r * 9798 + (1 << 14)) >> 15);
+          }
+        CHECK(outside_changed == 0);
+        CHECK(inside_wrong == 0);
+      }
     }
   }
 

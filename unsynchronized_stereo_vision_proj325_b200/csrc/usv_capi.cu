@@ -841,6 +841,21 @@ extern "C" int usv_preprocess_device(usv_ctx* ctx, const uint8_t* d_bgr, int32_t
   return USV_OK;
 }
 
+// `n` frames of `height` rows of `row_bytes` between host and device buffers of the same layout (rows `stride` apart,
+// frames `frame_stride` apart): only those bytes are read and written, never a row's padding or the gap between two
+// frames, which belong to the caller. One 2D copy when the frames are packed, one per frame otherwise.
+static int copy_frame_bytes(usv_ctx* ctx, uint8_t* dst, const uint8_t* src, int32_t n, int row_bytes, int height, int stride,
+                            int64_t frame_stride, cudaMemcpyKind kind) {
+  if (n == 1 || frame_stride == (int64_t)stride * height) {
+    CU(cudaMemcpy2DAsync(dst, stride, src, stride, row_bytes, (size_t)height * n, kind, ctx->stream));
+  } else {
+    for (int32_t i = 0; i < n; ++i)
+      CU(cudaMemcpy2DAsync(dst + (size_t)i * frame_stride, stride, src + (size_t)i * frame_stride, stride, row_bytes, height, kind,
+                           ctx->stream));
+  }
+  return USV_OK;
+}
+
 extern "C" int usv_preprocess_host(usv_ctx* ctx, const uint8_t* h_bgr, int32_t n_frames, const int16_t* h_map1, const uint16_t* h_map2,
                                    const usv_preprocess_params* p, uint8_t* h_gray) {
   if (!ctx) return USV_ERR_INVALID_ARG;
@@ -849,10 +864,14 @@ extern "C" int usv_preprocess_host(usv_ctx* ctx, const uint8_t* h_bgr, int32_t n
   if (n_frames == 0) return USV_OK;
   if (!h_bgr || !h_gray) return fail(ctx, USV_ERR_INVALID_ARG, "null host pointer");
   CU(cudaSetDevice(ctx->device));
+  // the device copies keep the caller's layout; only the frames' own bytes cross the bus
   const size_t src_bytes = (size_t)(n_frames - 1) * p->src_frame_stride + (size_t)p->src_stride * p->height;
   const size_t dst_bytes = (size_t)(n_frames - 1) * p->dst_frame_stride + (size_t)p->dst_stride * p->height;
   const size_t px = (size_t)p->width * p->height;
-  if ((rc = up(ctx, ctx->misc[0], h_bgr, src_bytes))) return rc;
+  if ((rc = grow(ctx, ctx->misc[0], src_bytes)) ||
+      (rc = copy_frame_bytes(ctx, (uint8_t*)ctx->misc[0].p, h_bgr, n_frames, 3 * p->width, p->height, p->src_stride,
+                             p->src_frame_stride, cudaMemcpyHostToDevice)))
+    return rc;
   if ((rc = grow(ctx, ctx->misc[1], dst_bytes))) return rc;
   if (h_map1) {
     if ((rc = up(ctx, ctx->misc[2], h_map1, px * 4))) return rc;
@@ -861,7 +880,9 @@ extern "C" int usv_preprocess_host(usv_ctx* ctx, const uint8_t* h_bgr, int32_t n
   rc = usv_preprocess_device(ctx, (const uint8_t*)ctx->misc[0].p, n_frames, h_map1 ? (const int16_t*)ctx->misc[2].p : nullptr,
                              h_map1 ? (const uint16_t*)ctx->misc[3].p : nullptr, p, (uint8_t*)ctx->misc[1].p, ctx->stream);
   if (rc) return rc;
-  CU(cudaMemcpyAsync(h_gray, ctx->misc[1].p, dst_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if ((rc = copy_frame_bytes(ctx, h_gray, (const uint8_t*)ctx->misc[1].p, n_frames, p->width, p->height, p->dst_stride,
+                             p->dst_frame_stride, cudaMemcpyDeviceToHost)))
+    return rc;
   CU(cudaStreamSynchronize(ctx->stream));
   return USV_OK;
 }
